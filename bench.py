@@ -9,8 +9,11 @@ torch.distributed traffic is the barrier / max-over-ranks of the timing).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path
   python bench.py --impl reference ...                            the reference's CPU decompress()
+  python bench.py ... --dump-outputs DIR                          also write the last timed step's outputs
 
 One JSON line on stdout (rank 0).  See DESIGN.md §Measurement for the definition of every key.
+The inputs are generated from fixed seeds, so two builds run with the same arguments decode the same
+streams and their --dump-outputs files can be compared array for array.
 """
 from __future__ import annotations
 
@@ -28,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 
 from tests import deflate_tools as T  # noqa: E402  (synthetic corpus generators)
 
@@ -230,6 +234,32 @@ def measured_peak_gbs():
         return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_STREAMS = 1 << 20   # at most this many entries of status / written (12 MiB as float32 + float64) ...
+DUMP_BYTES = 11 << 20    # ... and of the decompressed bytes (44 MiB as float32): under 64 MB in all
+
+
+def _sample(t, k: int):
+    """`t` itself when it has at most `k` elements, else `k` of them, one from each of `k` equal
+    strata at an offset drawn from a fixed seed: the same positions on every run."""
+    import torch
+    n = t.numel()
+    if n <= k:
+        return t
+    pos = np.arange(k, dtype=np.int64) * (n // k) + np.random.default_rng(0).integers(0, n // k, k)
+    return t[torch.from_numpy(pos).to(t.device)]
+
+
+def dump_outputs(out_dir: str, d_dst, total_out: int, d_status, d_written):
+    """What the decode step returned to its caller, as .npy files: status.npy (float32) and
+    written.npy (float64) per stream, and dst.npy (float32), the decompressed bytes of the whole
+    batch end to end; each is complete or a fixed sample of DUMP_STREAMS / DUMP_BYTES entries."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("status", _sample(d_status, DUMP_STREAMS).float()),
+                    ("written", _sample(d_written, DUMP_STREAMS).double()),
+                    ("dst", _sample(d_dst[:total_out], DUMP_BYTES).float())):
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def cpu_baseline(w, seconds_budget: float = 15.0, threads: int | None = None):
     """The reference's own CPU decompress() (oracle/_ref, built from the unmodified reference
     sources) — or the C port if that library is absent — one stream per core over all host cores,
@@ -284,7 +314,14 @@ def main():
     ap.add_argument("--shard-streams", type=int, default=1048576, help="streams of the sharded (strong-scaling) batch")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps of the headline workload, write "
+                    "what its last step returned (status, written, decompressed bytes as float32 / float64; a "
+                    "fixed sample of the larger ones, under 64 MB in all) as DIR/<name>.npy (rank 0 under torchrun)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -349,9 +386,10 @@ def main():
         except Exception:
             return None
 
-    def measure(name, w, steps, warmup, want_e2e, streams_total=None, min_region_ms=0.0):
+    def measure(name, w, steps, warmup, want_e2e, streams_total=None, min_region_ms=0.0, dump_dir=None):
         """One workload on this rank's GPU: device-timed steps (CUDA events, max over ranks), the
-        correctness gate, per-pass times, optionally the end-to-end number through host buffers."""
+        correctness gate, per-pass times, optionally the end-to-end number through host buffers and
+        the outputs of the last timed step (dump_dir)."""
         n = w["n"]
         to_i64 = lambda a: torch.from_numpy(a.view(np.int64))
         h_src = torch.from_numpy(w["src"]).pin_memory() if want_e2e else torch.from_numpy(w["src"])
@@ -434,6 +472,8 @@ def main():
         ms_per_step = total_ms / steps
         out_all = streams_total["total_out"] if streams_total else world * w["total_out"]
         value = out_all / (ms_per_step * 1e-3) / 1e9
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, d_dst, w["total_out"], d_status, d_written)
 
         e2e = None
         if want_e2e:
@@ -512,7 +552,8 @@ def main():
 
     # ---- the headline workload (BASELINE.json's metric is quoted on C2) ---------------------------
     w = make_workload(args.workload, n_streams, unique, rank, args.container)
-    head = measure(args.workload, w, args.steps, args.warmup, not args.no_e2e and args.container == "raw")
+    head = measure(args.workload, w, args.steps, args.warmup, not args.no_e2e and args.container == "raw",
+                   dump_dir=args.dump_outputs)
     line = {
         "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": head["ms_per_step"], "higher_is_better": True,
