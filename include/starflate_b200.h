@@ -216,6 +216,44 @@ int sfb200_decompress_container_batch_device(sfb200_ctx* ctx, int container, con
 int sfb200_decompress_container(sfb200_ctx* ctx, int container, const uint8_t* src, size_t src_len,
                                 uint8_t* dst, size_t dst_cap, uint8_t* status, uint64_t* written);
 
+/* gzip FILES: a series of gzip members (RFC 1952 §2.2), as gzip(1), zlib's gunzip and Python's
+ * gzip.decompress accept them — `cat a.gz b.gz`, and BGZF (BAM, bgzip / tabix .vcf.gz, .fastq.gz),
+ * whose members carry their compressed size in the header (extra subfield 'B','C').  The members
+ * are found on the device (BGZF members without any serial walk) and decoded side by side through
+ * the container batch path; a member without the BGZF field costs one extra decode of its payload
+ * to find where it ends.  Member k's output follows member k-1's in dst.
+ *   *status   Success; or the status of the FIRST failing member in file order (the DEFLATE status
+ *             of its payload, SFB200_CHECKSUM_MISMATCH, SFB200_SIZE_MISMATCH — also when a member's
+ *             payload produces more than its ISIZE while dst still had room (for a member without
+ *             the BGZF field: room for its whole payload, as its ISIZE is read only after it) —,
+ *             SFB200_DST_TOO_SMALL
+ *             when dst ends inside a member: every byte that fits is produced); SFB200_BAD_CONTAINER
+ *             for bytes behind the last member that are neither zero padding (ignored) nor a gzip
+ *             member, for a file that does not start with a member, and for a file that ends inside
+ *             a header or trailer.  An empty file is Success with 0 bytes.
+ *   *written  (may be NULL) bytes of dst that hold the file's output: on failure, that member's dst
+ *             offset plus what it produced.  On Success dst past *written is untouched; after a
+ *             failure the bytes past *written are unspecified (later members may have been decoded).
+ *   *members  (may be NULL) members found.
+ * `src` and `dst` are DEVICE pointers, the three results HOST pointers.  Synchronous on
+ * `cuda_stream` (the member count sizes the launches).  Members must be < 4 GiB compressed and
+ * decompressed (BGZF members are <= 64 KiB).  Memory touched: the member scan reads src in aligned
+ * 16-byte blocks, up to 15 bytes before its first and after its last byte.  More than 2^32 - 2
+ * BGZF header candidates (only a file of > 8 GiB of header-like bytes) is SFB200_RC_BAD_ARGUMENT. */
+int sfb200_decompress_gzip_file_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, uint8_t* dst,
+                                       uint64_t dst_cap, uint8_t* status, uint64_t* written, uint64_t* members,
+                                       void* cuda_stream);
+/* The same with HOST buffers.  The whole file and its output must fit in device memory (it is staged
+ * there whole); only the bytes produced are copied back. */
+int sfb200_decompress_gzip_file(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* dst, size_t dst_cap,
+                                uint8_t* status, uint64_t* written, uint64_t* members);
+/* Discovery only (HOST buffer): *size = the sum of ISIZE over the members the walk reaches,
+ * *members (may be NULL) their number; *complete (may be NULL) = 1 when they cover the file (zero
+ * padding aside).  A member without the BGZF field, or anything else that is not a BGZF member,
+ * ends the walk with *complete = 0.  BGZF callers size dst with it exactly. */
+int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint64_t* size, uint64_t* members,
+                          int* complete);
+
 /* Position-weighted 64-bit checksum of each stream's output region [0, len[i]) computed on the
  * device (used by tests/bench to verify multi-GiB outputs without a device->host copy):
  *   sum_j (byte_j + 1) * (0x9E3779B97F4A7C15 * (j + 1) | 1)   mod 2^64. */

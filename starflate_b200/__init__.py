@@ -167,6 +167,47 @@ class Context:
         self._check(rc, "sfb200_decompress_container")
         return st.value, d[:dst_cap].tobytes(), wr.value
 
+    def decompress_gzip_file(self, src: bytes, dst_cap: int, fill: int = 0):
+        """A gzip file of any number of members (BGZF, `cat a.gz b.gz`), host memory
+        -> (status, dst bytes, written, members)."""
+        s = np.frombuffer(src, dtype=np.uint8) if len(src) else np.zeros(1, np.uint8)
+        d = np.full(max(dst_cap, 1), fill, dtype=np.uint8)
+        st, wr, nm = C.c_uint8(0), C.c_uint64(0), C.c_uint64(0)
+        f = self.lib.sfb200_decompress_gzip_file
+        f.argtypes = [C.c_void_p, _u8p, C.c_size_t, _u8p, C.c_size_t, C.POINTER(C.c_uint8), C.POINTER(C.c_uint64),
+                      C.POINTER(C.c_uint64)]
+        f.restype = C.c_int
+        rc = f(self.h, _p(s, _u8p), len(src), _p(d, _u8p), dst_cap, C.byref(st), C.byref(wr), C.byref(nm))
+        self._check(rc, "sfb200_decompress_gzip_file")
+        return st.value, d[:dst_cap].tobytes(), wr.value, nm.value
+
+    def decompress_gzip_file_device(self, src, dst, stream=None):
+        """A gzip file in a uint8 CUDA tensor into another (synchronous) -> (status, written, members)."""
+        import torch
+        assert src.is_cuda and src.dtype == torch.uint8 and src.is_contiguous()
+        assert dst.is_cuda and dst.dtype == torch.uint8 and dst.is_contiguous()
+        if stream is None:
+            stream = torch.cuda.current_stream(src.device).cuda_stream
+        st, wr, nm = C.c_uint8(0), C.c_uint64(0), C.c_uint64(0)
+        f = self.lib.sfb200_decompress_gzip_file_device
+        f.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint8),
+                      C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
+        f.restype = C.c_int
+        rc = f(self.h, src.data_ptr(), src.numel(), dst.data_ptr(), dst.numel(), C.byref(st), C.byref(wr), C.byref(nm),
+               stream)
+        self._check(rc, "sfb200_decompress_gzip_file_device")
+        return st.value, wr.value, nm.value
+
+    def gzip_file_size(self, src: bytes):
+        """-> (sum of ISIZE over the BGZF members the walk reaches, their number, whether they cover the file)"""
+        s = np.frombuffer(src, dtype=np.uint8) if len(src) else np.zeros(1, np.uint8)
+        sz, nm, cp = C.c_uint64(0), C.c_uint64(0), C.c_int(0)
+        f = self.lib.sfb200_gzip_file_size
+        f.argtypes = [C.c_void_p, _u8p, C.c_size_t, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_int)]
+        f.restype = C.c_int
+        self._check(f(self.h, _p(s, _u8p), len(src), C.byref(sz), C.byref(nm), C.byref(cp)), "sfb200_gzip_file_size")
+        return sz.value, nm.value, bool(cp.value)
+
     def decompressed_size_batch_device(self, src, src_off, src_len, status, size, stream=None):
         """Size discovery: status[i] / size[i] of a decode into an unlimited dst; nothing is stored."""
         import torch

@@ -187,6 +187,35 @@ auto decompress_container(std::span<const std::byte> src, std::span<std::byte> d
   return static_cast<ContainerStatus>(status);
 }
 
+auto decompress_gzip_file(std::span<const std::byte> src, std::span<std::byte> dst, std::size_t* written,
+                          std::size_t* members) -> ContainerStatus
+{
+  std::uint8_t status = 0;
+  std::uint64_t wr = 0, nm = 0;
+  const auto lease = pool().borrow();
+  const int rc = sfb200_decompress_gzip_file(lease.get(), reinterpret_cast<const std::uint8_t*>(src.data()), src.size(),
+                                             reinterpret_cast<std::uint8_t*>(dst.data()), dst.size(), &status, &wr, &nm);
+  if (rc != SFB200_RC_OK) return static_cast<ContainerStatus>(infra("sfb200_decompress_gzip_file", rc, lease.get()));
+  if (written) *written = static_cast<std::size_t>(wr);
+  if (members) *members = static_cast<std::size_t>(nm);
+  return static_cast<ContainerStatus>(status);
+}
+
+auto gzip_file_size(std::span<const std::byte> src) -> std::optional<std::size_t>
+{
+  std::uint64_t size = 0;
+  int complete = 0;
+  const auto lease = pool().borrow();
+  const int rc = sfb200_gzip_file_size(lease.get(), reinterpret_cast<const std::uint8_t*>(src.data()), src.size(), &size,
+                                       nullptr, &complete);
+  if (rc != SFB200_RC_OK) {
+    infra("sfb200_gzip_file_size", rc, lease.get());
+    return std::nullopt;
+  }
+  if (!complete) return std::nullopt;
+  return static_cast<std::size_t>(size);
+}
+
 auto decompress_batch(std::span<const std::span<const std::byte>> src,
                       std::span<const std::span<std::byte>> dst, std::span<DecompressStatus> status,
                       std::span<std::size_t> written) -> bool

@@ -12,6 +12,7 @@
 #include <cstdint>
 #include <expected>
 #include <ranges>
+#include <optional>
 #include <span>
 
 namespace starflate {
@@ -90,6 +91,15 @@ enum class ContainerStatus : std::uint8_t
 /// (verified on the device).  `written`, if given, receives the number of bytes produced.
 auto decompress_container(std::span<const std::byte> src, std::span<std::byte> dst, Container container,
                           std::size_t* written = nullptr) -> ContainerStatus;
+/// A gzip FILE: any number of members (BGZF, `cat a.gz b.gz`; RFC 1952 §2.2), their outputs one
+/// behind the other in dst.  Success, or the status of the first failing member in file order
+/// (BadContainer: bytes behind the last member that are neither zero padding nor a member).
+/// `written` receives the bytes of dst that hold output, `members` the members found.
+auto decompress_gzip_file(std::span<const std::byte> src, std::span<std::byte> dst, std::size_t* written = nullptr,
+                          std::size_t* members = nullptr) -> ContainerStatus;
+/// The sum of ISIZE over the BGZF members of src — the dst.size() decompress_gzip_file needs — or
+/// nothing when they do not cover the file (a member without the BGZF field, trailing bytes).
+auto gzip_file_size(std::span<const std::byte> src) -> std::optional<std::size_t>;
 
 // ---- extension: the batched form the GPU is built for ------------------------------------------
 /// Stream i reads src[i] and writes dst[i] (host memory); status[i] / written[i] receive its

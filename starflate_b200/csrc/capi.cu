@@ -9,6 +9,7 @@
 #include "lz_window.cuh"
 #include "lz_jump.cuh"
 #include "container.cuh"
+#include "gzip_file.cuh"
 #include "deflate_compress.cuh"
 
 #include <cstdio>
@@ -97,9 +98,15 @@ struct sfb200_ctx {
   uint32_t* d_lens = nullptr;  // per-resident-lane code-length scratch
   uint32_t* d_bits = nullptr;  // match-head bitmap: 1 bit per dst byte (grown on demand)
   uint64_t d_bits_words = 0;
-  bool count_configured = false, check_configured = false;  // per-device function attributes set
+  bool count_configured = false, check_configured = false, end_configured = false;  // per-device function attributes set
   uint8_t* d_cont = nullptr;  // container route: payload offsets / sizes, kinds, trailer values, written
   uint64_t d_cont_cap = 0;
+  uint8_t* d_gzf = nullptr;   // gzip files (gzip_file.cuh): the walk's step, result, probe metadata, tile counts
+  uint64_t d_gzf_cap = 0;
+  uint8_t* d_gzc = nullptr;   // ... candidates and jump tables
+  uint64_t d_gzc_cap = 0;
+  uint8_t* d_gzm = nullptr;   // ... the member table (kGzfMemberBytes per member)
+  uint64_t d_gzm_n = 0;
   uint8_t* d_find = nullptr;  // single-stream pass 1 (block_finder.cuh): counters, hash table, jobs, candidates
   uint64_t d_find_cap = 0;
   uint8_t* d_jump = nullptr;  // single-stream pass 2 (lz_jump.cuh): pointers, tile flags, round flags
@@ -342,6 +349,9 @@ void sfb200_destroy(sfb200_ctx* ctx)
   cudaFree(ctx->d_jump);
   cudaFree(ctx->d_find);
   cudaFree(ctx->d_cont);
+  cudaFree(ctx->d_gzf);
+  cudaFree(ctx->d_gzc);
+  cudaFree(ctx->d_gzm);
   cudaFree(ctx->d_defer);
   cudaFree(ctx->d_order);
   cudaFree(ctx->d_queue);
@@ -402,11 +412,14 @@ int sfb200_get_launch_info(sfb200_ctx* ctx, sfb200_launch_info* out)
 }  // extern "C"
 
 namespace {
-// chunked input (sfb200_inflate_stream_feed): where each stream starts, and where its decode got to
+// chunked input (sfb200_inflate_stream_feed): where each stream starts, and where its decode got to.
+// start_bit == nullptr: not a continued decode — only `end`, which either route can serve.
 struct Resume {
-  const uint64_t* start_bit;
-  const uint64_t* start_out;
-  uint64_t* blk_end;
+  const uint64_t* start_bit = nullptr;
+  const uint64_t* start_out = nullptr;
+  uint64_t* blk_end = nullptr;
+  bool end = false;  // blk_end[2 i] also receives the end of the final block (huff_lanes_kernel: END;
+                     // huff_stream_kernel: StreamArgs::end_bit)
 };
 
 int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len,
@@ -474,7 +487,8 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
                                        LaneCfg::WARPS * 32 &&
                      dst_bytes / n >= 32768;
   if (const char* e = std::getenv("SFB200_STREAM_MODE")) stream_mode = e[0] == '1' && ctx->stream_ctas_per_sm > 0;
-  if (resume) stream_mode = false;  // (a decode that continues at a block boundary: the lane kernel only)
+  const bool chunked = resume && resume->start_bit;
+  if (chunked) stream_mode = false;  // (a decode that continues at a block boundary: the lane kernel only)
   // One stream: pass 2 works on the whole output at once (lz_jump.cuh) instead of one warp walking it
   // (also a FEW large streams, one after the other: sizes are only known on the device, so "large" is
   //  judged by the room the caller gave them)
@@ -534,6 +548,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
   // (SFB200_GEOMETRY=small) until the hand-over can overlap.
   bool use_small = false;
   if (const char* e = std::getenv("SFB200_GEOMETRY")) use_small = e[0] == 's' && ctx->small_ctas_per_sm > 0;
+  if (resume) use_small = false;  // (the small geometry reports neither resume point nor end)
   if (use_small && n > ctx->d_defer_n) {
     if (ctx->d_defer) SFB_TRY(ctx, cudaFree(ctx->d_defer));
     ctx->d_defer = nullptr;
@@ -732,6 +747,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
       sa.recs = nullptr;
       sa.rec_count = nullptr;
       sa.rec_cap = 0;
+      sa.end_bit = resume && resume->end ? resume->blk_end : nullptr;
       const uint64_t resident =
           static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->stream_ctas_per_sm);
       if (blocks) {
@@ -821,9 +837,17 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
       // (a batch that fits the lanes of the wide geometry takes it: see WideCfg)
       const uint64_t wide_resident =
           static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->wide_ctas_per_sm);
-      if (qmode)
+      if (qmode) {
         sfb::huff_lanes_kernel<LaneCfg, false, true><<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, s1>>>(a);
-      else if (!use_small && n_waves == 1 && wide_resident != 0 && want <= wide_resident)
+      } else if (resume && resume->end) {
+        auto kern = sfb::huff_lanes_kernel<LaneCfg, false, false, true>;
+        if (!ctx->end_configured) {  // (function attributes are per device)
+          SFB_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, LaneCfg::SMEM_BYTES));
+          cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+          ctx->end_configured = true;
+        }
+        kern<<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, s1>>>(a);
+      } else if (!use_small && n_waves == 1 && wide_resident != 0 && want <= wide_resident)
         sfb::huff_lanes_kernel<WideCfg><<<static_cast<unsigned>(want), WideCfg::WARPS * 32, WideCfg::SMEM_BYTES, s1>>>(a);
       else
         sfb::huff_lanes_kernel<LaneCfg><<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, s1>>>(a);
@@ -1710,6 +1734,317 @@ int sfb200_decompressed_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len
   SFB_TRY(ctx, cudaMemcpyAsync(size, d_m + 2, 8, cudaMemcpyDeviceToHost, nullptr));
   SFB_TRY(ctx, cudaMemcpyAsync(status, d_st, 1, cudaMemcpyDeviceToHost, nullptr));
   SFB_TRY(ctx, cudaStreamSynchronize(nullptr));
+  return SFB200_RC_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// gzip files of several members, BGZF at batch speed (gzip_file.cuh).  The members are found on the
+// device: candidates, jump tables, then a walk in steps — one step per run of BGZF members (a whole
+// BGZF file is one step), one more per plain member, whose length is known only after its payload
+// was decoded (the "probe": a single-stream decode over the rest of the file on whichever route the
+// size of dst selects; both report the bit behind the final block).  Then the member table goes
+// through the container batch path, and one kernel reduces the members' results to the file's.
+// (A plain member's probe has only the rest of dst as room, its ISIZE being unknown until its end is
+//  found: one whose payload overruns a corrupt ISIZE AND does not fit the rest of dst reports
+//  DstTooSmall, not SizeMismatch.)
+namespace {
+constexpr uint64_t kGzfMemberBytes = 5 * 8 + 1;    // pos, len, dst off, dst cap, written (u64); status (u8)
+constexpr uint64_t kGzfMaxLen = 0xffffff00ull - 1;  // the batch precondition on src_len / dst_cap
+
+struct GzfResult {
+  uint8_t status = 0;
+  uint64_t written = 0, members = 0, size = 0;
+  bool complete = false;
+};
+
+// room for `need` members in the table, keeping the first `keep`
+int gzf_reserve(sfb200_ctx* ctx, uint64_t need, uint64_t keep, cudaStream_t st)
+{
+  if (need <= ctx->d_gzm_n) return SFB200_RC_OK;
+  const uint64_t cap = need + need / 2 + 64;
+  uint8_t* q = nullptr;
+  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&q), cap * kGzfMemberBytes));
+  if (keep)
+    for (int w = 0; w < 5; ++w)
+      SFB_TRY(ctx, cudaMemcpyAsync(q + w * 8 * cap, ctx->d_gzm + w * 8 * ctx->d_gzm_n, keep * 8, cudaMemcpyDeviceToDevice, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  if (ctx->d_gzm) SFB_TRY(ctx, cudaFree(ctx->d_gzm));
+  ctx->d_gzm = q;
+  ctx->d_gzm_n = cap;
+  return SFB200_RC_OK;
+}
+
+// decode == false: discovery only (sizes of the BGZF members the walk reaches; a plain member ends it)
+int gzip_file_impl(sfb200_ctx* ctx, const uint8_t* src, uint64_t len, uint8_t* dst, uint64_t dst_cap, bool decode,
+                   cudaStream_t st, GzfResult* res)
+{
+  *res = GzfResult{};
+  if (len == 0) {  // an empty file is an empty series of members (Python, gzip(1))
+    res->complete = true;
+    return SFB200_RC_OK;
+  }
+  const uint64_t tile = static_cast<uint64_t>(sfb::GZF_THREADS) * sfb::GZF_BYTES;
+  const uint64_t tiles = (len + (reinterpret_cast<uintptr_t>(src) & 15u) + tile - 1) / tile;
+  // step (128 B) | result (2 x u64) | probe metadata (16 x u64) | tile counts (tiles + 1)
+  int rc = grow(ctx, &ctx->d_gzf, &ctx->d_gzf_cap, 128 + 16 + 128 + 8 * (tiles + 1));
+  if (rc != SFB200_RC_OK) return rc;
+  sfb::GzfArgs a{};
+  a.src = src;
+  a.len = len;
+  a.step = reinterpret_cast<sfb::GzfStep*>(ctx->d_gzf);
+  uint64_t* const d_result = reinterpret_cast<uint64_t*>(ctx->d_gzf + 128);
+  uint64_t* const pm = d_result + 2;
+  a.tile_count = pm + 16;
+  a.dst_cap = decode ? dst_cap : ~0ull;
+  // ---- candidates: count per tile, scan, then (with scratch for exactly that many) scatter ------
+  sfb::gzf_count_kernel<<<static_cast<unsigned>(tiles), sfb::GZF_THREADS, 0, st>>>(a);
+  sfb::gzf_exscan_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(a.tile_count, tiles);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 2;
+  uint64_t m = 0;
+  SFB_TRY(ctx, cudaMemcpyAsync(&m, a.tile_count + tiles, 8, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  if (m >= 0xffffffffull) {  // (candidate indices are 32-bit: only a file of > 8 GiB of header-like bytes gets here)
+    ctx->err = "gzip file: more than 2^32 - 2 BGZF header candidates";
+    return SFB200_RC_BAD_ARGUMENT;
+  }
+  uint32_t tables = 1;  // J_0 .. J_{tables-1}: enough that 2^tables > the longest chain (<= m members)
+  while ((1ull << tables) < m + 1) ++tables;
+  if (const char* e = std::getenv("SFB200_GZIP_CHAIN"))  // (tests: =walk takes the fallback)
+    if (e[0] == 'w') tables = 1;
+  auto cand_bytes = [&](uint32_t t) { return 16 * m + 4 * (m + 1) * static_cast<uint64_t>(t) + 64; };
+  rc = grow(ctx, &ctx->d_gzc, &ctx->d_gzc_cap, cand_bytes(tables));
+  if (rc == SFB200_RC_OUT_OF_MEMORY && tables > 1) {
+    // no room for the jump tables: one thread walks the chain on J_0 instead — slower, same results
+    cudaGetLastError();
+    ctx->err.clear();
+    tables = 1;
+    rc = grow(ctx, &ctx->d_gzc, &ctx->d_gzc_cap, cand_bytes(tables));
+  }
+  if (rc != SFB200_RC_OK) return rc;
+  a.cpos = reinterpret_cast<uint64_t*>(ctx->d_gzc);
+  a.cnext = a.cpos + m;
+  a.jump = reinterpret_cast<uint32_t*>(a.cnext + m);
+  a.m = m;
+  a.n_tables = tables;
+  const unsigned cgrid = static_cast<unsigned>((m + 1 + 255) / 256);
+  sfb::gzf_scatter_kernel<<<static_cast<unsigned>(tiles), sfb::GZF_THREADS, 0, st>>>(a);
+  sfb::gzf_succ_kernel<<<cgrid, 256, 0, st>>>(a);
+  for (uint32_t r = 0; r + 1 < tables; ++r) sfb::gzf_jump_kernel<<<cgrid, 256, 0, st>>>(a, r);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 1 + tables;
+  auto bind_members = [&]() {
+    a.mpos = reinterpret_cast<uint64_t*>(ctx->d_gzm);
+    a.mlen = a.mpos + ctx->d_gzm_n;
+    a.moff = a.mlen + ctx->d_gzm_n;
+    a.mcap = a.moff + ctx->d_gzm_n;
+  };
+  const unsigned skip_grid = static_cast<unsigned>(std::min<uint64_t>(tiles, static_cast<uint64_t>(ctx->sm_count) * 8));
+  sfb::GzfStep h{};
+  auto place = [&](uint64_t first, uint64_t count, uint64_t out_total) -> int {  // one member the host found
+    h = sfb::GzfStep{};
+    h.first = first;
+    h.count = count;
+    h.out_total = out_total;
+    SFB_TRY(ctx, cudaMemcpyAsync(a.step, &h, sizeof h, cudaMemcpyHostToDevice, st));
+    sfb::gzf_place_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(a);
+    SFB_TRY(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    SFB_TRY(ctx, cudaMemcpyAsync(&h, a.step, sizeof h, cudaMemcpyDeviceToHost, st));
+    SFB_TRY(ctx, cudaStreamSynchronize(st));
+    return SFB200_RC_OK;
+  };
+  // ---- the walk ---------------------------------------------------------------------------------
+  uint64_t pos = 0, skip = 0, members = 0, chained = 0, out_total = 0, tail_written = 0;
+  uint32_t tail_status = SFB200_SUCCESS;
+  bool complete = false;
+  for (;;) {
+    if (pos >= len) {
+      complete = true;
+      break;
+    }
+    // room for every member a chain can still bring: each candidate is on at most one chain
+    rc = gzf_reserve(ctx, members + (m - chained) + 1, members, st);
+    if (rc != SFB200_RC_OK) return rc;
+    bind_members();
+    h = sfb::GzfStep{};
+    h.start = pos;
+    h.skip = skip;
+    h.first = members;
+    h.out_total = out_total;
+    h.head = h.next = len;
+    SFB_TRY(ctx, cudaMemcpyAsync(a.step, &h, sizeof h, cudaMemcpyHostToDevice, st));
+    auto* const head = reinterpret_cast<unsigned long long*>(&a.step->head);
+    auto* const next = reinterpret_cast<unsigned long long*>(&a.step->next);
+    sfb::gzf_skip_kernel<<<skip_grid, sfb::GZF_THREADS, 0, st>>>(a, &a.step->start, &a.step->skip, head);
+    if (tables == 1) {
+      sfb::gzf_walk_kernel<<<1, 1, 0, st>>>(a);
+    } else {
+      sfb::gzf_chain_kernel<<<1, 1, 0, st>>>(a);
+      sfb::gzf_expand_kernel<<<cgrid, 256, 0, st>>>(a);
+      ctx->launches += 1;
+    }
+    sfb::gzf_place_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(a);
+    sfb::gzf_skip_kernel<<<skip_grid, sfb::GZF_THREADS, 0, st>>>(a, &a.step->stop, &a.step->count, next);
+    SFB_TRY(ctx, cudaGetLastError());
+    ctx->launches += 4;
+    SFB_TRY(ctx, cudaMemcpyAsync(&h, a.step, sizeof h, cudaMemcpyDeviceToHost, st));
+    SFB_TRY(ctx, cudaStreamSynchronize(st));
+    members += h.count;
+    chained += h.count;
+    out_total = h.out_total;
+    if (h.count) {  // continue behind the members (and the zero padding behind them)
+      pos = h.next;
+      skip = 1;
+      continue;
+    }
+    const uint64_t q = h.head;
+    if (q >= len) {  // only padding is left
+      complete = true;
+      break;
+    }
+    if (!decode) break;  // a member without the BGZF field (or not a member at all) ends discovery
+    // ---- a plain member at q: its header ---------------------------------------------------------
+    uint64_t hp[16] = {q, len - q};
+    SFB_TRY(ctx, cudaMemcpyAsync(pm, hp, 16, cudaMemcpyHostToDevice, st));
+    sfb::ContainerArgs c{};
+    c.src_base = src;
+    c.src_off = pm + 0;
+    c.src_len = pm + 1;
+    c.container = sfb::CT_GZIP;
+    c.n = 1;
+    c.pay_off = pm + 2;
+    c.pay_len = pm + 3;
+    c.kind = reinterpret_cast<uint32_t*>(pm + 4);
+    c.expect = c.kind + 1;
+    c.isize = c.kind + 2;
+    sfb::container_parse_kernel<<<1, 128, 0, st>>>(c);
+    SFB_TRY(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    SFB_TRY(ctx, cudaMemcpyAsync(hp, pm, 6 * 8, cudaMemcpyDeviceToHost, st));
+    SFB_TRY(ctx, cudaStreamSynchronize(st));
+    if (static_cast<uint32_t>(hp[4]) == sfb::CT_BAD) {  // not a gzip member, or its header is cut short
+      tail_status = sfb::ST_BAD_CONTAINER;
+      break;
+    }
+    // ---- its payload, decoded over the rest of the file into its place in dst --------------------
+    const uint64_t pay = hp[2];
+    const uint64_t off = std::min(out_total, dst_cap), room = dst_cap - off;
+    uint64_t pr[14] = {pay, std::min(len - pay, kGzfMaxLen), 0, 0, 0, 0,
+                       0 /* dst_off */, std::min(room, kGzfMaxLen), 0 /* written */, 0, 0, 0, 0 /* blk_end */,
+                       SFB200_ERROR /* status */};
+    SFB_TRY(ctx, cudaMemcpyAsync(pm, pr, sizeof pr, cudaMemcpyHostToDevice, st));
+    Resume rs;  // (not a continued decode: the route is chosen as for any single stream)
+    rs.blk_end = pm + 11;
+    rs.end = true;
+    rc = batch_device_impl(ctx, src, pm + 0, pm + 1, dst + off, pr[7], pm + 6, pm + 7, reinterpret_cast<uint8_t*>(pm + 13),
+                           pm + 8, 1, st, &rs);
+    if (rc != SFB200_RC_OK) return rc;
+    SFB_TRY(ctx, cudaMemcpyAsync(pr, pm, sizeof pr, cudaMemcpyDeviceToHost, st));
+    SFB_TRY(ctx, cudaStreamSynchronize(st));
+    const uint8_t pst = static_cast<uint8_t>(pr[13] & 0xffu);
+    if (pst != SFB200_SUCCESS) {  // the payload's own status; what it produced counts
+      tail_status = pst;
+      tail_written = pr[8];
+      break;
+    }
+    const uint64_t end = pay + (pr[11] + 7) / 8;  // the trailer starts at the byte behind the final block
+    if (end + 8 > len) {                          // the file ends inside the trailer
+      tail_status = sfb::ST_BAD_CONTAINER;
+      break;
+    }
+    rc = gzf_reserve(ctx, members + 1, members, st);
+    if (rc != SFB200_RC_OK) return rc;
+    bind_members();
+    const uint64_t ml[2] = {q, end + 8 - q};
+    SFB_TRY(ctx, cudaMemcpyAsync(a.mpos + members, &ml[0], 8, cudaMemcpyHostToDevice, st));
+    SFB_TRY(ctx, cudaMemcpyAsync(a.mlen + members, &ml[1], 8, cudaMemcpyHostToDevice, st));
+    rc = place(members, 1, out_total);
+    if (rc != SFB200_RC_OK) return rc;
+    out_total = h.out_total;
+    ++members;
+    pos = end + 8;
+    skip = 1;
+  }
+  res->members = members;
+  res->size = out_total;
+  res->complete = complete;
+  if (!decode) return SFB200_RC_OK;
+  // ---- the members side by side, then the file's result ------------------------------------------
+  uint8_t* const m_status = ctx->d_gzm + 40 * ctx->d_gzm_n;
+  uint64_t* const m_written = a.mcap + ctx->d_gzm_n;
+  if (members) {
+    rc = sfb200_decompress_container_batch_device(ctx, SFB200_CONTAINER_GZIP, src, a.mpos, a.mlen, dst, dst_cap, a.moff,
+                                                  a.mcap, m_status, m_written, members, st);
+    if (rc != SFB200_RC_OK) return rc;
+  }
+  sfb::gzf_result_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(a, m_status, m_written, members, tail_status, tail_written,
+                                                              d_result);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 1;
+  uint64_t out[2] = {0, 0};
+  SFB_TRY(ctx, cudaMemcpyAsync(out, d_result, sizeof out, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  res->status = static_cast<uint8_t>(out[0]);
+  res->written = out[1];
+  return SFB200_RC_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int sfb200_decompress_gzip_file_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, uint8_t* dst,
+                                       uint64_t dst_cap, uint8_t* status, uint64_t* written, uint64_t* members,
+                                       void* cuda_stream)
+{
+  if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  GzfResult r;
+  const int rc = gzip_file_impl(ctx, src, src_len, dst, dst_cap, true, static_cast<cudaStream_t>(cuda_stream), &r);
+  if (rc != SFB200_RC_OK) return rc;
+  *status = r.status;
+  if (written) *written = r.written;
+  if (members) *members = r.members;
+  return SFB200_RC_OK;
+}
+
+int sfb200_decompress_gzip_file(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* dst, size_t dst_cap,
+                                uint8_t* status, uint64_t* written, uint64_t* members)
+{
+  if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  int rc = grow(ctx, &ctx->d_src, &ctx->d_src_cap, static_cast<uint64_t>(src_len) + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  rc = grow(ctx, &ctx->d_dst, &ctx->d_dst_cap, static_cast<uint64_t>(dst_cap) + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  if (src_len) SFB_TRY(ctx, cudaMemcpy(ctx->d_src, src, src_len, cudaMemcpyHostToDevice));
+  GzfResult r;
+  rc = gzip_file_impl(ctx, ctx->d_src, src_len, ctx->d_dst, dst_cap, true, nullptr, &r);
+  if (rc != SFB200_RC_OK) return rc;
+  if (r.written > dst_cap) return SFB200_RC_CUDA_ERROR;  // (cannot happen)
+  if (r.written) SFB_TRY(ctx, cudaMemcpy(dst, ctx->d_dst, r.written, cudaMemcpyDeviceToHost));  // only what was produced
+  *status = r.status;
+  if (written) *written = r.written;
+  if (members) *members = r.members;
+  return SFB200_RC_OK;
+}
+
+int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint64_t* size, uint64_t* members,
+                          int* complete)
+{
+  if (!ctx || !size || (!src && src_len)) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  const int rc0 = grow(ctx, &ctx->d_src, &ctx->d_src_cap, static_cast<uint64_t>(src_len) + 64);
+  if (rc0 != SFB200_RC_OK) return rc0;
+  if (src_len) SFB_TRY(ctx, cudaMemcpy(ctx->d_src, src, src_len, cudaMemcpyHostToDevice));
+  GzfResult r;
+  const int rc = gzip_file_impl(ctx, ctx->d_src, src_len, nullptr, 0, false, nullptr, &r);
+  if (rc != SFB200_RC_OK) return rc;
+  *size = r.size;
+  if (members) *members = r.members;
+  if (complete) *complete = r.complete ? 1 : 0;
   return SFB200_RC_OK;
 }
 

@@ -11,7 +11,9 @@
 //
 // One member per stream, and the trailer is taken from the END of the stream's bytes: trailing
 // bytes after the member (or a second gzip member) are not supported and show up as a checksum
-// mismatch.  A preset dictionary (zlib FDICT) is not supported.
+// mismatch — a file of several gzip members (BGZF, `cat a.gz b.gz`) goes through
+// sfb200_decompress_gzip_file* (gzip_file.cuh), which finds the members and hands them to this path
+// one stream each.  A preset dictionary (zlib FDICT) is not supported.
 #pragma once
 
 #include <cstdint>

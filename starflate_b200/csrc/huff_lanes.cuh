@@ -238,7 +238,10 @@ constexpr uint32_t LANES = 32;
 // COUNT = true is the size-discovery mode (SURVEY.md §8 f2: the reference returns no size and asks
 // the caller to know it): the same decode with a writer that stores nothing and no capacity
 // limit; status[i] / written[i] are what a decode into a large enough dst would return.
-template <class C, bool COUNT = false, bool QUEUE = false>   // QUEUE: publish segments to a pass 2 that runs beside (QueueArgs)
+// END = true (a resumed decode, blk_end given): after the final block blk_end receives the bit behind
+// its end-of-block code — where a gzip member's trailer starts (gzip_file.cuh) — and the output
+// position.  A template parameter, so that the other instantiations keep their registers.
+template <class C, bool COUNT = false, bool QUEUE = false, bool END = false>   // QUEUE: publish segments to a pass 2 that runs beside (QueueArgs)
 __global__ void __launch_bounds__(C::WARPS * 32, C::CTAS)
 huff_lanes_kernel(const BatchArgs a)
 {
@@ -560,6 +563,10 @@ huff_lanes_kernel(const BatchArgs a)
       }
       ow.emit(p_chunk, p_n, p_skip, p_mt, p_hoff);  // drain the pipeline
       if (state == S_DONE && live) {
+        if (END && status == ST_SUCCESS) {  // (see END above)
+          a.blk_end[2 * idx] = static_cast<uint64_t>(br.bitpos());
+          a.blk_end[2 * idx + 1] = ow.written();
+        }
         ow.flush_tail();
         a.status[idx] = static_cast<uint8_t>(status);
         a.written[idx] = ow.written();

@@ -70,6 +70,10 @@ struct StreamArgs {
   WinRec* recs;         // window records: written in mode 1, read in mode 2
   uint32_t* rec_count;  // zeroed
   uint32_t rec_cap;
+  // (may be null) a stream that ends with Success: end_bit[2 * i] = the bit behind its final block's
+  // end-of-block code — where a gzip member's trailer starts (gzip_file.cuh); the layout of
+  // BatchArgs::blk_end
+  uint64_t* end_bit;
 };
 
 struct Tok {
@@ -513,6 +517,7 @@ __global__ void __launch_bounds__(32) huff_stream_kernel(const StreamArgs a)
       } else if (!one_block) {
         a.status[idx] = static_cast<uint8_t>(status);
         a.written[idx] = outpos;
+        if (a.end_bit != nullptr && status == ST_SUCCESS) a.end_bit[2 * idx] = bitpos;
       }
     }
   }
