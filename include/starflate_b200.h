@@ -254,6 +254,52 @@ int sfb200_decompress_gzip_file(sfb200_ctx* ctx, const uint8_t* src, size_t src_
 int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint64_t* size, uint64_t* members,
                           int* complete);
 
+/* COMPRESSION to zlib (RFC 1950) and gzip (RFC 1952): sfb200_compress_batch_device's streams with
+ * header and trailer, the Adler-32 / CRC-32 (and ISIZE) of each stream's SOURCE bytes computed on the
+ * device.  zlib: 78 9c, payload, Adler-32 big endian.  gzip: 1f 8b 08 00, MTIME 0, XFL 0, OS 255
+ * (the first 10 bytes Python's gzip.GzipFile writes at level 6 with mtime=0), payload, CRC-32 and ISIZE little
+ * endian.  The payload is what sfb200_compress_batch_device writes for the stream.  `container`:
+ * RAW (exactly sfb200_compress_batch_device), ZLIB or GZIP; AUTO is SFB200_RC_BAD_ARGUMENT.
+ * Statuses as there: SFB200_DST_TOO_SMALL with written[i] = 0 when the framed stream does not fit
+ * dst_cap[i] (sfb200_compress_container_bound(container, src_len) always does), SFB200_ERROR for
+ * src_len[i] >= 2^32 - 256.  Bytes of the dst region past written[i] may have been used as scratch.
+ * src is read twice (the compressor, then the checksum: 16-byte loads inside the same aligned 16-byte
+ * blocks as the stream's bytes).  The context keeps 16 bytes per stream of scratch.  All arrays are
+ * DEVICE pointers; asynchronous on `cuda_stream`. */
+uint64_t sfb200_compress_container_bound(int container, uint64_t src_len);
+int sfb200_compress_container_batch_device(sfb200_ctx* ctx, int container, const uint8_t* src_base,
+                                           const uint64_t* src_off, const uint64_t* src_len, uint8_t* dst_base,
+                                           const uint64_t* dst_off, const uint64_t* dst_cap, uint8_t* status,
+                                           uint64_t* written, uint64_t n, void* cuda_stream);
+/* One stream in host memory. */
+int sfb200_compress_container(sfb200_ctx* ctx, int container, const uint8_t* src, size_t src_len, uint8_t* dst,
+                              size_t dst_cap, uint8_t* status, uint64_t* written);
+
+/* COMPRESSION of one buffer to a BGZF file: the input is cut into pieces of 65 280 bytes (bgzip's), every
+ * piece compressed by the batch compressor as one BGZF member (header 1f 8b 08 04, MTIME 0, XFL 0,
+ * OS 255, XLEN 6, subfield 'B' 'C' SLEN 2 BSIZE = member length - 1; payload; CRC-32 and ISIZE),
+ * the pieces side by side, then the 28-byte EOF marker of the SAM/BAM specification.  The output
+ * decodes with gzip(1), Python's gzip, htslib and sfb200_decompress_gzip_file*.  Any src_len,
+ * 4 GiB and more included.
+ *   *status   Success; SFB200_DST_TOO_SMALL when the file does not fit dst_cap (never with dst_cap >=
+ *             sfb200_compress_bgzf_bound(src_len)): *written = 0, no byte past dst_cap is touched and
+ *             the bytes before it are unspecified.
+ *   *written  (may be NULL) the file's size.   *members  (may be NULL) members written, the EOF marker
+ *             included (what sfb200_decompress_gzip_file* reports for the file); 0 on failure.
+ * `src` and `dst` are DEVICE pointers, the three results HOST pointers; synchronous on `cuda_stream`.
+ * Scratch kept in the context: 64 KiB + 41 bytes per piece of a round.  A round holds at most
+ * SFB200_BGZF_SCRATCH_MB (default 8192) MiB of pieces' scratch; larger inputs take several rounds,
+ * with a constant number of kernel launches each and no host round trip between them.  src is read
+ * twice (the compressor, then the CRC-32), in 16-byte loads inside the aligned 16-byte blocks that
+ * hold its bytes; dst is written once. */
+uint64_t sfb200_compress_bgzf_bound(uint64_t src_len);
+int sfb200_compress_bgzf_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, uint8_t* dst, uint64_t dst_cap,
+                                uint8_t* status, uint64_t* written, uint64_t* members, void* cuda_stream);
+/* The same with HOST buffers: input and output are staged on the device whole; only the bytes written
+ * are copied back. */
+int sfb200_compress_bgzf(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* dst, size_t dst_cap,
+                         uint8_t* status, uint64_t* written, uint64_t* members);
+
 /* Position-weighted 64-bit checksum of each stream's output region [0, len[i]) computed on the
  * device (used by tests/bench to verify multi-GiB outputs without a device->host copy):
  *   sum_j (byte_j + 1) * (0x9E3779B97F4A7C15 * (j + 1) | 1)   mod 2^64. */

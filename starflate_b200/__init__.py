@@ -319,6 +319,84 @@ class Context:
         self._check(f(self.h, _p(s, _u8p), len(src), _p(d, _u8p), dst_cap, C.byref(st), C.byref(wr)), "sfb200_compress")
         return st.value, d[:wr.value].tobytes()
 
+    def compress_container_bound(self, container, n: int) -> int:
+        f = self.lib.sfb200_compress_container_bound
+        f.argtypes = [C.c_int, C.c_uint64]
+        f.restype = C.c_uint64
+        return int(f(container, n))
+
+    def compress_bgzf_bound(self, n: int) -> int:
+        f = self.lib.sfb200_compress_bgzf_bound
+        f.argtypes = [C.c_uint64]
+        f.restype = C.c_uint64
+        return int(f(n))
+
+    def compress_container_batch_device(self, container, src, src_off, src_len, dst, dst_off, dst_cap, status, written,
+                                        stream=None):
+        """Batched compression to zlib / gzip (or RAW), checksums of the sources computed on the device
+        (sfb200_compress_container_batch_device); torch CUDA tensors."""
+        import torch
+        n = src_off.numel()
+        for t in (src_off, src_len, dst_off, dst_cap, written):
+            assert t.is_cuda and t.dtype == torch.int64 and t.is_contiguous() and t.numel() == n
+        assert src.is_cuda and src.dtype == torch.uint8 and dst.is_cuda and dst.dtype == torch.uint8
+        assert status.is_cuda and status.dtype == torch.uint8 and status.numel() == n
+        if stream is None:
+            stream = torch.cuda.current_stream(src.device).cuda_stream
+        f = self.lib.sfb200_compress_container_batch_device
+        f.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8 + [C.c_uint64, C.c_void_p]
+        f.restype = C.c_int
+        rc = f(self.h, container, src.data_ptr(), src_off.data_ptr(), src_len.data_ptr(), dst.data_ptr(),
+               dst_off.data_ptr(), dst_cap.data_ptr(), status.data_ptr(), written.data_ptr(), n, stream)
+        self._check(rc, "sfb200_compress_container_batch_device")
+
+    def compress_container(self, container, src: bytes, dst_cap: int = -1):
+        """One stream in host memory -> (status, zlib / gzip / raw-DEFLATE bytes)."""
+        if dst_cap < 0:
+            dst_cap = self.compress_container_bound(container, len(src))
+        s = np.frombuffer(src, dtype=np.uint8) if len(src) else np.zeros(1, np.uint8)
+        d = np.zeros(max(dst_cap, 1), dtype=np.uint8)
+        st, wr = C.c_uint8(0), C.c_uint64(0)
+        f = self.lib.sfb200_compress_container
+        f.argtypes = [C.c_void_p, C.c_int, _u8p, C.c_size_t, _u8p, C.c_size_t, C.POINTER(C.c_uint8),
+                      C.POINTER(C.c_uint64)]
+        f.restype = C.c_int
+        self._check(f(self.h, container, _p(s, _u8p), len(src), _p(d, _u8p), dst_cap, C.byref(st), C.byref(wr)),
+                    "sfb200_compress_container")
+        return st.value, d[:wr.value].tobytes()
+
+    def compress_bgzf(self, src: bytes, dst_cap: int = -1):
+        """One buffer in host memory -> (status, BGZF file bytes, members incl. the EOF marker)."""
+        if dst_cap < 0:
+            dst_cap = self.compress_bgzf_bound(len(src))
+        s = np.frombuffer(src, dtype=np.uint8) if len(src) else np.zeros(1, np.uint8)
+        d = np.zeros(max(dst_cap, 1), dtype=np.uint8)
+        st, wr, nm = C.c_uint8(0), C.c_uint64(0), C.c_uint64(0)
+        f = self.lib.sfb200_compress_bgzf
+        f.argtypes = [C.c_void_p, _u8p, C.c_size_t, _u8p, C.c_size_t, C.POINTER(C.c_uint8), C.POINTER(C.c_uint64),
+                      C.POINTER(C.c_uint64)]
+        f.restype = C.c_int
+        rc = f(self.h, _p(s, _u8p), len(src), _p(d, _u8p), dst_cap, C.byref(st), C.byref(wr), C.byref(nm))
+        self._check(rc, "sfb200_compress_bgzf")
+        return st.value, d[:wr.value].tobytes(), nm.value
+
+    def compress_bgzf_device(self, src, dst, stream=None):
+        """A uint8 CUDA tensor as a BGZF file into another (synchronous) -> (status, written, members)."""
+        import torch
+        assert src.is_cuda and src.dtype == torch.uint8 and src.is_contiguous()
+        assert dst.is_cuda and dst.dtype == torch.uint8 and dst.is_contiguous()
+        if stream is None:
+            stream = torch.cuda.current_stream(src.device).cuda_stream
+        st, wr, nm = C.c_uint8(0), C.c_uint64(0), C.c_uint64(0)
+        f = self.lib.sfb200_compress_bgzf_device
+        f.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint8),
+                      C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
+        f.restype = C.c_int
+        rc = f(self.h, src.data_ptr(), src.numel(), dst.data_ptr(), dst.numel(), C.byref(st), C.byref(wr), C.byref(nm),
+               stream)
+        self._check(rc, "sfb200_compress_bgzf_device")
+        return st.value, wr.value, nm.value
+
     def inflate_stream(self) -> "InflateStream":
         """Chunked input for one stream (sfb200_inflate_stream_*)."""
         return InflateStream(self)

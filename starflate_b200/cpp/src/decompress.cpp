@@ -216,6 +216,45 @@ auto gzip_file_size(std::span<const std::byte> src) -> std::optional<std::size_t
   return static_cast<std::size_t>(size);
 }
 
+auto compress_container(std::span<const std::byte> src, std::span<std::byte> dst, Container container,
+                        std::size_t* written) -> ContainerStatus
+{
+  if (container == Container::Auto) return ContainerStatus::Error;
+  std::uint8_t status = 0;
+  std::uint64_t wr = 0;
+  const auto lease = pool().borrow();
+  const int rc = sfb200_compress_container(lease.get(), static_cast<int>(container),
+                                           reinterpret_cast<const std::uint8_t*>(src.data()), src.size(),
+                                           reinterpret_cast<std::uint8_t*>(dst.data()), dst.size(), &status, &wr);
+  if (rc != SFB200_RC_OK) return static_cast<ContainerStatus>(infra("sfb200_compress_container", rc, lease.get()));
+  if (written) *written = static_cast<std::size_t>(wr);
+  return static_cast<ContainerStatus>(status);
+}
+
+auto compress_bgzf(std::span<const std::byte> src, std::span<std::byte> dst, std::size_t* written,
+                   std::size_t* members) -> ContainerStatus
+{
+  std::uint8_t status = 0;
+  std::uint64_t wr = 0, nm = 0;
+  const auto lease = pool().borrow();
+  const int rc = sfb200_compress_bgzf(lease.get(), reinterpret_cast<const std::uint8_t*>(src.data()), src.size(),
+                                      reinterpret_cast<std::uint8_t*>(dst.data()), dst.size(), &status, &wr, &nm);
+  if (rc != SFB200_RC_OK) return static_cast<ContainerStatus>(infra("sfb200_compress_bgzf", rc, lease.get()));
+  if (written) *written = static_cast<std::size_t>(wr);
+  if (members) *members = static_cast<std::size_t>(nm);
+  return static_cast<ContainerStatus>(status);
+}
+
+auto compress_bound(Container container, std::size_t src_size) -> std::size_t
+{
+  return static_cast<std::size_t>(sfb200_compress_container_bound(static_cast<int>(container), src_size));
+}
+
+auto compress_bgzf_bound(std::size_t src_size) -> std::size_t
+{
+  return static_cast<std::size_t>(sfb200_compress_bgzf_bound(src_size));
+}
+
 auto decompress_batch(std::span<const std::span<const std::byte>> src,
                       std::span<const std::span<std::byte>> dst, std::span<DecompressStatus> status,
                       std::span<std::size_t> written) -> bool

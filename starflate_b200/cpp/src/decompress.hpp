@@ -101,6 +101,21 @@ auto decompress_gzip_file(std::span<const std::byte> src, std::span<std::byte> d
 /// nothing when they do not cover the file (a member without the BGZF field, trailing bytes).
 auto gzip_file_size(std::span<const std::byte> src) -> std::optional<std::size_t>;
 
+// ---- extension: compression to raw DEFLATE, zlib, gzip and BGZF ---------------------------------
+/// Compresses src into dst as one raw-DEFLATE, zlib or gzip stream (Auto is Error), the checksum of
+/// src computed on the device.  Success, or DstTooSmall (nothing written) when it does not fit;
+/// dst.size() >= compress_bound(container, src.size()) always fits.  `written` receives the size.
+auto compress_container(std::span<const std::byte> src, std::span<std::byte> dst, Container container,
+                        std::size_t* written = nullptr) -> ContainerStatus;
+/// Compresses src into dst as a BGZF file (pieces of 65 280 bytes compressed side by side, then the
+/// EOF marker); it decodes with decompress_gzip_file, gzip(1) and htslib.  `members` receives the
+/// members written, the EOF marker included.
+auto compress_bgzf(std::span<const std::byte> src, std::span<std::byte> dst, std::size_t* written = nullptr,
+                   std::size_t* members = nullptr) -> ContainerStatus;
+/// The dst.size() that always holds the output (0 for Auto).
+auto compress_bound(Container container, std::size_t src_size) -> std::size_t;
+auto compress_bgzf_bound(std::size_t src_size) -> std::size_t;
+
 // ---- extension: the batched form the GPU is built for ------------------------------------------
 /// Stream i reads src[i] and writes dst[i] (host memory); status[i] / written[i] receive its
 /// result.  One call = one H2D copy, two kernels, one D2H copy.  Returns false on an

@@ -11,6 +11,7 @@
 #include "container.cuh"
 #include "gzip_file.cuh"
 #include "deflate_compress.cuh"
+#include "container_write.cuh"
 
 #include <cstdio>
 #include <cstdlib>
@@ -107,6 +108,11 @@ struct sfb200_ctx {
   uint64_t d_gzc_cap = 0;
   uint8_t* d_gzm = nullptr;   // ... the member table (kGzfMemberBytes per member)
   uint64_t d_gzm_n = 0;
+  bool seal_configured = false;
+  uint8_t* d_wrap = nullptr;  // writing containers (container_write.cuh): the payloads' offsets and capacities
+  uint64_t d_wrap_cap = 0;
+  uint8_t* d_bgzf = nullptr;  // writing BGZF: a round's scratch slots, the compressor's arrays, the call's state
+  uint64_t d_bgzf_cap = 0;
   uint8_t* d_find = nullptr;  // single-stream pass 1 (block_finder.cuh): counters, hash table, jobs, candidates
   uint64_t d_find_cap = 0;
   uint8_t* d_jump = nullptr;  // single-stream pass 2 (lz_jump.cuh): pointers, tile flags, round flags
@@ -352,6 +358,8 @@ void sfb200_destroy(sfb200_ctx* ctx)
   cudaFree(ctx->d_gzf);
   cudaFree(ctx->d_gzc);
   cudaFree(ctx->d_gzm);
+  cudaFree(ctx->d_wrap);
+  cudaFree(ctx->d_bgzf);
   cudaFree(ctx->d_defer);
   cudaFree(ctx->d_order);
   cudaFree(ctx->d_queue);
@@ -2045,6 +2053,203 @@ int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, u
   *size = r.size;
   if (members) *members = r.members;
   if (complete) *complete = r.complete ? 1 : 0;
+  return SFB200_RC_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// Writing zlib, gzip and BGZF (container_write.cuh): the compressor writes the payloads, the seal
+// kernel adds header and trailer with the checksum of the source bytes, all on the device.
+namespace {
+int seal_launch(sfb200_ctx* ctx, const sfb::SealArgs& s, cudaStream_t st)
+{
+  if (!ctx->seal_configured) {  // (function attributes are per device)
+    SFB_TRY(ctx, cudaFuncSetAttribute(sfb::container_seal_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      sfb::CHECK_SMEM_BYTES));
+    ctx->seal_configured = true;
+  }
+  const uint64_t want = (s.n * 32 + sfb::CHECK_THREADS - 1) / sfb::CHECK_THREADS;
+  const uint64_t resident = static_cast<uint64_t>(ctx->sm_count);  // (one block per SM: 128 KiB of tables)
+  sfb::container_seal_kernel<<<static_cast<unsigned>(want < resident ? want : resident), sfb::CHECK_THREADS,
+                               sfb::CHECK_SMEM_BYTES, st>>>(s);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 1;
+  return SFB200_RC_OK;
+}
+}  // namespace
+
+extern "C" {
+
+uint64_t sfb200_compress_container_bound(int container, uint64_t src_len)
+{
+  const uint64_t raw = sfb200_compress_bound(src_len);
+  switch (container) {
+    case SFB200_CONTAINER_RAW: return raw;
+    case SFB200_CONTAINER_ZLIB: return raw + 6;
+    case SFB200_CONTAINER_GZIP: return raw + 18;
+    default: return 0;
+  }
+}
+
+int sfb200_compress_container_batch_device(sfb200_ctx* ctx, int container, const uint8_t* src_base,
+                                           const uint64_t* src_off, const uint64_t* src_len, uint8_t* dst_base,
+                                           const uint64_t* dst_off, const uint64_t* dst_cap, uint8_t* status,
+                                           uint64_t* written, uint64_t n, void* cuda_stream)
+{
+  if (!ctx || container < SFB200_CONTAINER_RAW || container > SFB200_CONTAINER_GZIP) return SFB200_RC_BAD_ARGUMENT;
+  if (container == SFB200_CONTAINER_RAW)
+    return sfb200_compress_batch_device(ctx, src_base, src_off, src_len, dst_base, dst_off, dst_cap, status, written, n,
+                                        cuda_stream);
+  if (n == 0) return SFB200_RC_OK;
+  if (!src_off || !src_len || !dst_off || !dst_cap || !status || !written) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  int rc = grow(ctx, &ctx->d_wrap, &ctx->d_wrap_cap, n * 16 + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  uint64_t* const pay_off = reinterpret_cast<uint64_t*>(ctx->d_wrap);
+  uint64_t* const pay_cap = pay_off + n;
+  sfb::container_frame_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(
+      static_cast<uint32_t>(container), dst_off, dst_cap, pay_off, pay_cap, n);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 1;
+  rc = sfb200_compress_batch_device(ctx, src_base, src_off, src_len, dst_base, pay_off, pay_cap, status, written, n,
+                                    cuda_stream);
+  if (rc != SFB200_RC_OK) return rc;
+  sfb::SealArgs s{};
+  s.src_base = src_base;
+  s.src_off = src_off;
+  s.src_len = src_len;
+  s.dst_base = dst_base;
+  s.dst_off = dst_off;
+  s.dst_cap = dst_cap;
+  s.status = status;
+  s.written = written;
+  s.n = n;
+  s.container = static_cast<uint32_t>(container);
+  return seal_launch(ctx, s, st);
+}
+
+int sfb200_compress_container(sfb200_ctx* ctx, int container, const uint8_t* src, size_t src_len, uint8_t* dst,
+                              size_t dst_cap, uint8_t* status, uint64_t* written)
+{
+  if (!ctx || !status || !written || (src_len && !src) || (dst_cap && !dst)) return SFB200_RC_BAD_ARGUMENT;
+  if (container < SFB200_CONTAINER_RAW || container > SFB200_CONTAINER_GZIP) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  uint8_t* buf = nullptr;
+  const uint64_t in_pad = (static_cast<uint64_t>(src_len) + 255) & ~255ull;
+  const uint64_t total = in_pad + dst_cap + 256 + 64;
+  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&buf), total));
+  auto done = [&](int rc) {
+    cudaFree(buf);
+    return rc;
+  };
+  uint64_t h[6] = {0, src_len, 0, dst_cap, 0, 0};
+  uint64_t* meta = reinterpret_cast<uint64_t*>(buf + in_pad + ((dst_cap + 255) & ~255ull));
+  if (src_len && cudaMemcpy(buf, src, src_len, cudaMemcpyHostToDevice) != cudaSuccess)
+    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(src)"));
+  if (cudaMemcpy(meta, h, sizeof h, cudaMemcpyHostToDevice) != cudaSuccess)
+    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(meta)"));
+  int rc = sfb200_compress_container_batch_device(ctx, container, buf, meta + 0, meta + 1, buf + in_pad, meta + 2,
+                                                  meta + 3, reinterpret_cast<uint8_t*>(meta + 5), meta + 4, 1, nullptr);
+  if (rc != SFB200_RC_OK) return done(rc);
+  if (cudaMemcpy(h, meta, sizeof h, cudaMemcpyDeviceToHost) != cudaSuccess)
+    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(meta back)"));
+  *status = static_cast<uint8_t>(h[5] & 0xffu);
+  *written = h[4];
+  if (h[4] && cudaMemcpy(dst, buf + in_pad, h[4], cudaMemcpyDeviceToHost) != cudaSuccess)
+    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(dst)"));
+  return done(SFB200_RC_OK);
+}
+
+uint64_t sfb200_compress_bgzf_bound(uint64_t src_len)
+{
+  return (src_len + sfb::BGZF_PIECE - 1) / sfb::BGZF_PIECE * (sfb::BGZF_PIECE + 5 + sfb::BGZF_FRAME) + sfb::BGZF_EOF_BYTES;
+}
+
+int sfb200_compress_bgzf_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, uint8_t* dst, uint64_t dst_cap,
+                                uint8_t* status, uint64_t* written, uint64_t* members, void* cuda_stream)
+{
+  if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  const uint64_t pieces = (src_len + sfb::BGZF_PIECE - 1) / sfb::BGZF_PIECE;
+  uint64_t budget_mb = 8192;  // scratch of a round: 64 KiB per piece (SFB200_BGZF_SCRATCH_MB)
+  if (const char* e = std::getenv("SFB200_BGZF_SCRATCH_MB")) budget_mb = std::max<long long>(1, std::atoll(e));
+  const uint64_t slots = std::max<uint64_t>(1, (budget_mb << 20) / sfb::BGZF_SLOT);
+  const uint64_t r = std::max<uint64_t>(1, std::min(pieces, slots));
+  // slots (r x 64 KiB) | src_off, src_len, dst_off, dst_cap (r x u64 each) | written (r + 1) | state (4) | status (r)
+  const uint64_t meta_at = r * sfb::BGZF_SLOT;
+  int rc = grow(ctx, &ctx->d_bgzf, &ctx->d_bgzf_cap, meta_at + 8 * (5 * r + 5) + r + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  uint8_t* const slot = ctx->d_bgzf;
+  uint64_t* const so = reinterpret_cast<uint64_t*>(ctx->d_bgzf + meta_at);
+  uint64_t* const sl = so + r;
+  uint64_t* const dof = sl + r;
+  uint64_t* const dc = dof + r;
+  uint64_t* const wr = dc + r;
+  uint64_t* const state = wr + r + 1;
+  uint8_t* const pst = reinterpret_cast<uint8_t*>(state + 4);
+  SFB_TRY(ctx, cudaMemsetAsync(state, 0, 4 * sizeof(uint64_t), st));
+  sfb::SealArgs s{};
+  s.src_base = src;
+  s.src_off = so;
+  s.src_len = sl;
+  s.dst_base = dst;
+  s.status = pst;
+  s.written = wr;
+  s.container = sfb::CT_BGZF;
+  s.slots = slot;
+  s.state = state;
+  s.dst_bytes = dst_cap;
+  uint64_t first = 0;
+  do {  // one round per r pieces (an empty input: one round without pieces, for the EOF marker)
+    const uint64_t n = std::min(r, pieces - first);
+    const bool last = first + n >= pieces;
+    if (n) {
+      sfb::bgzf_split_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(src_len, sfb::BGZF_PIECE, first, n,
+                                                                                   so, sl, dof, dc);
+      SFB_TRY(ctx, cudaGetLastError());
+      ctx->launches += 1;
+      rc = sfb200_compress_batch_device(ctx, src, so, sl, slot, dof, dc, pst, wr, n, st);
+      if (rc != SFB200_RC_OK) return rc;
+      sfb::gzf_exscan_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(wr, n);
+      SFB_TRY(ctx, cudaGetLastError());
+      ctx->launches += 1;
+      s.n = n;
+      rc = seal_launch(ctx, s, st);
+      if (rc != SFB200_RC_OK) return rc;
+    }
+    sfb::bgzf_advance_kernel<<<1, 1, 0, st>>>(state, wr, n, dst, dst_cap, last ? 1 : 0);
+    SFB_TRY(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    first += n;
+  } while (first < pieces);
+  uint64_t res[2] = {0, 0};
+  SFB_TRY(ctx, cudaMemcpyAsync(res, state + 1, sizeof res, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  *status = static_cast<uint8_t>(res[0]);
+  if (written) *written = res[1];
+  if (members) *members = res[0] == SFB200_SUCCESS ? pieces + 1 : 0;
+  return SFB200_RC_OK;
+}
+
+int sfb200_compress_bgzf(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* dst, size_t dst_cap,
+                         uint8_t* status, uint64_t* written, uint64_t* members)
+{
+  if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  int rc = grow(ctx, &ctx->d_src, &ctx->d_src_cap, static_cast<uint64_t>(src_len) + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  rc = grow(ctx, &ctx->d_dst, &ctx->d_dst_cap, static_cast<uint64_t>(dst_cap) + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  if (src_len) SFB_TRY(ctx, cudaMemcpy(ctx->d_src, src, src_len, cudaMemcpyHostToDevice));
+  uint64_t wr = 0;
+  rc = sfb200_compress_bgzf_device(ctx, ctx->d_src, src_len, ctx->d_dst, dst_cap, status, &wr, members, nullptr);
+  if (rc != SFB200_RC_OK) return rc;
+  if (wr > dst_cap) return SFB200_RC_CUDA_ERROR;  // (cannot happen)
+  if (wr) SFB_TRY(ctx, cudaMemcpy(dst, ctx->d_dst, wr, cudaMemcpyDeviceToHost));  // only what was written
+  if (written) *written = wr;
   return SFB200_RC_OK;
 }
 

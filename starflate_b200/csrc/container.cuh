@@ -153,22 +153,123 @@ __global__ void container_parse_kernel(const ContainerArgs a)
 constexpr int CHECK_THREADS = 1024;
 constexpr int CHECK_SMEM_BYTES = 4 * 256 * 32 * 4;  // the per-lane CRC tables
 
-__global__ void __launch_bounds__(CHECK_THREADS) container_check_kernel(const ContainerArgs a)
+// CRC-32, four bytes per step: T(k, b) = CRC of byte b followed by k zero bytes.  The four tables
+// are kept once PER LANE (entry (k, b) of lane l at word (k * 256 + b) * 32 + l: bank = lane), so
+// the 32 lanes' look-ups at 32 unrelated indices never meet in a bank: 128 KiB, one block per SM.
+// Every thread of the block calls it; a __syncthreads() must follow before the tables are read.
+__device__ __forceinline__ void crc_tables_init(uint32_t* crc_tab)
 {
-  constexpr unsigned FULL = 0xffffffffu;
-  // CRC-32, four bytes per step: T(k, b) = CRC of byte b followed by k zero bytes.  The four tables
-  // are kept once PER LANE (entry (k, b) of lane l at word (k * 256 + b) * 32 + l: bank = lane), so
-  // the 32 lanes' look-ups at 32 unrelated indices never meet in a bank: 128 KiB, one block per SM.
-#ifdef SFB_CPU_EMU
-  uint32_t* const crc_tab = SFB_EMU_CRC_SMEM;  // tests/cpu_emu: the block's shared memory
-#else
-  extern __shared__ uint32_t crc_tab[];
-#endif
   for (uint32_t e = threadIdx.x; e < 1024u; e += blockDim.x) {
     uint32_t c = crc_byte_table_entry(e & 255u);
     for (uint32_t k = 0; k < (e >> 8); ++k) c = crc_byte_table_entry(c & 0xffu) ^ (c >> 8);
     for (uint32_t l = 0; l < 32u; ++l) crc_tab[e * 32u + l] = c;
   }
+}
+
+// Adler-32 (RFC 1950 §8.2) of d[0 .. n) by the whole warp; every lane returns it.
+// s1 = 1 + sum b_j, s2 = n + sum (n - j) b_j, both mod 65521 (a lane takes aligned words, 128 bytes
+// per warp and step; the weight n - j is kept modulo 65521 by subtracting 128 per step, so the inner
+// loop has no division)
+__device__ __forceinline__ uint32_t warp_adler32(const uint8_t* d, uint64_t n, uint32_t lane)
+{
+  constexpr unsigned FULL = 0xffffffffu;
+  uint64_t s1 = 0, s2 = 0;
+  const uint32_t mis = static_cast<uint32_t>(reinterpret_cast<uintptr_t>(d)) & 3u;
+  const uint64_t head = mis ? (4u - mis < n ? 4u - mis : n) : 0u;  // bytes before the first aligned word
+  const uint64_t words = (n - head) >> 2;
+  const uint64_t tail0 = head + 4u * words;
+  if (lane == 0) {  // the few bytes around the aligned part
+    for (uint64_t j = 0; j < head; ++j) {
+      s1 += d[j];
+      s2 += ((n - j) % 65521u) * d[j];
+    }
+    for (uint64_t j = tail0; j < n; ++j) {
+      s1 += d[j];
+      s2 += ((n - j) % 65521u) * d[j];
+    }
+  }
+  const uint32_t* const dw = reinterpret_cast<const uint32_t*>(d + head);
+  // weight of the first byte of my first word, then 128 less every step (mod 65521)
+  uint32_t wm = static_cast<uint32_t>((n - head - 4u * lane) % 65521u);
+  for (uint64_t k = lane; k < words; k += 32) {
+    const uint32_t w = dw[k];
+    const uint32_t b0 = w & 0xffu, b1 = (w >> 8) & 0xffu, b2 = (w >> 16) & 0xffu, b3 = w >> 24;
+    const uint32_t bs = b0 + b1 + b2 + b3;
+    s1 += bs;
+    // sum (wm - i) b_i  =  wm * bs - (b1 + 2 b2 + 3 b3); wm may be < 3: add 65521 first (same residue)
+    s2 += static_cast<uint64_t>(wm + 65521u) * bs - (b1 + 2u * b2 + 3u * b3);
+    wm = wm >= 128u ? wm - 128u : wm + 65521u - 128u;
+  }
+  for (int o = 16; o; o >>= 1) {
+    s1 += __shfl_down_sync(FULL, s1, o);
+    s2 += __shfl_down_sync(FULL, s2, o);
+  }
+  s1 = (1u + s1) % 65521u;
+  s2 = (n % 65521u + s2) % 65521u;
+  return __shfl_sync(FULL, static_cast<uint32_t>((s2 << 16) | s1), 0);
+}
+
+// CRC-32 of d[0 .. n) by the whole warp over the lane-private tables of crc_tables_init; every lane
+// returns it.  64 contiguous pieces, two per lane (two independent chains hide the look-up latency),
+// then  crc(A || B) = crc(A) * x^(8 |B|) + crc(B)  front to back.
+__device__ __forceinline__ uint32_t warp_crc32(const uint8_t* d, uint64_t n, uint32_t lane, const uint32_t* crc_tab)
+{
+  constexpr unsigned FULL = 0xffffffffu;
+  const uint32_t* const tl = crc_tab + lane;
+  auto step1 = [&](uint32_t c, uint32_t byte) { return tl[((c ^ byte) & 0xffu) * 32u] ^ (c >> 8); };
+  auto step4 = [&](uint32_t c, uint32_t word) {
+    c ^= word;
+    return tl[(768u + (c & 0xffu)) * 32u] ^ tl[(512u + ((c >> 8) & 0xffu)) * 32u] ^
+           tl[(256u + ((c >> 16) & 0xffu)) * 32u] ^ tl[(c >> 24) * 32u];
+  };
+  const uint64_t piece = ((n + 63) / 64 + 15) & ~15ull;
+  auto lo_of = [&](uint32_t pc) { return piece * pc < n ? piece * pc : n; };
+  auto hi_of = [&](uint32_t pc) { return lo_of(pc) + piece < n ? lo_of(pc) + piece : n; };
+  uint64_t j0 = lo_of(lane), j1 = lo_of(lane + 32u);
+  const uint64_t h0 = hi_of(lane), h1 = hi_of(lane + 32u);
+  uint32_t c0 = 0xffffffffu, c1 = 0xffffffffu;
+  // bytes up to a 16-byte boundary, 16-byte loads (a lane walks its own piece: a 32-byte
+  // sector then serves two loads instead of eight), the bytes left over
+  for (; j0 < h0 && ((reinterpret_cast<uintptr_t>(d + j0)) & 15u); ++j0) c0 = step1(c0, d[j0]);
+  for (; j1 < h1 && ((reinterpret_cast<uintptr_t>(d + j1)) & 15u); ++j1) c1 = step1(c1, d[j1]);
+  while (j0 + 16 <= h0 && j1 + 16 <= h1) {
+    const uint4 v0 = *reinterpret_cast<const uint4*>(d + j0);
+    const uint4 v1 = *reinterpret_cast<const uint4*>(d + j1);
+    c0 = step4(c0, v0.x);
+    c1 = step4(c1, v1.x);
+    c0 = step4(c0, v0.y);
+    c1 = step4(c1, v1.y);
+    c0 = step4(c0, v0.z);
+    c1 = step4(c1, v1.z);
+    c0 = step4(c0, v0.w);
+    c1 = step4(c1, v1.w);
+    j0 += 16;
+    j1 += 16;
+  }
+  for (; j0 + 4 <= h0; j0 += 4) c0 = step4(c0, *reinterpret_cast<const uint32_t*>(d + j0));
+  for (; j1 + 4 <= h1; j1 += 4) c1 = step4(c1, *reinterpret_cast<const uint32_t*>(d + j1));
+  for (; j0 < h0; ++j0) c0 = step1(c0, d[j0]);
+  for (; j1 < h1; ++j1) c1 = step1(c1, d[j1]);
+  c0 = ~c0;  // each piece's own CRC-32 (of an empty piece: 0)
+  c1 = ~c1;
+  const uint32_t shift_full = crc_x8n(piece);
+  uint32_t acc = 0;
+  for (uint32_t pc = 0; pc < 64u; ++pc) {
+    const uint32_t cl = __shfl_sync(FULL, pc < 32u ? c0 : c1, static_cast<int>(pc & 31u));
+    const uint64_t l_len = hi_of(pc) - lo_of(pc);
+    if (lane == 0 && l_len) acc = crc_mulmod(l_len == piece ? shift_full : crc_x8n(l_len), acc) ^ cl;
+  }
+  return __shfl_sync(FULL, acc, 0);
+}
+
+__global__ void __launch_bounds__(CHECK_THREADS) container_check_kernel(const ContainerArgs a)
+{
+#ifdef SFB_CPU_EMU
+  uint32_t* const crc_tab = SFB_EMU_CRC_SMEM;  // tests/cpu_emu: the block's shared memory
+#else
+  extern __shared__ uint32_t crc_tab[];
+#endif
+  crc_tables_init(crc_tab);
   __syncthreads();
   const uint32_t lane = threadIdx.x & 31u;
   const uint64_t warps = (static_cast<uint64_t>(gridDim.x) * blockDim.x) >> 5;
@@ -184,94 +285,7 @@ __global__ void __launch_bounds__(CHECK_THREADS) container_check_kernel(const Co
     if (kind == CT_RAW || a.status[i] != 0) continue;  // raw: nothing to check; failed: the decoder's status stands
     const uint8_t* d = a.dst_base + a.dst_off[i];
     const uint64_t n = a.written[i];
-    uint32_t got;
-    if (kind == CT_ZLIB) {
-      // Adler-32 (RFC 1950 §8.2): s1 = 1 + sum b_j, s2 = n + sum (n - j) b_j, both mod 65521
-      // (a lane takes aligned words, 128 bytes per warp and step; the weight n - j is kept modulo
-      //  65521 by subtracting 128 per step, so the inner loop has no division)
-      uint64_t s1 = 0, s2 = 0;
-      const uint32_t mis = static_cast<uint32_t>(reinterpret_cast<uintptr_t>(d)) & 3u;
-      const uint64_t head = mis ? (4u - mis < n ? 4u - mis : n) : 0u;  // bytes before the first aligned word
-      const uint64_t words = (n - head) >> 2;
-      const uint64_t tail0 = head + 4u * words;
-      if (lane == 0) {  // the few bytes around the aligned part
-        for (uint64_t j = 0; j < head; ++j) {
-          s1 += d[j];
-          s2 += ((n - j) % 65521u) * d[j];
-        }
-        for (uint64_t j = tail0; j < n; ++j) {
-          s1 += d[j];
-          s2 += ((n - j) % 65521u) * d[j];
-        }
-      }
-      const uint32_t* const dw = reinterpret_cast<const uint32_t*>(d + head);
-      // weight of the first byte of my first word, then 128 less every step (mod 65521)
-      uint32_t wm = static_cast<uint32_t>((n - head - 4u * lane) % 65521u);
-      for (uint64_t k = lane; k < words; k += 32) {
-        const uint32_t w = dw[k];
-        const uint32_t b0 = w & 0xffu, b1 = (w >> 8) & 0xffu, b2 = (w >> 16) & 0xffu, b3 = w >> 24;
-        const uint32_t bs = b0 + b1 + b2 + b3;
-        s1 += bs;
-        // sum (wm - i) b_i  =  wm * bs - (b1 + 2 b2 + 3 b3); wm may be < 3: add 65521 first (same residue)
-        s2 += static_cast<uint64_t>(wm + 65521u) * bs - (b1 + 2u * b2 + 3u * b3);
-        wm = wm >= 128u ? wm - 128u : wm + 65521u - 128u;
-      }
-      for (int o = 16; o; o >>= 1) {
-        s1 += __shfl_down_sync(FULL, s1, o);
-        s2 += __shfl_down_sync(FULL, s2, o);
-      }
-      s1 = (1u + s1) % 65521u;
-      s2 = (n % 65521u + s2) % 65521u;
-      got = static_cast<uint32_t>((s2 << 16) | s1);
-    } else {
-      // CRC-32: 64 contiguous pieces, two per lane (two independent chains hide the look-up latency),
-      // then  crc(A || B) = crc(A) * x^(8 |B|) + crc(B)  front to back
-      const uint32_t* const tl = crc_tab + lane;
-      auto step1 = [&](uint32_t c, uint32_t byte) { return tl[((c ^ byte) & 0xffu) * 32u] ^ (c >> 8); };
-      auto step4 = [&](uint32_t c, uint32_t word) {
-        c ^= word;
-        return tl[(768u + (c & 0xffu)) * 32u] ^ tl[(512u + ((c >> 8) & 0xffu)) * 32u] ^
-               tl[(256u + ((c >> 16) & 0xffu)) * 32u] ^ tl[(c >> 24) * 32u];
-      };
-      const uint64_t piece = ((n + 63) / 64 + 15) & ~15ull;
-      auto lo_of = [&](uint32_t pc) { return piece * pc < n ? piece * pc : n; };
-      auto hi_of = [&](uint32_t pc) { return lo_of(pc) + piece < n ? lo_of(pc) + piece : n; };
-      uint64_t j0 = lo_of(lane), j1 = lo_of(lane + 32u);
-      const uint64_t h0 = hi_of(lane), h1 = hi_of(lane + 32u);
-      uint32_t c0 = 0xffffffffu, c1 = 0xffffffffu;
-      // bytes up to a 16-byte boundary, 16-byte loads (a lane walks its own piece: a 32-byte
-      // sector then serves two loads instead of eight), the bytes left over
-      for (; j0 < h0 && ((reinterpret_cast<uintptr_t>(d + j0)) & 15u); ++j0) c0 = step1(c0, d[j0]);
-      for (; j1 < h1 && ((reinterpret_cast<uintptr_t>(d + j1)) & 15u); ++j1) c1 = step1(c1, d[j1]);
-      while (j0 + 16 <= h0 && j1 + 16 <= h1) {
-        const uint4 v0 = *reinterpret_cast<const uint4*>(d + j0);
-        const uint4 v1 = *reinterpret_cast<const uint4*>(d + j1);
-        c0 = step4(c0, v0.x);
-        c1 = step4(c1, v1.x);
-        c0 = step4(c0, v0.y);
-        c1 = step4(c1, v1.y);
-        c0 = step4(c0, v0.z);
-        c1 = step4(c1, v1.z);
-        c0 = step4(c0, v0.w);
-        c1 = step4(c1, v1.w);
-        j0 += 16;
-        j1 += 16;
-      }
-      for (; j0 + 4 <= h0; j0 += 4) c0 = step4(c0, *reinterpret_cast<const uint32_t*>(d + j0));
-      for (; j1 + 4 <= h1; j1 += 4) c1 = step4(c1, *reinterpret_cast<const uint32_t*>(d + j1));
-      for (; j0 < h0; ++j0) c0 = step1(c0, d[j0]);
-      for (; j1 < h1; ++j1) c1 = step1(c1, d[j1]);
-      c0 = ~c0;  // each piece's own CRC-32 (of an empty piece: 0)
-      c1 = ~c1;
-      const uint32_t shift_full = crc_x8n(piece);
-      uint32_t acc = 0;
-      for (uint32_t pc = 0; pc < 64u; ++pc) {
-        const uint32_t cl = __shfl_sync(FULL, pc < 32u ? c0 : c1, static_cast<int>(pc & 31u));
-        const uint64_t l_len = hi_of(pc) - lo_of(pc);
-        if (lane == 0 && l_len) acc = crc_mulmod(l_len == piece ? shift_full : crc_x8n(l_len), acc) ^ cl;
-      }
-      got = __shfl_sync(FULL, acc, 0);
-    }
+    const uint32_t got = kind == CT_ZLIB ? warp_adler32(d, n, lane) : warp_crc32(d, n, lane, crc_tab);
     if (lane == 0) {
       if (got != a.expect[i]) a.status[i] = ST_CHECKSUM_MISMATCH;
       else if (kind == CT_GZIP && a.isize[i] != static_cast<uint32_t>(n)) a.status[i] = ST_SIZE_MISMATCH;
