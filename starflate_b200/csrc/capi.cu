@@ -62,6 +62,36 @@ using StreamCfg = sfb::Cfg<SFB_STREAM_ROOT_LIT, SFB_STREAM_ROOT_DIST, SFB_POOL, 
 // [4k+3] number of streams handed from the small to the large geometry
 constexpr uint64_t kMaxWaves = 256;
 constexpr uint64_t kCountersPerWave = 4;
+// d_order per stream: its place in the processing order (u32); behind all of those, one byte each,
+// "stored_streams_kernel finished it"
+constexpr uint64_t kOrderBytes = sizeof(uint32_t) + 1;
+
+// Device memory owned by a context or an inflate stream, freed with its owner (which is deleted
+// while a DeviceGuard for its device is alive).  reserve() grows it.
+struct DevBuf {
+  uint8_t* p = nullptr;
+  uint64_t cap = 0;  // bytes
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { release(); }
+  void release()
+  {
+    if (p) cudaFree(p);
+    p = nullptr;
+    cap = 0;
+  }
+  void swap(DevBuf& o)
+  {
+    std::swap(p, o.p);
+    std::swap(cap, o.cap);
+  }
+  template <class T>
+  T* as() const
+  {
+    return reinterpret_cast<T*>(p);
+  }
+};
 
 }  // namespace
 
@@ -76,11 +106,9 @@ struct sfb200_ctx {
                                // measured with the long periodic fill in: 5 (48 registers) beats 6 (40, spills
                                // in the chunk loop) on C2 8.5 / 8.9 ms and C4 5.0 / 5.5 ms — SFB200_LZW_CTAS)
   bool lzw_pf = false;         // SFB200_LZW_PF=1: lz_window_kernel with the source prefetch (measured slower; 5 CTAs per SM only)
-  uint8_t* d_queue = nullptr;  // hand-over queue of the overlapped mode (QueueArgs): counters, turns, states, items
-  uint64_t d_queue_cap = 0;
+  DevBuf d_queue;              // hand-over queue of the overlapped mode (QueueArgs): counters, turns, states, items
   int queue_mode = 0;          // SFB200_QUEUE=1: pass 2 runs beside pass 1 (lz_window_queue_kernel)
   int queue_ctas = 4;          // ... with this many of its CTAs per SM on the second stream (SFB200_QUEUE_CTAS)
-  bool compress_configured = false;
   int compress_ctas_per_sm = 0;
   bool no_stored = false;      // SFB200_NO_STORED=1: stored streams go through the lane kernel like the others (A/B runs)
   uint32_t no_pair = 0;        // SFB200_NO_PAIR=1: pass 1 takes one token per iteration (A/B runs)
@@ -90,50 +118,32 @@ struct sfb200_ctx {
   int small_regs_per_thread = 0;
   int stream_ctas_per_sm = 0;  // huff_stream_kernel (0: not usable)
   int stream_regs_per_thread = 0;
-  uint32_t* d_defer = nullptr;  // streams handed from the small to the large geometry
-  uint64_t d_defer_n = 0;
-  uint32_t* d_order = nullptr;  // processing order (streams sorted by first block type); behind its d_order_n
-                                // entries: one byte per stream, "stored_streams_kernel finished it"
-  uint64_t d_order_n = 0;
-  unsigned long long* d_counter = nullptr;  // 2 * kMaxWaves work counters
-  uint32_t* d_lens = nullptr;  // per-resident-lane code-length scratch
-  uint32_t* d_bits = nullptr;  // match-head bitmap: 1 bit per dst byte (grown on demand)
-  uint64_t d_bits_words = 0;
-  bool count_configured = false, check_configured = false, end_configured = false;  // per-device function attributes set
-  uint8_t* d_cont = nullptr;  // container route: payload offsets / sizes, kinds, trailer values, written
-  uint64_t d_cont_cap = 0;
-  uint8_t* d_gzf = nullptr;   // gzip files (gzip_file.cuh): the walk's step, result, probe metadata, tile counts
-  uint64_t d_gzf_cap = 0;
-  uint8_t* d_gzc = nullptr;   // ... candidates and jump tables
-  uint64_t d_gzc_cap = 0;
-  uint8_t* d_gzm = nullptr;   // ... the member table (kGzfMemberBytes per member)
-  uint64_t d_gzm_n = 0;
-  bool seal_configured = false;
-  uint8_t* d_wrap = nullptr;  // writing containers (container_write.cuh): the payloads' offsets and capacities
-  uint64_t d_wrap_cap = 0;
-  uint8_t* d_bgzf = nullptr;  // writing BGZF: a round's scratch slots, the compressor's arrays, the call's state
-  uint64_t d_bgzf_cap = 0;
-  uint8_t* d_find = nullptr;  // single-stream pass 1 (block_finder.cuh): counters, hash table, jobs, candidates
-  uint64_t d_find_cap = 0;
-  uint8_t* d_jump = nullptr;  // single-stream pass 2 (lz_jump.cuh): pointers, tile flags, round flags
-  uint64_t d_jump_cap = 0;
-  uint64_t* d_written = nullptr;  // pass-1 -> pass-2 sizes when the caller passes written == NULL
-  uint64_t d_written_n = 0;
+  DevBuf d_defer;    // streams handed from the small to the large geometry
+  DevBuf d_order;    // processing order (streams sorted by first block type), kOrderBytes per stream
+  DevBuf d_counter;  // 2 * kMaxWaves work counters
+  DevBuf d_lens;     // per-resident-lane code-length scratch
+  DevBuf d_bits;     // match-head bitmap: 1 bit per dst byte (bitmap_bytes)
+  DevBuf d_cont;     // container route: payload offsets / sizes, kinds, trailer values, written
+  DevBuf d_gzf;      // gzip files (gzip_file.cuh): the walk's step, result, probe metadata, tile counts
+  DevBuf d_gzc;      // ... candidates and jump tables
+  DevBuf d_gzm;      // ... the member table (kGzfMemberBytes per member, gzm_members)
+  DevBuf d_wrap;     // writing containers (container_write.cuh): the payloads' offsets and capacities
+  DevBuf d_bgzf;     // writing BGZF: a round's scratch slots, the compressor's arrays, the call's state
+  DevBuf d_find;     // single-stream pass 1 (block_finder.cuh): counters, hash table, jobs, candidates
+  DevBuf d_jump;     // single-stream pass 2 (lz_jump.cuh): pointers, tile flags, round flags
+  DevBuf d_written;  // pass-1 -> pass-2 sizes when the caller passes written == NULL
   uint64_t launches = 0;
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};  // call start | pass 1 start | pass 1 end | pass 2 end
   bool ev_valid = false;
   std::string err;
   // staging for the host-buffer entry points: a ring of kStageSlots sub-batch slots in device memory
-  // (bounded whatever the batch: SFB200_HOST_STAGING_MB), plus the single-stream helpers' buffers
-  uint8_t* d_src = nullptr;   // (single-stream helpers: size discovery, containers)
-  uint64_t d_src_cap = 0;
-  uint8_t* d_dst = nullptr;
-  uint64_t d_dst_cap = 0;
-  uint8_t* st_src[3] = {nullptr, nullptr, nullptr};
-  uint8_t* st_dst[3] = {nullptr, nullptr, nullptr};
-  uint64_t st_src_cap = 0, st_dst_cap = 0;      // per slot
-  int st_slots = 0;                             // slots allocated so far (a small call needs one)
-  uint64_t* st_meta[3] = {nullptr, nullptr, nullptr};  // per slot: src_off, src_len, dst_off, dst_cap, written (u64 x n), status (u8 x n)
+  // (bounded whatever the batch: SFB200_HOST_STAGING_MB), plus the single-buffer calls' buffers
+  DevBuf d_src, d_dst;  // (single-buffer calls: host_buffer_call)
+  DevBuf d_meta;        // ... their metadata block
+  DevBuf st_src[3], st_dst[3];             // exactly st_src_cap + 64 and st_dst_cap + 64 bytes each
+  uint64_t st_src_cap = 0, st_dst_cap = 0;  // per slot
+  int st_slots = 0;                         // slots allocated so far (a small call needs one)
+  DevBuf st_meta[3];  // per slot: src_off, src_len, dst_off, dst_cap, written (u64 x st_meta_n), status (u8 x st_meta_n)
   uint64_t* st_hmeta[3] = {nullptr, nullptr, nullptr};  // pinned mirror: the four input arrays (rebased) + written + status
   uint64_t st_meta_n = 0;
   cudaStream_t s_meta = nullptr;                // status / written read-back
@@ -179,15 +189,82 @@ struct DeviceGuard {
     if (e_ != cudaSuccess) return fail((ctx), e_, #call);    \
   } while (0)
 
-int grow(sfb200_ctx* ctx, uint8_t** p, uint64_t* cap, uint64_t need)
+// Room for `need` bytes in b: grown to need + need / 8 + 256 bytes (exactly `need` when `exact`),
+// never shrunk.  keep == 0: the old memory is freed first, so that a failed allocation returns
+// SFB200_RC_OUT_OF_MEMORY with b empty and valid, and the caller may take a route that needs less.
+// keep > 0: the first `keep` bytes move to the new memory.
+int reserve(sfb200_ctx* ctx, DevBuf& b, uint64_t need, uint64_t keep = 0, bool exact = false)
 {
-  if (need <= *cap) return SFB200_RC_OK;
-  if (*p) SFB_TRY(ctx, cudaFree(*p));
-  *p = nullptr;
-  *cap = 0;
-  const uint64_t want = need + need / 8 + 256;
-  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(p), want));
-  *cap = want;
+  if (need <= b.cap) return SFB200_RC_OK;
+  if (!keep) b.release();
+  DevBuf q;
+  const uint64_t want = exact ? need : need + need / 8 + 256;
+  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&q.p), want));
+  q.cap = want;
+  if (keep) SFB_TRY(ctx, cudaMemcpy(q.p, b.p, keep, cudaMemcpyDeviceToDevice));
+  b.swap(q);  // (q frees the old memory)
+  return SFB200_RC_OK;
+}
+
+// The kernel's function attributes (they are per device: set once, by sfb200_create): the dynamic
+// shared memory it may take (smem > 0) and, with `carveout`, the largest shared-memory carve-out.
+// per_sm / regs (if given) receive its resident CTAs per SM at `threads` and `smem`, and its
+// registers per thread.
+template <class Kernel>
+cudaError_t setup_kernel(Kernel kern, int smem, bool carveout, int threads = 0, int* per_sm = nullptr,
+                         int* regs = nullptr)
+{
+  cudaError_t e = cudaSuccess;
+  if (smem > 0 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess)
+    return e;
+  if (carveout && (e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                            cudaSharedmemCarveoutMaxShared)) != cudaSuccess)
+    return e;
+  if (per_sm && (e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, kern, threads, smem)) != cudaSuccess)
+    return e;
+  cudaFuncAttributes fa;
+  if (regs && (e = cudaFuncGetAttributes(&fa, kern)) != cudaSuccess) return e;
+  if (regs) *regs = fa.numRegs;
+  return cudaSuccess;
+}
+
+// CTAs of a launch that pulls its work dynamically: what the work wants, at most what is resident
+unsigned grid_size(uint64_t want, uint64_t resident) { return static_cast<unsigned>(std::min(want, resident)); }
+
+// pass 2's match-head bitmap: one bit per byte of dst (counted from its 128-byte aligned base,
+// `delta` bytes in front of dst_base) and eight guard words
+uint64_t bitmap_bytes(uint64_t dst_bytes, uint64_t delta) { return ((dst_bytes + delta) / 32 + 8) * sizeof(uint32_t); }
+
+// The single-buffer host calls.  src is staged in the context's d_src, `device(d_src, d_dst, meta, &wr)`
+// makes the device call into d_dst on the legacy default stream, and of dst only the `wr` bytes it
+// produced come back.  meta is the context's block {src_off = 0, src_len, dst_off = 0, dst_cap}, then
+// written and status (u8) for the call to fill: a batch of one stream, whose results read_meta() returns.
+template <class Device>
+int host_buffer_call(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, uint8_t* dst, uint64_t dst_cap,
+                     uint64_t* written, Device device)
+{
+  int rc = reserve(ctx, ctx->d_src, src_len + 64);
+  if (rc == SFB200_RC_OK) rc = reserve(ctx, ctx->d_dst, dst_cap + 64);
+  if (rc == SFB200_RC_OK) rc = reserve(ctx, ctx->d_meta, 6 * sizeof(uint64_t), 0, true);
+  if (rc != SFB200_RC_OK) return rc;
+  const uint64_t h[6] = {0, src_len, 0, dst_cap, 0, 0};
+  uint64_t* const meta = ctx->d_meta.as<uint64_t>();
+  if (src_len) SFB_TRY(ctx, cudaMemcpyAsync(ctx->d_src.p, src, src_len, cudaMemcpyHostToDevice, nullptr));
+  SFB_TRY(ctx, cudaMemcpyAsync(meta, h, sizeof h, cudaMemcpyHostToDevice, nullptr));
+  uint64_t wr = 0;
+  rc = device(ctx->d_src.p, ctx->d_dst.p, meta, &wr);
+  if (rc != SFB200_RC_OK) return rc;
+  if (wr > dst_cap) return SFB200_RC_CUDA_ERROR;  // (cannot happen)
+  if (wr) SFB_TRY(ctx, cudaMemcpy(dst, ctx->d_dst.p, wr, cudaMemcpyDeviceToHost));  // only what was produced
+  if (written) *written = wr;
+  return SFB200_RC_OK;
+}
+
+int read_meta(sfb200_ctx* ctx, const uint64_t* meta, uint64_t* written, uint8_t* status)
+{
+  SFB_TRY(ctx, cudaMemcpyAsync(written, meta + 4, 8, cudaMemcpyDeviceToHost, nullptr));
+  SFB_TRY(ctx, cudaMemcpyAsync(status, meta + 5, 1, cudaMemcpyDeviceToHost, nullptr));
+  SFB_TRY(ctx, cudaStreamSynchronize(nullptr));
   return SFB200_RC_OK;
 }
 
@@ -221,120 +298,73 @@ int sfb200_create(int device, sfb200_ctx** out)
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return bail(SFB200_RC_CUDA_ERROR);
   ctx->sm_count = prop.multiProcessorCount;
-  auto kern = sfb::huff_lanes_kernel<LaneCfg>;
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           LaneCfg::SMEM_BYTES) != cudaSuccess)
+  if (const char* e = std::getenv("SFB200_LZ_V1")) ctx->lz_v1 = e[0] == '1';
+  if (const char* e = std::getenv("SFB200_NO_PAIR")) ctx->no_pair = e[0] == '1';
+  if (const char* e = std::getenv("SFB200_NO_STORED")) ctx->no_stored = e[0] == '1';
+  if (const char* e = std::getenv("SFB200_QUEUE")) ctx->queue_mode = std::atoi(e);
+  if (const char* e = std::getenv("SFB200_LZW_PF")) ctx->lzw_pf = e[0] == '1';
+  if (const char* e = std::getenv("SFB200_QUEUE_CTAS")) ctx->queue_ctas = std::max(1, std::atoi(e));
+  if (const char* e = std::getenv("SFB200_LZW_CTAS")) {
+    const int v = std::atoi(e);
+    if (v == 4 || v == 5 || v == 6) ctx->lzw_minb = v;
+  }
+  static_assert(sfb::LZ_THREADS == sfb::LZW_THREADS, "one launch geometry for both pass-2 kernels");
+  static_assert(LaneCfg::WARPS == WideCfg::WARPS, "the wide launch takes the CTA count computed for the large one");
+  const void* lzw = ctx->lzw_minb == 4   ? reinterpret_cast<const void*>(sfb::lz_window_kernel<4>)
+                    : ctx->lzw_minb == 5 ? reinterpret_cast<const void*>(sfb::lz_window_kernel<5>)
+                                         : reinterpret_cast<const void*>(sfb::lz_window_kernel<6>);
+  const void* lz = ctx->lz_v1 ? reinterpret_cast<const void*>(sfb::lz_resolve_kernel) : lzw;
+  // the kernels the calls launch (pass 1, size discovery, the END decode of gzip members, the container
+  // checksums and seal, compression, pass 2): a context has them all
+  int lz_per_sm = 0;
+  if (setup_kernel(sfb::huff_lanes_kernel<LaneCfg>, LaneCfg::SMEM_BYTES, true, LaneCfg::WARPS * 32, &ctx->ctas_per_sm,
+                   &ctx->regs_per_thread) != cudaSuccess ||
+      ctx->ctas_per_sm < 1 ||
+      setup_kernel(sfb::huff_lanes_kernel<LaneCfg, true>, LaneCfg::SMEM_BYTES, true) != cudaSuccess ||
+      setup_kernel(sfb::huff_lanes_kernel<LaneCfg, false, false, true>, LaneCfg::SMEM_BYTES, true) != cudaSuccess ||
+      setup_kernel(sfb::container_check_kernel, sfb::CHECK_SMEM_BYTES, false) != cudaSuccess ||
+      setup_kernel(sfb::container_seal_kernel, sfb::CHECK_SMEM_BYTES, false) != cudaSuccess ||
+      setup_kernel(sfb::deflate_compress_kernel, sfb::CMP_SMEM_BYTES, false, sfb::CMP_WARPS * 32,
+                   &ctx->compress_ctas_per_sm) != cudaSuccess ||
+      setup_kernel(lz, 0, false, sfb::LZ_THREADS, &lz_per_sm, &ctx->lz_regs_per_thread) != cudaSuccess || lz_per_sm < 1)
     return bail(SFB200_RC_CUDA_ERROR);
-  cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout,
-                       cudaSharedmemCarveoutMaxShared);
-  int per_sm = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, LaneCfg::WARPS * 32,
-                                                    LaneCfg::SMEM_BYTES) != cudaSuccess ||
-      per_sm < 1)
-    return bail(SFB200_RC_CUDA_ERROR);
-  ctx->ctas_per_sm = per_sm;
-  cudaFuncAttributes fa;
-  if (cudaFuncGetAttributes(&fa, kern) == cudaSuccess) ctx->regs_per_thread = fa.numRegs;
-  {
-    if (const char* e = std::getenv("SFB200_LZ_V1")) ctx->lz_v1 = e[0] == '1';
-    if (const char* e = std::getenv("SFB200_NO_PAIR")) ctx->no_pair = e[0] == '1';
-    if (const char* e = std::getenv("SFB200_NO_STORED")) ctx->no_stored = e[0] == '1';
-    if (const char* e = std::getenv("SFB200_QUEUE")) ctx->queue_mode = std::atoi(e);
-    if (const char* e = std::getenv("SFB200_LZW_PF")) ctx->lzw_pf = e[0] == '1';
-    if (const char* e = std::getenv("SFB200_QUEUE_CTAS")) ctx->queue_ctas = std::max(1, std::atoi(e));
-    static_assert(sfb::LZ_THREADS == sfb::LZW_THREADS, "one launch geometry for both pass-2 kernels");
-    static_assert(LaneCfg::WARPS == WideCfg::WARPS, "the wide launch takes the CTA count computed for the large one");
-    int lz_per_sm = 0;
-    if (const char* e = std::getenv("SFB200_LZW_CTAS")) {
-      const int v = std::atoi(e);
-      if (v == 4 || v == 5 || v == 6) ctx->lzw_minb = v;
-    }
-    const void* lzw = ctx->lzw_minb == 4   ? reinterpret_cast<const void*>(sfb::lz_window_kernel<4>)
-                      : ctx->lzw_minb == 5 ? reinterpret_cast<const void*>(sfb::lz_window_kernel<5>)
-                                           : reinterpret_cast<const void*>(sfb::lz_window_kernel<6>);
-    if ((ctx->lz_v1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&lz_per_sm, sfb::lz_resolve_kernel, sfb::LZ_THREADS, 0)
-                    : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&lz_per_sm, lzw, sfb::LZW_THREADS, 0)) !=
-            cudaSuccess ||
-        lz_per_sm < 1)
+  ctx->compress_ctas_per_sm = std::max(1, ctx->compress_ctas_per_sm);
+  // The queue-mode pass 2 must be able to share an SM with pass 1: an SM changes its shared-memory
+  // carve-out only when it is idle, so a kernel that asks for none of it, once resident, keeps
+  // pass 1 (112 KiB per CTA) off that SM for as long as it runs — ask for pass 1's carve-out.
+  if (ctx->queue_mode) {
+    const void* lzq = ctx->lzw_minb == 4   ? reinterpret_cast<const void*>(sfb::lz_window_queue_kernel<4>)
+                      : ctx->lzw_minb == 5 ? reinterpret_cast<const void*>(sfb::lz_window_queue_kernel<5>)
+                                           : reinterpret_cast<const void*>(sfb::lz_window_queue_kernel<6>);
+    if (setup_kernel(sfb::huff_lanes_kernel<LaneCfg, false, true>, LaneCfg::SMEM_BYTES, true) != cudaSuccess ||
+        setup_kernel(lzq, 0, true) != cudaSuccess)
       return bail(SFB200_RC_CUDA_ERROR);
-    // The queue-mode pass 2 must be able to share an SM with pass 1: an SM changes its shared-memory
-    // carve-out only when it is idle, so a kernel that asks for none of it, once resident, keeps
-    // pass 1 (112 KiB per CTA) off that SM for as long as it runs — ask for pass 1's carve-out.
-    if (ctx->queue_mode) {
-      auto qk = sfb::huff_lanes_kernel<LaneCfg, false, true>;
-      if (cudaFuncSetAttribute(qk, cudaFuncAttributeMaxDynamicSharedMemorySize, LaneCfg::SMEM_BYTES) != cudaSuccess ||
-          cudaFuncSetAttribute(qk, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared) !=
-              cudaSuccess)
-        return bail(SFB200_RC_CUDA_ERROR);
-      const void* lzq = ctx->lzw_minb == 4   ? reinterpret_cast<const void*>(sfb::lz_window_queue_kernel<4>)
-                        : ctx->lzw_minb == 5 ? reinterpret_cast<const void*>(sfb::lz_window_queue_kernel<5>)
-                                             : reinterpret_cast<const void*>(sfb::lz_window_queue_kernel<6>);
-      if (cudaFuncSetAttribute(lzq, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared) !=
-          cudaSuccess)
-        return bail(SFB200_RC_CUDA_ERROR);
-    }
-    // fewer resident warps keep the streams' 32 KiB windows inside the L2 (DESIGN.md)
-    int cap = SFB_LZ_CTAS_PER_SM;
-    if (const char* e = std::getenv("SFB200_LZ_CTAS_PER_SM")) cap = std::atoi(e);
-    ctx->lz_ctas_per_sm = (cap > 0 && cap < lz_per_sm) ? cap : lz_per_sm;
-    cudaFuncAttributes lfa;
-    if ((ctx->lz_v1 ? cudaFuncGetAttributes(&lfa, sfb::lz_resolve_kernel) : cudaFuncGetAttributes(&lfa, lzw)) == cudaSuccess)
-      ctx->lz_regs_per_thread = lfa.numRegs;
   }
-  if (cudaMalloc(reinterpret_cast<void**>(&ctx->d_counter), (kCountersPerWave * kMaxWaves + 16) * sizeof(unsigned long long)) !=
-      cudaSuccess)
-    return bail(SFB200_RC_OUT_OF_MEMORY);
-  {
-    auto sk = sfb::huff_lanes_kernel<SmallCfg>;
-    int sp = 0;
-    if (cudaFuncSetAttribute(sk, cudaFuncAttributeMaxDynamicSharedMemorySize, SmallCfg::SMEM_BYTES) ==
-            cudaSuccess &&
-        cudaFuncSetAttribute(sk, cudaFuncAttributePreferredSharedMemoryCarveout,
-                             cudaSharedmemCarveoutMaxShared) == cudaSuccess &&
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sp, sk, SmallCfg::WARPS * 32,
-                                                      SmallCfg::SMEM_BYTES) == cudaSuccess)
-      ctx->small_ctas_per_sm = sp;
-    cudaFuncAttributes sfa;
-    if (cudaFuncGetAttributes(&sfa, sk) == cudaSuccess) ctx->small_regs_per_thread = sfa.numRegs;
-    cudaGetLastError();
-  }
-  {
-    auto sk = sfb::huff_lanes_kernel<WideCfg>;
-    int sp = 0;
-    bool off = false;
-    if (const char* e = std::getenv("SFB200_NO_WIDE")) off = e[0] == '1';
-    if (!off &&
-        cudaFuncSetAttribute(sk, cudaFuncAttributeMaxDynamicSharedMemorySize, WideCfg::SMEM_BYTES) ==
-            cudaSuccess &&
-        cudaFuncSetAttribute(sk, cudaFuncAttributePreferredSharedMemoryCarveout,
-                             cudaSharedmemCarveoutMaxShared) == cudaSuccess &&
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sp, sk, WideCfg::WARPS * 32,
-                                                      WideCfg::SMEM_BYTES) == cudaSuccess)
-      ctx->wide_ctas_per_sm = sp;
-    cudaGetLastError();
-  }
-  {
-    auto sk = sfb::huff_stream_kernel<StreamCfg>;
-    int sp = 0;
-    if (cudaFuncSetAttribute(sk, cudaFuncAttributeMaxDynamicSharedMemorySize, StreamCfg::SMEM_BYTES) ==
-            cudaSuccess &&
-        cudaFuncSetAttribute(sk, cudaFuncAttributePreferredSharedMemoryCarveout,
-                             cudaSharedmemCarveoutMaxShared) == cudaSuccess &&
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sp, sk, 32, StreamCfg::SMEM_BYTES) == cudaSuccess)
-      ctx->stream_ctas_per_sm = sp;
-    cudaFuncAttributes sfa;
-    if (cudaFuncGetAttributes(&sfa, sk) == cudaSuccess) ctx->stream_regs_per_thread = sfa.numRegs;
-    cudaGetLastError();
-  }
-  const size_t big_warps = std::max(static_cast<size_t>(per_sm) * LaneCfg::WARPS,
+  // fewer resident warps keep the streams' 32 KiB windows inside the L2 (DESIGN.md)
+  int cap = SFB_LZ_CTAS_PER_SM;
+  if (const char* e = std::getenv("SFB200_LZ_CTAS_PER_SM")) cap = std::atoi(e);
+  ctx->lz_ctas_per_sm = (cap > 0 && cap < lz_per_sm) ? cap : lz_per_sm;
+  // the other geometries: one that cannot be set up is not used (0 CTAs per SM)
+  if (setup_kernel(sfb::huff_lanes_kernel<SmallCfg>, SmallCfg::SMEM_BYTES, true, SmallCfg::WARPS * 32,
+                   &ctx->small_ctas_per_sm, &ctx->small_regs_per_thread) != cudaSuccess)
+    ctx->small_ctas_per_sm = 0;
+  bool no_wide = false;
+  if (const char* e = std::getenv("SFB200_NO_WIDE")) no_wide = e[0] == '1';
+  if (no_wide || setup_kernel(sfb::huff_lanes_kernel<WideCfg>, WideCfg::SMEM_BYTES, true, WideCfg::WARPS * 32,
+                              &ctx->wide_ctas_per_sm) != cudaSuccess)
+    ctx->wide_ctas_per_sm = 0;
+  if (setup_kernel(sfb::huff_stream_kernel<StreamCfg>, StreamCfg::SMEM_BYTES, true, 32, &ctx->stream_ctas_per_sm,
+                   &ctx->stream_regs_per_thread) != cudaSuccess)
+    ctx->stream_ctas_per_sm = 0;
+  cudaGetLastError();
+  const size_t big_warps = std::max(static_cast<size_t>(ctx->ctas_per_sm) * LaneCfg::WARPS,
                                     static_cast<size_t>(ctx->stream_ctas_per_sm));
   const size_t small_warps = static_cast<size_t>(ctx->small_ctas_per_sm) * SmallCfg::WARPS;
   const size_t lens_bytes = static_cast<size_t>(ctx->sm_count) * std::max(big_warps, small_warps) *
                             sfb::SCRATCH_WORDS * 32 * sizeof(uint32_t);
-  if (cudaMalloc(reinterpret_cast<void**>(&ctx->d_lens), lens_bytes) != cudaSuccess) {
-    cudaFree(ctx->d_counter);
-    return bail(SFB200_RC_OUT_OF_MEMORY);
-  }
+  int rc = reserve(ctx, ctx->d_counter, (kCountersPerWave * kMaxWaves + 16) * sizeof(unsigned long long), 0, true);
+  if (rc == SFB200_RC_OK) rc = reserve(ctx, ctx->d_lens, lens_bytes, 0, true);
+  if (rc != SFB200_RC_OK) return bail(rc);
   for (auto& e : ctx->ev)
     if (cudaEventCreate(&e) != cudaSuccess) {
       sfb200_destroy(ctx);
@@ -347,28 +377,8 @@ int sfb200_create(int device, sfb200_ctx** out)
 void sfb200_destroy(sfb200_ctx* ctx)
 {
   if (!ctx) return;
-  DeviceGuard guard_(ctx->device);
-  cudaFree(ctx->d_counter);
-  cudaFree(ctx->d_lens);
-  cudaFree(ctx->d_bits);
-  cudaFree(ctx->d_written);
-  cudaFree(ctx->d_jump);
-  cudaFree(ctx->d_find);
-  cudaFree(ctx->d_cont);
-  cudaFree(ctx->d_gzf);
-  cudaFree(ctx->d_gzc);
-  cudaFree(ctx->d_gzm);
-  cudaFree(ctx->d_wrap);
-  cudaFree(ctx->d_bgzf);
-  cudaFree(ctx->d_defer);
-  cudaFree(ctx->d_order);
-  cudaFree(ctx->d_queue);
-  cudaFree(ctx->d_src);
-  cudaFree(ctx->d_dst);
+  DeviceGuard guard_(ctx->device);  // (the context's device memory is freed with it, on its device)
   for (int k = 0; k < 3; ++k) {
-    cudaFree(ctx->st_src[k]);
-    cudaFree(ctx->st_dst[k]);
-    cudaFree(ctx->st_meta[k]);
     if (ctx->st_hmeta[k]) cudaFreeHost(ctx->st_hmeta[k]);
     for (auto& e : ctx->st_ev[k])
       if (e) cudaEventDestroy(e);
@@ -390,10 +400,10 @@ const char* sfb200_last_error(const sfb200_ctx* ctx) { return ctx ? ctx->err.c_s
 // the device and copies the queue's eight counters — tail, head, final_tail, done, dbg[0..3].
 int sfb200_debug_queue(sfb200_ctx* ctx, unsigned long long* out8)
 {
-  if (!ctx || !out8 || !ctx->d_queue) return SFB200_RC_BAD_ARGUMENT;
+  if (!ctx || !out8 || !ctx->d_queue.p) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
   SFB_TRY(ctx, cudaDeviceSynchronize());
-  SFB_TRY(ctx, cudaMemcpy(out8, ctx->d_queue, 64, cudaMemcpyDeviceToHost));
+  SFB_TRY(ctx, cudaMemcpy(out8, ctx->d_queue.p, 64, cudaMemcpyDeviceToHost));
   return SFB200_RC_OK;
 }
 
@@ -462,26 +472,15 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
   // the kernels index dst (and the bitmap) from a 128-byte aligned base
   const uint64_t delta = reinterpret_cast<uintptr_t>(dst_base) & 127u;
   dst_base -= delta;
-  // scratch: one bit per dst byte (+ guard words), grown on demand and kept
-  const uint64_t bits_words = (dst_bytes + delta) / 32 + 8;
-  if (bits_words > ctx->d_bits_words) {
-    if (ctx->d_bits) SFB_TRY(ctx, cudaFree(ctx->d_bits));
-    ctx->d_bits = nullptr;
-    ctx->d_bits_words = 0;
-    const uint64_t want = bits_words + bits_words / 8 + 64;
-    SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_bits), want * sizeof(uint32_t)));
-    ctx->d_bits_words = want;
-  }
+  const uint64_t bits_bytes = bitmap_bytes(dst_bytes, delta);
+  int rc = reserve(ctx, ctx->d_bits, bits_bytes);
+  if (rc != SFB200_RC_OK) return rc;
+  uint32_t* const match_bits = ctx->d_bits.as<uint32_t>();
+  unsigned long long* const ctrs = ctx->d_counter.as<unsigned long long>();
   if (!written) {
-    if (n > ctx->d_written_n) {
-      if (ctx->d_written) SFB_TRY(ctx, cudaFree(ctx->d_written));
-      ctx->d_written = nullptr;
-      ctx->d_written_n = 0;
-      const uint64_t want = n + n / 8 + 64;
-      SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_written), want * sizeof(uint64_t)));
-      ctx->d_written_n = want;
-    }
-    written = ctx->d_written;
+    rc = reserve(ctx, ctx->d_written, n * sizeof(uint64_t));
+    if (rc != SFB200_RC_OK) return rc;
+    written = ctx->d_written.as<uint64_t>();
   }
   // Few streams: a lane per stream would leave the GPU empty, so each stream gets a warp that
   // decodes 32 spans of it speculatively (huff_stream.cuh).  Same results, by construction.
@@ -512,7 +511,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
     const uint64_t stripes = (jump_tiles + stripe_tiles - 1) / stripe_tiles;
     const uint64_t need = jump_tiles * sfb::JUMP_TILE * 4 + jump_tiles * 4 * (1 + sfb::JUMP_TILE / 128) +
                           stripes * (sfb::JUMP_MAX_ROUNDS + 1) * 4;
-    const int rc = grow(ctx, &ctx->d_jump, &ctx->d_jump_cap, need);
+    rc = reserve(ctx, ctx->d_jump, need);
     if (rc == SFB200_RC_OUT_OF_MEMORY) {
       // no room for the pointer array (4 bytes per dst byte): a warp walks the stream instead —
       // slower, same results
@@ -539,7 +538,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
     const uint64_t need = 64 + 4ull * tab_size + sizeof(sfb::BlockJob) * static_cast<uint64_t>(job_cap) +
                           8ull * cand_cap + sizeof(sfb::WinRec) * static_cast<uint64_t>(rec_cap) +
                           28ull * job_cap + 64;
-    const int rc = grow(ctx, &ctx->d_find, &ctx->d_find_cap, need);
+    rc = reserve(ctx, ctx->d_find, need);
     if (rc == SFB200_RC_OUT_OF_MEMORY) {  // blocks one after the other instead of side by side
       cudaGetLastError();
       ctx->err.clear();
@@ -557,13 +556,9 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
   bool use_small = false;
   if (const char* e = std::getenv("SFB200_GEOMETRY")) use_small = e[0] == 's' && ctx->small_ctas_per_sm > 0;
   if (resume) use_small = false;  // (the small geometry reports neither resume point nor end)
-  if (use_small && n > ctx->d_defer_n) {
-    if (ctx->d_defer) SFB_TRY(ctx, cudaFree(ctx->d_defer));
-    ctx->d_defer = nullptr;
-    ctx->d_defer_n = 0;
-    const uint64_t want = n + n / 8 + 64;
-    SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_defer), want * sizeof(uint32_t)));
-    ctx->d_defer_n = want;
+  if (use_small) {
+    rc = reserve(ctx, ctx->d_defer, n * sizeof(uint32_t));
+    if (rc != SFB200_RC_OK) return rc;
   }
   // Waves.  The two passes run BACK TO BACK over the whole batch: one launch each, inside which
   // warps pull groups of streams dynamically.  Cutting the batch into waves and running pass 2 of
@@ -598,7 +593,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
   if (qmode) {
     n_waves = 1;
     qcap = 2 * n + ((dst_bytes + delta) >> sfb::Q_SEG_SHIFT) + 64;
-    const int rc = grow(ctx, &ctx->d_queue, &ctx->d_queue_cap, 64 + 24 * n + 8 * qcap + 64);
+    rc = reserve(ctx, ctx->d_queue, 64 + 24 * n + 8 * qcap + 64);
     if (rc != SFB200_RC_OK) return rc;
   }
   const uint64_t per_wave = n_waves == 1 ? n : wave;
@@ -621,33 +616,27 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
   cudaStream_t s2 = overlap ? ctx->ps[1] : st;  // pass-2 chain
   ctx->ev_valid = false;
   SFB_TRY(ctx, cudaEventRecord(ctx->ev[0], st));
-  SFB_TRY(ctx, cudaMemsetAsync(ctx->d_counter, 0,
+  SFB_TRY(ctx, cudaMemsetAsync(ctrs, 0,
                                kCountersPerWave * std::max<uint64_t>(n_waves, 1) * sizeof(unsigned long long), st));
-  SFB_TRY(ctx, cudaMemsetAsync(ctx->d_counter + kCountersPerWave * kMaxWaves, 0, 16 * sizeof(unsigned long long), st));
-  SFB_TRY(ctx, cudaMemsetAsync(ctx->d_bits, 0, bits_words * sizeof(uint32_t), st));
-  if (qmode) SFB_TRY(ctx, cudaMemsetAsync(ctx->d_queue, 0, 64 + 24 * n + 8 * qcap, st));
+  SFB_TRY(ctx, cudaMemsetAsync(ctrs + kCountersPerWave * kMaxWaves, 0, 16 * sizeof(unsigned long long), st));
+  SFB_TRY(ctx, cudaMemsetAsync(match_bits, 0, bits_bytes, st));
+  if (qmode) SFB_TRY(ctx, cudaMemsetAsync(ctx->d_queue.p, 0, 64 + 24 * n + 8 * qcap, st));
   // Order the streams by the type of their first block (see lz_warp.cuh: PrepArgs)
   uint8_t* handled = nullptr;
   bool sorted = n >= 64 && n < 0xffffffffull && !stream_mode && !resume;
   if (const char* e = std::getenv("SFB200_NO_SORT"))
     if (e[0] == '1') sorted = false;
   if (sorted) {
-    if (n > ctx->d_order_n) {
-      if (ctx->d_order) SFB_TRY(ctx, cudaFree(ctx->d_order));
-      ctx->d_order = nullptr;
-      ctx->d_order_n = 0;
-      const uint64_t want = n + n / 8 + 64;
-      SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_order), want * (sizeof(uint32_t) + 1)));
-      ctx->d_order_n = want;
-    }
+    rc = reserve(ctx, ctx->d_order, n * kOrderBytes);
+    if (rc != SFB200_RC_OK) return rc;
     sfb::PrepArgs pa;
     pa.src_base = src_base;
     pa.src_off = src_off;
     pa.src_len = src_len;
     pa.n = n;
-    pa.type_count = ctx->d_counter + kCountersPerWave * kMaxWaves;
+    pa.type_count = ctrs + kCountersPerWave * kMaxWaves;
     pa.type_cursor = pa.type_count + 4;
-    pa.order = ctx->d_order;
+    pa.order = ctx->d_order.as<uint32_t>();
     const unsigned grid = static_cast<unsigned>((n + sfb::PREP_THREADS - 1) / sfb::PREP_THREADS);
     sfb::prep_count_kernel<<<grid, sfb::PREP_THREADS, 0, st>>>(pa);
     sfb::prep_scatter_kernel<<<grid, sfb::PREP_THREADS, 0, st>>>(pa);
@@ -656,7 +645,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
     // Streams of stored blocks: a warp each, wide copies (stored_copy.cuh); the lane kernel skips
     // what this kernel finished.
     if (!ctx->no_stored) {
-      handled = reinterpret_cast<uint8_t*>(ctx->d_order + ctx->d_order_n);
+      handled = ctx->d_order.p + sizeof(uint32_t) * (ctx->d_order.cap / kOrderBytes);  // (behind the entries)
       SFB_TRY(ctx, cudaMemsetAsync(handled, 0, n, st));
       sfb::StoredArgs sa;
       sa.src_base = src_base;
@@ -668,7 +657,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
       sa.status = status;
       sa.written = written;
       sa.handled = handled;
-      sa.order = ctx->d_order;
+      sa.order = pa.order;
       sa.type_count = pa.type_count;
       sa.counter = pa.type_count + 8;
       const uint64_t warps = static_cast<uint64_t>(ctx->sm_count) * 8 * (sfb::STORED_THREADS / 32);
@@ -687,8 +676,8 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
   for (uint64_t k = 0; k < n_waves; ++k) {
     const uint64_t first = k * per_wave;
     const uint64_t cnt = std::min(per_wave, n - first);
-    unsigned long long* const ctr = ctx->d_counter + kCountersPerWave * k;
-    const uint32_t* const order = sorted ? ctx->d_order + first : nullptr;
+    unsigned long long* const ctr = ctrs + kCountersPerWave * k;
+    const uint32_t* const order = sorted ? ctx->d_order.as<uint32_t>() + first : nullptr;
     // pass 1: Huffman layer, one lane per stream
     sfb::BatchArgs a{};
     a.src_base = src_base;
@@ -702,34 +691,31 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
     a.written = written;
     a.n = cnt;
     a.idx_base = first;
-    a.lens_scratch = ctx->d_lens;
-    a.match_bits = ctx->d_bits;
-    a.defer_list = nullptr;
-    a.defer_count = nullptr;
+    a.lens_scratch = ctx->d_lens.as<uint32_t>();
+    a.match_bits = match_bits;
     a.todo_list = order;
-    a.todo_count = nullptr;
     a.no_pair = ctx->no_pair;
     a.handled = handled;
     a.start_bit = resume ? resume->start_bit : nullptr;
     a.start_out = resume ? resume->start_out : nullptr;
     a.blk_end = resume ? resume->blk_end : nullptr;
     if (qmode) {
-      unsigned long long* const c = reinterpret_cast<unsigned long long*>(ctx->d_queue);
+      unsigned long long* const c = ctx->d_queue.as<unsigned long long>();
       a.q.tail = c + 0;
       a.q.head = c + 1;
       a.q.final_tail = c + 2;
       a.q.done = reinterpret_cast<unsigned int*>(c + 3);
       a.q.dbg = c + 4;
-      a.q.turn = reinterpret_cast<unsigned int*>(ctx->d_queue + 64);
-      a.q.state = reinterpret_cast<uint32_t*>(ctx->d_queue + 64 + 4 * n);
-      a.q.items = reinterpret_cast<unsigned long long*>(ctx->d_queue + 64 + 24 * n);
+      a.q.turn = reinterpret_cast<unsigned int*>(ctx->d_queue.p + 64);
+      a.q.state = reinterpret_cast<uint32_t*>(ctx->d_queue.p + 64 + 4 * n);
+      a.q.items = reinterpret_cast<unsigned long long*>(ctx->d_queue.p + 64 + 24 * n);
       a.q.cap = qcap;
       a.q.seg_shift = sfb::Q_SEG_SHIFT;
       a.q.lag = sfb::Q_LAG;
     }
     const uint64_t groups = (cnt + 31) / 32;
     if (stream_mode) {
-      sfb::StreamArgs sa;
+      sfb::StreamArgs sa{};
       sa.src_base = src_base;
       sa.src_off = src_off;
       sa.src_len = src_len;
@@ -739,28 +725,17 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
       sa.dst_cap = dst_cap;
       sa.status = status;
       sa.written = written;
-      sa.list = nullptr;
       sa.idx_base = first;
       sa.n = cnt;
       sa.stream_counter = ctr + 0;
-      sa.lens_scratch = ctx->d_lens;
-      sa.match_bits = ctx->d_bits;
-      sa.mode = 0;
-      sa.jobs = nullptr;
-      sa.job_count = nullptr;
-      sa.job_cap = 0;
-      sa.job_tab = nullptr;
-      sa.tab_mask = 0;
-      sa.tail_job = nullptr;
-      sa.recs = nullptr;
-      sa.rec_count = nullptr;
-      sa.rec_cap = 0;
+      sa.lens_scratch = ctx->d_lens.as<uint32_t>();
+      sa.match_bits = match_bits;
       sa.end_bit = resume && resume->end ? resume->blk_end : nullptr;
       const uint64_t resident =
           static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->stream_ctas_per_sm);
       if (blocks) {
         // find block starts | count each candidate block | chain | write the chained blocks
-        uint32_t* const counters = reinterpret_cast<uint32_t*>(ctx->d_find);  // cand_count, job_count, tail_job
+        uint32_t* const counters = ctx->d_find.as<uint32_t>();  // cand_count, job_count, tail_job
         sfb::FindArgs f;
         f.src_base = src_base;
         f.src_off = src_off;
@@ -771,9 +746,9 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
         f.tail_job = counters + 2;
         f.job_tab = counters + 16;
         f.tab_mask = tab_size - 1;
-        f.jobs = reinterpret_cast<sfb::BlockJob*>(ctx->d_find + 64 + 4ull * tab_size);
+        f.jobs = reinterpret_cast<sfb::BlockJob*>(ctx->d_find.p + 64 + 4ull * tab_size);
         f.job_cap = job_cap;
-        f.cand = reinterpret_cast<uint64_t*>(ctx->d_find + 64 + 4ull * tab_size +
+        f.cand = reinterpret_cast<uint64_t*>(ctx->d_find.p + 64 + 4ull * tab_size +
                                              sizeof(sfb::BlockJob) * static_cast<uint64_t>(job_cap));
         f.cand_cap = cand_cap;
         f.dst_cap = dst_cap;
@@ -798,7 +773,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
         for (uint64_t si = 0; si < cnt; ++si) {
           f.idx = first + si;
           sa.idx_base = first + si;
-          SFB_TRY(ctx, cudaMemsetAsync(ctx->d_find, 0, 64 + 4ull * tab_size, s1));
+          SFB_TRY(ctx, cudaMemsetAsync(ctx->d_find.p, 0, 64 + 4ull * tab_size, s1));
           if (si) SFB_TRY(ctx, cudaMemsetAsync(ctr, 0, 2 * sizeof(unsigned long long), s1));
           sfb::find_candidates_kernel<<<ctx->sm_count * 8, sfb::FIND_THREADS, 0, s1>>>(f);
           sfb::verify_candidates_kernel<<<ctx->sm_count * 4, sfb::FIND_THREADS, 0, s1>>>(f);
@@ -814,26 +789,26 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
         }
         ctx->launches += 5 * cnt;
       } else {
-        const unsigned grid = static_cast<unsigned>(cnt < resident ? cnt : resident);
+        const unsigned grid = grid_size(cnt, resident);
         sfb::huff_stream_kernel<StreamCfg><<<grid, 32, StreamCfg::SMEM_BYTES, s1>>>(sa);
         SFB_TRY(ctx, cudaGetLastError());
         ctx->launches += 1;
       }
     } else if (use_small) {
       a.group_counter = ctr + 0;
-      a.defer_list = ctx->d_defer + first;
+      a.defer_list = ctx->d_defer.as<uint32_t>() + first;
       a.defer_count = ctr + 3;
       const uint64_t want = (groups + SmallCfg::WARPS - 1) / SmallCfg::WARPS;
       const uint64_t resident =
           static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->small_ctas_per_sm);
-      const unsigned grid = static_cast<unsigned>(want < resident ? want : resident);
+      const unsigned grid = grid_size(want, resident);
       sfb::huff_lanes_kernel<SmallCfg><<<grid, SmallCfg::WARPS * 32, SmallCfg::SMEM_BYTES, s1>>>(a);
       SFB_TRY(ctx, cudaGetLastError());
       ctx->launches += 1;
       // the streams it handed on (none for low-entropy data: this launch then ends at once)
       a.defer_list = nullptr;
       a.defer_count = nullptr;
-      a.todo_list = ctx->d_defer + first;
+      a.todo_list = ctx->d_defer.as<uint32_t>() + first;
       a.todo_count = ctr + 3;
     }
     if (!stream_mode) {
@@ -841,20 +816,14 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
       const uint64_t want = (groups + LaneCfg::WARPS - 1) / LaneCfg::WARPS;
       const uint64_t resident =
           static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->ctas_per_sm);
-      const unsigned grid = static_cast<unsigned>(want < resident ? want : resident);
+      const unsigned grid = grid_size(want, resident);
       // (a batch that fits the lanes of the wide geometry takes it: see WideCfg)
       const uint64_t wide_resident =
           static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->wide_ctas_per_sm);
       if (qmode) {
         sfb::huff_lanes_kernel<LaneCfg, false, true><<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, s1>>>(a);
       } else if (resume && resume->end) {
-        auto kern = sfb::huff_lanes_kernel<LaneCfg, false, false, true>;
-        if (!ctx->end_configured) {  // (function attributes are per device)
-          SFB_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, LaneCfg::SMEM_BYTES));
-          cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-          ctx->end_configured = true;
-        }
-        kern<<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, s1>>>(a);
+        sfb::huff_lanes_kernel<LaneCfg, false, false, true><<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, s1>>>(a);
       } else if (!use_small && n_waves == 1 && wide_resident != 0 && want <= wide_resident)
         sfb::huff_lanes_kernel<WideCfg><<<static_cast<unsigned>(want), WideCfg::WARPS * 32, WideCfg::SMEM_BYTES, s1>>>(a);
       else
@@ -873,7 +842,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
     r.dst_delta = delta;
     r.dst_off = dst_off;
     r.written = written;
-    r.match_bits = ctx->d_bits;
+    r.match_bits = match_bits;
     r.n = cnt;
     r.idx_base = first;
     r.todo_list = order;
@@ -905,8 +874,8 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
       j.dst_delta = delta;
       j.dst_off = dst_off;
       j.written = written;
-      j.match_bits = ctx->d_bits;
-      j.ptr = reinterpret_cast<uint32_t*>(ctx->d_jump);
+      j.match_bits = match_bits;
+      j.ptr = ctx->d_jump.as<uint32_t>();
       j.tile_done = j.ptr + jump_tiles * sfb::JUMP_TILE;
       j.todo = j.tile_done + jump_tiles;
       const uint64_t stripes = (jump_tiles + stripe_tiles - 1) / stripe_tiles;
@@ -925,7 +894,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
           j.tile_hi = static_cast<uint32_t>(std::min<uint64_t>(jump_tiles, (sp + 1) * stripe_tiles));
           j.todo = todo0 + sp * (sfb::JUMP_MAX_ROUNDS + 1);
           const uint64_t want = (j.tile_hi - j.tile_lo + wpc - 1) / wpc;
-          return static_cast<unsigned>(want < resident ? want : resident);
+          return grid_size(want, resident);
         };
         j.round = 0;
         sfb::lz_jump_init_kernel<<<set_stripe(0), sfb::JUMP_THREADS, 0, s2>>>(j);
@@ -956,7 +925,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
       const uint64_t resident =
           static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->lz_ctas_per_sm);
       const uint64_t want = (cnt + wpc - 1) / wpc;
-      const unsigned grid = static_cast<unsigned>(want < resident ? want : resident);
+      const unsigned grid = grid_size(want, resident);
       if (ctx->lz_v1) sfb::lz_resolve_kernel<<<grid, sfb::LZ_THREADS, 0, s2>>>(r);
       else if (ctx->lzw_minb == 4) sfb::lz_window_kernel<4><<<grid, sfb::LZW_THREADS, 0, s2>>>(r);
       else if (ctx->lzw_minb == 5 && ctx->lzw_pf) sfb::lz_window_kernel<5, true><<<grid, sfb::LZW_THREADS, 0, s2>>>(r);
@@ -979,7 +948,7 @@ int batch_device_impl(sfb200_ctx* ctx, const uint8_t* src_base, const uint64_t* 
     //  lzq_give_up — fails the call instead of leaving matches unresolved behind a success)
     unsigned long long q8[8] = {0};
     SFB_TRY(ctx, cudaStreamSynchronize(st));
-    SFB_TRY(ctx, cudaMemcpy(q8, ctx->d_queue, sizeof(q8), cudaMemcpyDeviceToHost));
+    SFB_TRY(ctx, cudaMemcpy(q8, ctx->d_queue.p, sizeof(q8), cudaMemcpyDeviceToHost));
     if (q8[4] != 0ull) {
       ctx->err = "queue mode: a pass-2 consumer gave up waiting (" + std::string(q8[4] == 1ull ? "for an item" : "for its turn") +
                  ", " + std::to_string(q8[5]) + " / " + std::to_string(q8[6]) + " / " + std::to_string(q8[7]) + ")";
@@ -1004,42 +973,24 @@ int sfb200_decompressed_size_batch_device(sfb200_ctx* ctx, const uint8_t* src_ba
   SFB_ENTER(ctx);
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
   ctx->ev_valid = false;
-  SFB_TRY(ctx, cudaMemsetAsync(ctx->d_counter, 0, kCountersPerWave * sizeof(unsigned long long), st));
+  unsigned long long* const ctrs = ctx->d_counter.as<unsigned long long>();
+  SFB_TRY(ctx, cudaMemsetAsync(ctrs, 0, kCountersPerWave * sizeof(unsigned long long), st));
+  // (the counting writer never touches dst, its capacities or the bitmap: they stay null)
   sfb::BatchArgs a{};
   a.src_base = src_base;
   a.src_off = src_off;
   a.src_len = src_len;
-  a.dst_base = nullptr;  // the counting writer never touches dst, its capacities or the bitmap
-  a.dst_delta = 0;
-  a.dst_off = nullptr;
-  a.dst_cap = nullptr;
   a.status = status;
   a.written = size;
   a.n = n;
-  a.idx_base = 0;
-  a.group_counter = ctx->d_counter + 1;
-  a.lens_scratch = ctx->d_lens;
-  a.match_bits = nullptr;
-  a.defer_list = nullptr;
-  a.defer_count = nullptr;
-  a.todo_list = nullptr;
-  a.todo_count = nullptr;
+  a.group_counter = ctrs + 1;
+  a.lens_scratch = ctx->d_lens.as<uint32_t>();
   a.no_pair = ctx->no_pair;
-  a.handled = nullptr;
-  a.start_bit = nullptr;
-  a.start_out = nullptr;
-  a.blk_end = nullptr;
-  auto kern = sfb::huff_lanes_kernel<LaneCfg, true>;
-  if (!ctx->count_configured) {  // (function attributes are per device)
-    SFB_TRY(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, LaneCfg::SMEM_BYTES));
-    cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    ctx->count_configured = true;
-  }
   const uint64_t groups = (n + 31) / 32;
   const uint64_t want = (groups + LaneCfg::WARPS - 1) / LaneCfg::WARPS;
   const uint64_t resident = static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->ctas_per_sm);
-  const unsigned grid = static_cast<unsigned>(want < resident ? want : resident);
-  kern<<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, st>>>(a);
+  const unsigned grid = grid_size(want, resident);
+  sfb::huff_lanes_kernel<LaneCfg, true><<<grid, LaneCfg::WARPS * 32, LaneCfg::SMEM_BYTES, st>>>(a);
   SFB_TRY(ctx, cudaGetLastError());
   ctx->launches += 1;
   return SFB200_RC_OK;
@@ -1159,30 +1110,32 @@ int sfb200_decompress_batch_host(sfb200_ctx* ctx, const uint8_t* src, uint64_t s
   if (slot_dst > ctx->st_dst_cap || slot_src > ctx->st_src_cap) {
     sync_all();
     for (int k = 0; k < S; ++k) {
-      if (ctx->st_src[k]) SFB_TRY(ctx, cudaFree(ctx->st_src[k]));
-      if (ctx->st_dst[k]) SFB_TRY(ctx, cudaFree(ctx->st_dst[k]));
-      ctx->st_src[k] = ctx->st_dst[k] = nullptr;
+      ctx->st_src[k].release();
+      ctx->st_dst[k].release();
     }
     ctx->st_slots = 0;
     ctx->st_src_cap = std::max(slot_src, ctx->st_src_cap);
     ctx->st_dst_cap = std::max(slot_dst, ctx->st_dst_cap);
   }
+  int rc = SFB200_RC_OK;
   for (; ctx->st_slots < need_slots; ++ctx->st_slots) {
     const int k = ctx->st_slots;
-    SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->st_src[k]), ctx->st_src_cap + 64));
-    SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->st_dst[k]), ctx->st_dst_cap + 64));
+    rc = reserve(ctx, ctx->st_src[k], ctx->st_src_cap + 64, 0, true);
+    if (rc == SFB200_RC_OK) rc = reserve(ctx, ctx->st_dst[k], ctx->st_dst_cap + 64, 0, true);
+    if (rc != SFB200_RC_OK) return rc;
   }
   if (want_n > ctx->st_meta_n) {
     sync_all();
     for (int k = 0; k < S; ++k) {
-      if (ctx->st_meta[k]) SFB_TRY(ctx, cudaFree(ctx->st_meta[k]));
+      ctx->st_meta[k].release();
       if (ctx->st_hmeta[k]) SFB_TRY(ctx, cudaFreeHost(ctx->st_hmeta[k]));
-      ctx->st_meta[k] = ctx->st_hmeta[k] = nullptr;
+      ctx->st_hmeta[k] = nullptr;
     }
     ctx->st_meta_n = 0;
     const uint64_t cap = want_n + want_n / 8 + 64;
     for (int k = 0; k < S; ++k) {
-      SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->st_meta[k]), cap * (5 * 8 + 1) + 64));
+      rc = reserve(ctx, ctx->st_meta[k], cap * (5 * 8 + 1) + 64, 0, true);
+      if (rc != SFB200_RC_OK) return rc;
       SFB_TRY(ctx, cudaMallocHost(reinterpret_cast<void**>(&ctx->st_hmeta[k]), cap * (5 * 8 + 1) + 64));
     }
     ctx->st_meta_n = cap;
@@ -1203,25 +1156,11 @@ int sfb200_decompress_batch_host(sfb200_ctx* ctx, const uint8_t* src, uint64_t s
       big = std::max(big, sb.dst_hi - sb.dst_lo);
       big_n = std::max(big_n, sb.count);
     }
-    const uint64_t bits_words = (big + 128) / 32 + 8;
-    if (bits_words > ctx->d_bits_words) {
-      sync_all();
-      if (ctx->d_bits) SFB_TRY(ctx, cudaFree(ctx->d_bits));
-      ctx->d_bits = nullptr;
-      ctx->d_bits_words = 0;
-      const uint64_t want = bits_words + bits_words / 8 + 64;
-      SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_bits), want * sizeof(uint32_t)));
-      ctx->d_bits_words = want;
-    }
-    if (big_n > ctx->d_order_n) {
-      sync_all();
-      if (ctx->d_order) SFB_TRY(ctx, cudaFree(ctx->d_order));
-      ctx->d_order = nullptr;
-      ctx->d_order_n = 0;
-      const uint64_t want = big_n + big_n / 8 + 64;
-      SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&ctx->d_order), want * (sizeof(uint32_t) + 1)));
-      ctx->d_order_n = want;
-    }
+    const uint64_t bits = bitmap_bytes(big, 127), order = big_n * kOrderBytes;
+    if (bits > ctx->d_bits.cap || order > ctx->d_order.cap) sync_all();
+    rc = reserve(ctx, ctx->d_bits, bits);
+    if (rc == SFB200_RC_OK) rc = reserve(ctx, ctx->d_order, order);
+    if (rc != SFB200_RC_OK) return rc;
   }
   auto cleanup = [&](int code) {
     sync_all();
@@ -1233,7 +1172,7 @@ int sfb200_decompress_batch_host(sfb200_ctx* ctx, const uint8_t* src, uint64_t s
     if (e_ != cudaSuccess) return cleanup(fail(ctx, e_, #call)); \
   } while (0)
   // slot k % S: device arrays and their pinned mirror
-  auto d_arr = [&](int slot, int which) { return ctx->st_meta[slot] + static_cast<uint64_t>(which) * cap_n; };
+  auto d_arr = [&](int slot, int which) { return ctx->st_meta[slot].as<uint64_t>() + static_cast<uint64_t>(which) * cap_n; };
   auto h_arr = [&](int slot, int which) { return ctx->st_hmeta[slot] + static_cast<uint64_t>(which) * cap_n; };
   auto enqueue = [&](size_t k) -> int {
     const Sub& sb = subs[k];
@@ -1251,16 +1190,16 @@ int sfb200_decompress_batch_host(sfb200_ctx* ctx, const uint8_t* src, uint64_t s
       h_dc[j] = dst_cap[f + j];
     }
     if (sb.src_hi > sb.src_lo)
-      SFB_TRYC(cudaMemcpyAsync(ctx->st_src[slot], src + sb.src_lo, sb.src_hi - sb.src_lo, cudaMemcpyHostToDevice, s_in));
+      SFB_TRYC(cudaMemcpyAsync(ctx->st_src[slot].p, src + sb.src_lo, sb.src_hi - sb.src_lo, cudaMemcpyHostToDevice, s_in));
     // (the four arrays are contiguous in both mirrors when c == cap_n; copy them one by one)
     for (int w = 0; w < 4; ++w)
       SFB_TRYC(cudaMemcpyAsync(d_arr(slot, w), h_arr(slot, w), c * 8, cudaMemcpyHostToDevice, s_in));
     SFB_TRYC(cudaEventRecord(ctx->st_ev[slot][0], s_in));
     SFB_TRYC(cudaStreamWaitEvent(s_run, ctx->st_ev[slot][0], 0));
     uint8_t* const d_status = reinterpret_cast<uint8_t*>(d_arr(slot, 5));
-    const int r = sfb200_decompress_batch_device(ctx, ctx->st_src[slot], d_arr(slot, 0), d_arr(slot, 1), ctx->st_dst[slot],
-                                                 sb.dst_hi - sb.dst_lo, d_arr(slot, 2), d_arr(slot, 3), d_status,
-                                                 d_arr(slot, 4), c, s_run);
+    const int r = sfb200_decompress_batch_device(ctx, ctx->st_src[slot].p, d_arr(slot, 0), d_arr(slot, 1),
+                                                 ctx->st_dst[slot].p, sb.dst_hi - sb.dst_lo, d_arr(slot, 2),
+                                                 d_arr(slot, 3), d_status, d_arr(slot, 4), c, s_run);
     if (r) return cleanup(r);
     SFB_TRYC(cudaEventRecord(ctx->st_ev[slot][1], s_run));
     SFB_TRYC(cudaStreamWaitEvent(s_meta, ctx->st_ev[slot][1], 0));
@@ -1269,7 +1208,6 @@ int sfb200_decompress_batch_host(sfb200_ctx* ctx, const uint8_t* src, uint64_t s
     SFB_TRYC(cudaEventRecord(ctx->st_ev[slot][2], s_meta));
     return SFB200_RC_OK;
   };
-  int rc = SFB200_RC_OK;
   size_t enq = 0;
   for (; enq < subs.size() && enq < static_cast<size_t>(S) - 1; ++enq) {
     rc = enqueue(enq);
@@ -1292,7 +1230,7 @@ int sfb200_decompress_batch_host(sfb200_ctx* ctx, const uint8_t* src, uint64_t s
     uint64_t run_lo = 0, run_hi = 0;  // pending run [run_lo, run_hi) of produced bytes (caller's offsets)
     auto flush_run = [&]() -> int {
       if (run_hi > run_lo)
-        SFB_TRYC(cudaMemcpyAsync(dst + run_lo, ctx->st_dst[slot] + (run_lo - sb.dst_lo), run_hi - run_lo,
+        SFB_TRYC(cudaMemcpyAsync(dst + run_lo, ctx->st_dst[slot].p + (run_lo - sb.dst_lo), run_hi - run_lo,
                                  cudaMemcpyDeviceToHost, s_out));
       run_lo = run_hi = 0;
       return SFB200_RC_OK;
@@ -1403,34 +1341,20 @@ int sfb200_decompress(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8
 // buffer, so that distances reach into it as they would in one call).
 struct sfb200_inflate_stream {
   sfb200_ctx* ctx = nullptr;
-  uint8_t* d_in[2] = {nullptr, nullptr};   // buffered input (the other one is the target of the next compaction)
-  uint64_t d_in_cap[2] = {0, 0};
+  DevBuf d_in[2];          // buffered input (the other one is the target of the next compaction)
   int cur = 0;
   uint64_t in_len = 0;     // bytes buffered
   uint64_t bit = 0;        // bit offset of the next block header inside the buffer (0..7 between calls)
-  uint8_t* d_out = nullptr;   // [32 KiB window | output of one call]
-  uint64_t d_out_cap = 0;
-  uint8_t* d_tmp = nullptr;   // 32 KiB (window moves that overlap)
+  DevBuf d_out;            // [32 KiB window | output of one call]
+  DevBuf d_tmp;            // 32 KiB (window moves that overlap)
   uint64_t hist = 0;       // valid window bytes, right-aligned in the first 32 KiB of d_out
-  uint64_t* d_meta = nullptr;  // src_off, src_len, dst_off, dst_cap, written, start_bit, start_out, blk_end[2], status
+  DevBuf d_meta;           // u64: src_off, src_len, dst_off, dst_cap, written, start_bit, start_out, blk_end[2], status
   bool finished = false;
   uint8_t final_status = 0;
 };
 
 namespace {
 constexpr uint64_t kWindow = 32768;
-int keep_bytes(sfb200_ctx* ctx, uint8_t** p, uint64_t* cap, uint64_t need, uint64_t keep)
-{
-  if (need <= *cap) return SFB200_RC_OK;
-  uint8_t* q = nullptr;
-  const uint64_t want = need + need / 2 + 4096;
-  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&q), want));
-  if (keep) SFB_TRY(ctx, cudaMemcpy(q, *p, keep, cudaMemcpyDeviceToDevice));
-  if (*p) SFB_TRY(ctx, cudaFree(*p));
-  *p = q;
-  *cap = want;
-  return SFB200_RC_OK;
-}
 }  // namespace
 
 int sfb200_inflate_stream_create(sfb200_ctx* ctx, sfb200_inflate_stream** out)
@@ -1440,12 +1364,12 @@ int sfb200_inflate_stream_create(sfb200_ctx* ctx, sfb200_inflate_stream** out)
   sfb200_inflate_stream* s = new (std::nothrow) sfb200_inflate_stream;
   if (!s) return SFB200_RC_OUT_OF_MEMORY;
   s->ctx = ctx;
-  if (cudaMalloc(reinterpret_cast<void**>(&s->d_tmp), kWindow) != cudaSuccess ||
-      cudaMalloc(reinterpret_cast<void**>(&s->d_meta), 16 * sizeof(uint64_t)) != cudaSuccess) {
-    cudaFree(s->d_tmp);
+  int rc = reserve(ctx, s->d_tmp, kWindow, 0, true);
+  if (rc == SFB200_RC_OK) rc = reserve(ctx, s->d_meta, 16 * sizeof(uint64_t), 0, true);
+  if (rc != SFB200_RC_OK) {
     delete s;
     cudaGetLastError();
-    return SFB200_RC_OUT_OF_MEMORY;
+    return rc;
   }
   *out = s;
   return SFB200_RC_OK;
@@ -1454,12 +1378,7 @@ int sfb200_inflate_stream_create(sfb200_ctx* ctx, sfb200_inflate_stream** out)
 void sfb200_inflate_stream_destroy(sfb200_inflate_stream* s)
 {
   if (!s) return;
-  DeviceGuard guard_(s->ctx->device);
-  cudaFree(s->d_in[0]);
-  cudaFree(s->d_in[1]);
-  cudaFree(s->d_out);
-  cudaFree(s->d_tmp);
-  cudaFree(s->d_meta);
+  DeviceGuard guard_(s->ctx->device);  // (its device memory is freed with it, on its device)
   delete s;
 }
 
@@ -1479,12 +1398,12 @@ int sfb200_inflate_stream_feed(sfb200_inflate_stream* s, const uint8_t* src, siz
   *status = SFB200_SUCCESS;
   if (s->in_len + src_len >= 0xffffff00ull || kWindow + dst_cap >= 0xffffff00ull) return SFB200_RC_BAD_ARGUMENT;
   // the new input goes behind what is buffered
-  int rc = keep_bytes(ctx, &s->d_in[s->cur], &s->d_in_cap[s->cur], s->in_len + src_len + 64, s->in_len);
+  int rc = reserve(ctx, s->d_in[s->cur], s->in_len + src_len + 64, s->in_len);
   if (rc != SFB200_RC_OK) return rc;
-  if (src_len) SFB_TRY(ctx, cudaMemcpy(s->d_in[s->cur] + s->in_len, src, src_len, cudaMemcpyHostToDevice));
+  if (src_len) SFB_TRY(ctx, cudaMemcpy(s->d_in[s->cur].p + s->in_len, src, src_len, cudaMemcpyHostToDevice));
   s->in_len += src_len;
   if (dst_cap == 0 && !last) return SFB200_RC_OK;  // (only buffering)
-  rc = keep_bytes(ctx, &s->d_out, &s->d_out_cap, kWindow + dst_cap + 256, s->d_out ? kWindow : 0);
+  rc = reserve(ctx, s->d_out, kWindow + dst_cap + 256, s->d_out.p ? kWindow : 0);
   if (rc != SFB200_RC_OK) return rc;
   // one lane-kernel decode from the pending block header, behind the window
   uint64_t h[16] = {0};
@@ -1498,15 +1417,16 @@ int sfb200_inflate_stream_feed(sfb200_inflate_stream* s, const uint8_t* src, siz
   h[7] = s->bit;                   // blk_end: bit, output position (stay like this when no header is reached)
   h[8] = s->hist;
   h[9] = SFB200_ERROR;             // status (first byte)
-  SFB_TRY(ctx, cudaMemcpy(s->d_meta, h, sizeof h, cudaMemcpyHostToDevice));
+  uint64_t* const m = s->d_meta.as<uint64_t>();
+  SFB_TRY(ctx, cudaMemcpy(m, h, sizeof h, cudaMemcpyHostToDevice));
   Resume rs;
-  rs.start_bit = s->d_meta + 5;
-  rs.start_out = s->d_meta + 6;
-  rs.blk_end = s->d_meta + 7;
-  rc = batch_device_impl(ctx, s->d_in[s->cur], s->d_meta + 0, s->d_meta + 1, s->d_out, kWindow + dst_cap, s->d_meta + 2,
-                         s->d_meta + 3, reinterpret_cast<uint8_t*>(s->d_meta + 9), s->d_meta + 4, 1, nullptr, &rs);
+  rs.start_bit = m + 5;
+  rs.start_out = m + 6;
+  rs.blk_end = m + 7;
+  rc = batch_device_impl(ctx, s->d_in[s->cur].p, m + 0, m + 1, s->d_out.p, kWindow + dst_cap, m + 2, m + 3,
+                         reinterpret_cast<uint8_t*>(m + 9), m + 4, 1, nullptr, &rs);
   if (rc != SFB200_RC_OK) return rc;
-  SFB_TRY(ctx, cudaMemcpy(h, s->d_meta, sizeof h, cudaMemcpyDeviceToHost));
+  SFB_TRY(ctx, cudaMemcpy(h, m, sizeof h, cudaMemcpyDeviceToHost));
   const uint8_t st = static_cast<uint8_t>(h[9] & 0xffu);
   const uint64_t total = h[4], be_bit = h[7], be_out = h[8];
   uint64_t produced = 0;
@@ -1525,20 +1445,20 @@ int sfb200_inflate_stream_feed(sfb200_inflate_stream* s, const uint8_t* src, siz
     produced = be_out - s->hist;
     s->bit = be_bit;
   }
-  if (produced) SFB_TRY(ctx, cudaMemcpy(dst, s->d_out + kWindow, produced, cudaMemcpyDeviceToHost));
+  if (produced) SFB_TRY(ctx, cudaMemcpy(dst, s->d_out.p + kWindow, produced, cudaMemcpyDeviceToHost));
   *written = produced;
   if (!s->finished) {
     // the window: the last 32 KiB of everything produced so far
     const uint64_t have = s->hist + produced;
     const uint64_t keep = have < kWindow ? have : kWindow;
     if (produced) {
-      const uint8_t* from = s->d_out + kWindow + produced - keep;
-      uint8_t* to = s->d_out + kWindow - keep;
+      const uint8_t* from = s->d_out.p + kWindow + produced - keep;
+      uint8_t* to = s->d_out.p + kWindow - keep;
       if (produced >= kWindow) {
         SFB_TRY(ctx, cudaMemcpy(to, from, keep, cudaMemcpyDeviceToDevice));
       } else {
-        SFB_TRY(ctx, cudaMemcpy(s->d_tmp, from, keep, cudaMemcpyDeviceToDevice));
-        SFB_TRY(ctx, cudaMemcpy(to, s->d_tmp, keep, cudaMemcpyDeviceToDevice));
+        SFB_TRY(ctx, cudaMemcpy(s->d_tmp.p, from, keep, cudaMemcpyDeviceToDevice));
+        SFB_TRY(ctx, cudaMemcpy(to, s->d_tmp.p, keep, cudaMemcpyDeviceToDevice));
       }
     }
     s->hist = keep;
@@ -1547,9 +1467,9 @@ int sfb200_inflate_stream_feed(sfb200_inflate_stream* s, const uint8_t* src, siz
     if (drop) {
       const int other = s->cur ^ 1;
       const uint64_t rest = s->in_len - drop;
-      rc = keep_bytes(ctx, &s->d_in[other], &s->d_in_cap[other], rest + 64, 0);
+      rc = reserve(ctx, s->d_in[other], rest + 64);
       if (rc != SFB200_RC_OK) return rc;
-      if (rest) SFB_TRY(ctx, cudaMemcpy(s->d_in[other], s->d_in[s->cur] + drop, rest, cudaMemcpyDeviceToDevice));
+      if (rest) SFB_TRY(ctx, cudaMemcpy(s->d_in[other].p, s->d_in[s->cur].p + drop, rest, cudaMemcpyDeviceToDevice));
       s->cur = other;
       s->in_len = rest;
       s->bit &= 7u;
@@ -1577,16 +1497,7 @@ int sfb200_compress_batch_device(sfb200_ctx* ctx, const uint8_t* src_base, const
   if (!src_off || !src_len || !dst_off || !dst_cap || !status || !written) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-  if (!ctx->compress_configured) {  // (function attributes are per device)
-    SFB_TRY(ctx, cudaFuncSetAttribute(sfb::deflate_compress_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      sfb::CMP_SMEM_BYTES));
-    int per_sm = 0;
-    SFB_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sfb::deflate_compress_kernel,
-                                                               sfb::CMP_WARPS * 32, sfb::CMP_SMEM_BYTES));
-    ctx->compress_ctas_per_sm = per_sm < 1 ? 1 : per_sm;
-    ctx->compress_configured = true;
-  }
-  SFB_TRY(ctx, cudaMemsetAsync(ctx->d_counter, 0, sizeof(unsigned long long), st));
+  SFB_TRY(ctx, cudaMemsetAsync(ctx->d_counter.p, 0, sizeof(unsigned long long), st));
   sfb::CompressArgs a;
   a.src_base = src_base;
   a.src_off = src_off;
@@ -1597,13 +1508,12 @@ int sfb200_compress_batch_device(sfb200_ctx* ctx, const uint8_t* src_base, const
   a.status = status;
   a.written = written;
   a.n = n;
-  a.counter = ctx->d_counter;
+  a.counter = ctx->d_counter.as<unsigned long long>();
   a.fixed_only = 0;   // SFB200_COMPRESS_FIXED=1: the first generation (one pass, fixed-Huffman blocks only) for A/B runs
   if (const char* e = std::getenv("SFB200_COMPRESS_FIXED")) a.fixed_only = e[0] == '1';
   const uint64_t want = (n + sfb::CMP_WARPS - 1) / sfb::CMP_WARPS;
   const uint64_t resident = static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->compress_ctas_per_sm);
-  sfb::deflate_compress_kernel<<<static_cast<unsigned>(want < resident ? want : resident), sfb::CMP_WARPS * 32,
-                                 sfb::CMP_SMEM_BYTES, st>>>(a);
+  sfb::deflate_compress_kernel<<<grid_size(want, resident), sfb::CMP_WARPS * 32, sfb::CMP_SMEM_BYTES, st>>>(a);
   SFB_TRY(ctx, cudaGetLastError());
   ctx->launches += 1;
   return SFB200_RC_OK;
@@ -1612,34 +1522,8 @@ int sfb200_compress_batch_device(sfb200_ctx* ctx, const uint8_t* src_base, const
 int sfb200_compress(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* dst, size_t dst_cap,
                     uint8_t* status, uint64_t* written)
 {
-  if (!ctx || !status || !written || (src_len && !src) || (dst_cap && !dst)) return SFB200_RC_BAD_ARGUMENT;
-  SFB_ENTER(ctx);
-  uint8_t* buf = nullptr;
-  const uint64_t in_pad = (static_cast<uint64_t>(src_len) + 255) & ~255ull;
-  const uint64_t total = in_pad + dst_cap + 256 + 64;
-  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&buf), total));
-  auto done = [&](int rc) {
-    cudaFree(buf);
-    return rc;
-  };
-  uint64_t h[6] = {0, src_len, 0, dst_cap, 0, 0};
-  uint64_t* meta = reinterpret_cast<uint64_t*>(buf + in_pad + ((dst_cap + 255) & ~255ull));
-  if (src_len && cudaMemcpy(buf, src, src_len, cudaMemcpyHostToDevice) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(src)"));
-  if (cudaMemcpy(meta, h, sizeof h, cudaMemcpyHostToDevice) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(meta)"));
-  int rc = sfb200_compress_batch_device(ctx, buf, meta + 0, meta + 1, buf + in_pad, meta + 2, meta + 3,
-                                        reinterpret_cast<uint8_t*>(meta + 5), meta + 4, 1, nullptr);
-  if (rc != SFB200_RC_OK) return done(rc);
-  if (cudaMemcpy(h, meta, sizeof h, cudaMemcpyDeviceToHost) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(meta back)"));
-  *status = static_cast<uint8_t>(h[5] & 0xffu);
-  *written = h[4];
-  if (h[4] && cudaMemcpy(dst, buf + in_pad, h[4], cudaMemcpyDeviceToHost) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(dst)"));
-  return done(SFB200_RC_OK);
+  return sfb200_compress_container(ctx, SFB200_CONTAINER_RAW, src, src_len, dst, dst_cap, status, written);
 }
-
 
 int sfb200_decompress_container_batch_device(sfb200_ctx* ctx, int container, const uint8_t* src_base,
                                              const uint64_t* src_off, const uint64_t* src_len,
@@ -1656,7 +1540,7 @@ int sfb200_decompress_container_batch_device(sfb200_ctx* ctx, int container, con
                                           status, written, n, cuda_stream);
   SFB_ENTER(ctx);
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-  int rc = grow(ctx, &ctx->d_cont, &ctx->d_cont_cap, n * 36 + 64);
+  int rc = reserve(ctx, ctx->d_cont, n * 36 + 64);
   if (rc != SFB200_RC_OK) return rc;
   sfb::ContainerArgs c;
   c.src_base = src_base;
@@ -1664,7 +1548,7 @@ int sfb200_decompress_container_batch_device(sfb200_ctx* ctx, int container, con
   c.src_len = src_len;
   c.container = static_cast<uint32_t>(container);
   c.n = n;
-  c.pay_off = reinterpret_cast<uint64_t*>(ctx->d_cont);
+  c.pay_off = ctx->d_cont.as<uint64_t>();
   c.pay_len = c.pay_off + n;
   uint64_t* const own_written = c.pay_len + n;
   c.kind = reinterpret_cast<uint32_t*>(own_written + n);
@@ -1680,15 +1564,9 @@ int sfb200_decompress_container_batch_device(sfb200_ctx* ctx, int container, con
   rc = sfb200_decompress_batch_device(ctx, src_base, c.pay_off, c.pay_len, dst_base, dst_bytes, dst_off, dst_cap,
                                       status, c.written, n, cuda_stream);
   if (rc != SFB200_RC_OK) return rc;
-  if (!ctx->check_configured) {  // (function attributes are per device)
-    SFB_TRY(ctx, cudaFuncSetAttribute(sfb::container_check_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      sfb::CHECK_SMEM_BYTES));
-    ctx->check_configured = true;
-  }
   const uint64_t want = (n * 32 + sfb::CHECK_THREADS - 1) / sfb::CHECK_THREADS;
   const uint64_t resident = static_cast<uint64_t>(ctx->sm_count);  // (one block per SM: 128 KiB of tables)
-  sfb::container_check_kernel<<<static_cast<unsigned>(want < resident ? want : resident), sfb::CHECK_THREADS,
-                                sfb::CHECK_SMEM_BYTES, st>>>(c);
+  sfb::container_check_kernel<<<grid_size(want, resident), sfb::CHECK_THREADS, sfb::CHECK_SMEM_BYTES, st>>>(c);
   SFB_TRY(ctx, cudaGetLastError());
   ctx->launches += 2;
   return SFB200_RC_OK;
@@ -1699,28 +1577,12 @@ int sfb200_decompress_container(sfb200_ctx* ctx, int container, const uint8_t* s
 {
   if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
-  const uint64_t meta_at = (static_cast<uint64_t>(src_len) + 15) & ~15ull;
-  int rc = grow(ctx, &ctx->d_src, &ctx->d_src_cap, meta_at + 64);
-  if (rc != SFB200_RC_OK) return rc;
-  rc = grow(ctx, &ctx->d_dst, &ctx->d_dst_cap, static_cast<uint64_t>(dst_cap) + 64);
-  if (rc != SFB200_RC_OK) return rc;
-  // metadata behind the stream in the staging buffer: src_off, src_len, dst_off, dst_cap, written (u64), status (u8)
-  uint64_t meta[5] = {0, static_cast<uint64_t>(src_len), 0, static_cast<uint64_t>(dst_cap), 0};
-  uint64_t* const d_m = reinterpret_cast<uint64_t*>(ctx->d_src + meta_at);
-  uint8_t* const d_st = reinterpret_cast<uint8_t*>(d_m + 5);
-  if (src_len) SFB_TRY(ctx, cudaMemcpyAsync(ctx->d_src, src, src_len, cudaMemcpyHostToDevice, nullptr));
-  SFB_TRY(ctx, cudaMemcpyAsync(d_m, meta, sizeof(meta), cudaMemcpyHostToDevice, nullptr));
-  rc = sfb200_decompress_container_batch_device(ctx, container, ctx->d_src, d_m, d_m + 1, ctx->d_dst, dst_cap, d_m + 2,
-                                                d_m + 3, d_st, d_m + 4, 1, nullptr);
-  if (rc != SFB200_RC_OK) return rc;
-  uint64_t wr = 0;
-  SFB_TRY(ctx, cudaMemcpyAsync(&wr, d_m + 4, 8, cudaMemcpyDeviceToHost, nullptr));
-  SFB_TRY(ctx, cudaMemcpyAsync(status, d_st, 1, cudaMemcpyDeviceToHost, nullptr));
-  SFB_TRY(ctx, cudaStreamSynchronize(nullptr));
-  if (wr > dst_cap) return SFB200_RC_CUDA_ERROR;  // (cannot happen)
-  if (wr) SFB_TRY(ctx, cudaMemcpy(dst, ctx->d_dst, wr, cudaMemcpyDeviceToHost));  // only what was produced
-  if (written) *written = wr;
-  return SFB200_RC_OK;
+  return host_buffer_call(ctx, src, src_len, dst, dst_cap, written,
+                          [&](uint8_t* s, uint8_t* d, uint64_t* m, uint64_t* wr) {
+    const int rc = sfb200_decompress_container_batch_device(ctx, container, s, m, m + 1, d, dst_cap, m + 2, m + 3,
+                                                            reinterpret_cast<uint8_t*>(m + 5), m + 4, 1, nullptr);
+    return rc != SFB200_RC_OK ? rc : read_meta(ctx, m, wr, status);
+  });
 }
 
 int sfb200_decompressed_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* status,
@@ -1728,21 +1590,13 @@ int sfb200_decompressed_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len
 {
   if (!ctx || !status || !size || (!src && src_len)) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
-  int rc = grow(ctx, &ctx->d_src, &ctx->d_src_cap, static_cast<uint64_t>(src_len) + 64);
-  if (rc != SFB200_RC_OK) return rc;
-  // metadata lives behind the stream in the same staging buffer: off, len, size (u64), status (u8)
-  const uint64_t meta_at = (static_cast<uint64_t>(src_len) + 15) & ~15ull;
-  uint64_t meta[3] = {0, static_cast<uint64_t>(src_len), 0};
-  uint64_t* const d_m = reinterpret_cast<uint64_t*>(ctx->d_src + meta_at);
-  uint8_t* const d_st = reinterpret_cast<uint8_t*>(d_m + 3);
-  if (src_len) SFB_TRY(ctx, cudaMemcpyAsync(ctx->d_src, src, src_len, cudaMemcpyHostToDevice, nullptr));
-  SFB_TRY(ctx, cudaMemcpyAsync(d_m, meta, sizeof(meta), cudaMemcpyHostToDevice, nullptr));
-  rc = sfb200_decompressed_size_batch_device(ctx, ctx->d_src, d_m, d_m + 1, d_st, d_m + 2, 1, nullptr);
-  if (rc != SFB200_RC_OK) return rc;
-  SFB_TRY(ctx, cudaMemcpyAsync(size, d_m + 2, 8, cudaMemcpyDeviceToHost, nullptr));
-  SFB_TRY(ctx, cudaMemcpyAsync(status, d_st, 1, cudaMemcpyDeviceToHost, nullptr));
-  SFB_TRY(ctx, cudaStreamSynchronize(nullptr));
-  return SFB200_RC_OK;
+  // (the size goes to *size: no bytes of dst)
+  return host_buffer_call(ctx, src, src_len, nullptr, 0, nullptr,
+                          [&](uint8_t* s, uint8_t*, uint64_t* m, uint64_t*) {
+    const int rc = sfb200_decompressed_size_batch_device(ctx, s, m, m + 1, reinterpret_cast<uint8_t*>(m + 5), m + 4, 1,
+                                                         nullptr);
+    return rc != SFB200_RC_OK ? rc : read_meta(ctx, m, size, status);
+  });
 }
 
 }  // extern "C"
@@ -1767,20 +1621,24 @@ struct GzfResult {
   bool complete = false;
 };
 
+// members the table has room for: its columns (five of u64, then status) are strided by this
+uint64_t gzm_members(const sfb200_ctx* ctx) { return ctx->d_gzm.cap / kGzfMemberBytes; }
+
 // room for `need` members in the table, keeping the first `keep`
 int gzf_reserve(sfb200_ctx* ctx, uint64_t need, uint64_t keep, cudaStream_t st)
 {
-  if (need <= ctx->d_gzm_n) return SFB200_RC_OK;
-  const uint64_t cap = need + need / 2 + 64;
-  uint8_t* q = nullptr;
-  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&q), cap * kGzfMemberBytes));
+  const uint64_t old_n = gzm_members(ctx);
+  if (need <= old_n) return SFB200_RC_OK;
+  DevBuf q;
+  const int rc = reserve(ctx, q, (need + need / 2 + 64) * kGzfMemberBytes, 0, true);
+  if (rc != SFB200_RC_OK) return rc;
+  const uint64_t cap = q.cap / kGzfMemberBytes;
   if (keep)
     for (int w = 0; w < 5; ++w)
-      SFB_TRY(ctx, cudaMemcpyAsync(q + w * 8 * cap, ctx->d_gzm + w * 8 * ctx->d_gzm_n, keep * 8, cudaMemcpyDeviceToDevice, st));
+      SFB_TRY(ctx, cudaMemcpyAsync(q.p + w * 8 * cap, ctx->d_gzm.p + w * 8 * old_n, keep * 8, cudaMemcpyDeviceToDevice,
+                                   st));
   SFB_TRY(ctx, cudaStreamSynchronize(st));
-  if (ctx->d_gzm) SFB_TRY(ctx, cudaFree(ctx->d_gzm));
-  ctx->d_gzm = q;
-  ctx->d_gzm_n = cap;
+  ctx->d_gzm.swap(q);  // (q frees the old table)
   return SFB200_RC_OK;
 }
 
@@ -1796,13 +1654,13 @@ int gzip_file_impl(sfb200_ctx* ctx, const uint8_t* src, uint64_t len, uint8_t* d
   const uint64_t tile = static_cast<uint64_t>(sfb::GZF_THREADS) * sfb::GZF_BYTES;
   const uint64_t tiles = (len + (reinterpret_cast<uintptr_t>(src) & 15u) + tile - 1) / tile;
   // step (128 B) | result (2 x u64) | probe metadata (16 x u64) | tile counts (tiles + 1)
-  int rc = grow(ctx, &ctx->d_gzf, &ctx->d_gzf_cap, 128 + 16 + 128 + 8 * (tiles + 1));
+  int rc = reserve(ctx, ctx->d_gzf, 128 + 16 + 128 + 8 * (tiles + 1));
   if (rc != SFB200_RC_OK) return rc;
   sfb::GzfArgs a{};
   a.src = src;
   a.len = len;
-  a.step = reinterpret_cast<sfb::GzfStep*>(ctx->d_gzf);
-  uint64_t* const d_result = reinterpret_cast<uint64_t*>(ctx->d_gzf + 128);
+  a.step = ctx->d_gzf.as<sfb::GzfStep>();
+  uint64_t* const d_result = reinterpret_cast<uint64_t*>(ctx->d_gzf.p + 128);
   uint64_t* const pm = d_result + 2;
   a.tile_count = pm + 16;
   a.dst_cap = decode ? dst_cap : ~0ull;
@@ -1823,16 +1681,16 @@ int gzip_file_impl(sfb200_ctx* ctx, const uint8_t* src, uint64_t len, uint8_t* d
   if (const char* e = std::getenv("SFB200_GZIP_CHAIN"))  // (tests: =walk takes the fallback)
     if (e[0] == 'w') tables = 1;
   auto cand_bytes = [&](uint32_t t) { return 16 * m + 4 * (m + 1) * static_cast<uint64_t>(t) + 64; };
-  rc = grow(ctx, &ctx->d_gzc, &ctx->d_gzc_cap, cand_bytes(tables));
+  rc = reserve(ctx, ctx->d_gzc, cand_bytes(tables));
   if (rc == SFB200_RC_OUT_OF_MEMORY && tables > 1) {
     // no room for the jump tables: one thread walks the chain on J_0 instead — slower, same results
     cudaGetLastError();
     ctx->err.clear();
     tables = 1;
-    rc = grow(ctx, &ctx->d_gzc, &ctx->d_gzc_cap, cand_bytes(tables));
+    rc = reserve(ctx, ctx->d_gzc, cand_bytes(tables));
   }
   if (rc != SFB200_RC_OK) return rc;
-  a.cpos = reinterpret_cast<uint64_t*>(ctx->d_gzc);
+  a.cpos = ctx->d_gzc.as<uint64_t>();
   a.cnext = a.cpos + m;
   a.jump = reinterpret_cast<uint32_t*>(a.cnext + m);
   a.m = m;
@@ -1844,10 +1702,11 @@ int gzip_file_impl(sfb200_ctx* ctx, const uint8_t* src, uint64_t len, uint8_t* d
   SFB_TRY(ctx, cudaGetLastError());
   ctx->launches += 1 + tables;
   auto bind_members = [&]() {
-    a.mpos = reinterpret_cast<uint64_t*>(ctx->d_gzm);
-    a.mlen = a.mpos + ctx->d_gzm_n;
-    a.moff = a.mlen + ctx->d_gzm_n;
-    a.mcap = a.moff + ctx->d_gzm_n;
+    const uint64_t cap = gzm_members(ctx);
+    a.mpos = ctx->d_gzm.as<uint64_t>();
+    a.mlen = a.mpos + cap;
+    a.moff = a.mlen + cap;
+    a.mcap = a.moff + cap;
   };
   const unsigned skip_grid = static_cast<unsigned>(std::min<uint64_t>(tiles, static_cast<uint64_t>(ctx->sm_count) * 8));
   sfb::GzfStep h{};
@@ -1981,8 +1840,8 @@ int gzip_file_impl(sfb200_ctx* ctx, const uint8_t* src, uint64_t len, uint8_t* d
   res->complete = complete;
   if (!decode) return SFB200_RC_OK;
   // ---- the members side by side, then the file's result ------------------------------------------
-  uint8_t* const m_status = ctx->d_gzm + 40 * ctx->d_gzm_n;
-  uint64_t* const m_written = a.mcap + ctx->d_gzm_n;
+  uint8_t* const m_status = ctx->d_gzm.p + 40 * gzm_members(ctx);
+  uint64_t* const m_written = a.mcap + gzm_members(ctx);
   if (members) {
     rc = sfb200_decompress_container_batch_device(ctx, SFB200_CONTAINER_GZIP, src, a.mpos, a.mlen, dst, dst_cap, a.moff,
                                                   a.mcap, m_status, m_written, members, st);
@@ -2023,18 +1882,15 @@ int sfb200_decompress_gzip_file(sfb200_ctx* ctx, const uint8_t* src, size_t src_
 {
   if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
-  int rc = grow(ctx, &ctx->d_src, &ctx->d_src_cap, static_cast<uint64_t>(src_len) + 64);
-  if (rc != SFB200_RC_OK) return rc;
-  rc = grow(ctx, &ctx->d_dst, &ctx->d_dst_cap, static_cast<uint64_t>(dst_cap) + 64);
-  if (rc != SFB200_RC_OK) return rc;
-  if (src_len) SFB_TRY(ctx, cudaMemcpy(ctx->d_src, src, src_len, cudaMemcpyHostToDevice));
   GzfResult r;
-  rc = gzip_file_impl(ctx, ctx->d_src, src_len, ctx->d_dst, dst_cap, true, nullptr, &r);
+  const int rc = host_buffer_call(ctx, src, src_len, dst, dst_cap, written,
+                                  [&](uint8_t* s, uint8_t* d, uint64_t*, uint64_t* wr) {
+    const int e = gzip_file_impl(ctx, s, src_len, d, dst_cap, true, nullptr, &r);
+    *wr = r.written;
+    return e;
+  });
   if (rc != SFB200_RC_OK) return rc;
-  if (r.written > dst_cap) return SFB200_RC_CUDA_ERROR;  // (cannot happen)
-  if (r.written) SFB_TRY(ctx, cudaMemcpy(dst, ctx->d_dst, r.written, cudaMemcpyDeviceToHost));  // only what was produced
   *status = r.status;
-  if (written) *written = r.written;
   if (members) *members = r.members;
   return SFB200_RC_OK;
 }
@@ -2044,11 +1900,11 @@ int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, u
 {
   if (!ctx || !size || (!src && src_len)) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
-  const int rc0 = grow(ctx, &ctx->d_src, &ctx->d_src_cap, static_cast<uint64_t>(src_len) + 64);
-  if (rc0 != SFB200_RC_OK) return rc0;
-  if (src_len) SFB_TRY(ctx, cudaMemcpy(ctx->d_src, src, src_len, cudaMemcpyHostToDevice));
   GzfResult r;
-  const int rc = gzip_file_impl(ctx, ctx->d_src, src_len, nullptr, 0, false, nullptr, &r);
+  const int rc = host_buffer_call(ctx, src, src_len, nullptr, 0, nullptr,
+                                  [&](uint8_t* s, uint8_t*, uint64_t*, uint64_t*) {
+    return gzip_file_impl(ctx, s, src_len, nullptr, 0, false, nullptr, &r);
+  });
   if (rc != SFB200_RC_OK) return rc;
   *size = r.size;
   if (members) *members = r.members;
@@ -2064,15 +1920,9 @@ int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, u
 namespace {
 int seal_launch(sfb200_ctx* ctx, const sfb::SealArgs& s, cudaStream_t st)
 {
-  if (!ctx->seal_configured) {  // (function attributes are per device)
-    SFB_TRY(ctx, cudaFuncSetAttribute(sfb::container_seal_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      sfb::CHECK_SMEM_BYTES));
-    ctx->seal_configured = true;
-  }
   const uint64_t want = (s.n * 32 + sfb::CHECK_THREADS - 1) / sfb::CHECK_THREADS;
   const uint64_t resident = static_cast<uint64_t>(ctx->sm_count);  // (one block per SM: 128 KiB of tables)
-  sfb::container_seal_kernel<<<static_cast<unsigned>(want < resident ? want : resident), sfb::CHECK_THREADS,
-                               sfb::CHECK_SMEM_BYTES, st>>>(s);
+  sfb::container_seal_kernel<<<grid_size(want, resident), sfb::CHECK_THREADS, sfb::CHECK_SMEM_BYTES, st>>>(s);
   SFB_TRY(ctx, cudaGetLastError());
   ctx->launches += 1;
   return SFB200_RC_OK;
@@ -2105,9 +1955,9 @@ int sfb200_compress_container_batch_device(sfb200_ctx* ctx, int container, const
   if (!src_off || !src_len || !dst_off || !dst_cap || !status || !written) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
   cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
-  int rc = grow(ctx, &ctx->d_wrap, &ctx->d_wrap_cap, n * 16 + 64);
+  int rc = reserve(ctx, ctx->d_wrap, n * 16 + 64);
   if (rc != SFB200_RC_OK) return rc;
-  uint64_t* const pay_off = reinterpret_cast<uint64_t*>(ctx->d_wrap);
+  uint64_t* const pay_off = ctx->d_wrap.as<uint64_t>();
   uint64_t* const pay_cap = pay_off + n;
   sfb::container_frame_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(
       static_cast<uint32_t>(container), dst_off, dst_cap, pay_off, pay_cap, n);
@@ -2136,30 +1986,12 @@ int sfb200_compress_container(sfb200_ctx* ctx, int container, const uint8_t* src
   if (!ctx || !status || !written || (src_len && !src) || (dst_cap && !dst)) return SFB200_RC_BAD_ARGUMENT;
   if (container < SFB200_CONTAINER_RAW || container > SFB200_CONTAINER_GZIP) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
-  uint8_t* buf = nullptr;
-  const uint64_t in_pad = (static_cast<uint64_t>(src_len) + 255) & ~255ull;
-  const uint64_t total = in_pad + dst_cap + 256 + 64;
-  SFB_TRY(ctx, cudaMalloc(reinterpret_cast<void**>(&buf), total));
-  auto done = [&](int rc) {
-    cudaFree(buf);
-    return rc;
-  };
-  uint64_t h[6] = {0, src_len, 0, dst_cap, 0, 0};
-  uint64_t* meta = reinterpret_cast<uint64_t*>(buf + in_pad + ((dst_cap + 255) & ~255ull));
-  if (src_len && cudaMemcpy(buf, src, src_len, cudaMemcpyHostToDevice) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(src)"));
-  if (cudaMemcpy(meta, h, sizeof h, cudaMemcpyHostToDevice) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(meta)"));
-  int rc = sfb200_compress_container_batch_device(ctx, container, buf, meta + 0, meta + 1, buf + in_pad, meta + 2,
-                                                  meta + 3, reinterpret_cast<uint8_t*>(meta + 5), meta + 4, 1, nullptr);
-  if (rc != SFB200_RC_OK) return done(rc);
-  if (cudaMemcpy(h, meta, sizeof h, cudaMemcpyDeviceToHost) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(meta back)"));
-  *status = static_cast<uint8_t>(h[5] & 0xffu);
-  *written = h[4];
-  if (h[4] && cudaMemcpy(dst, buf + in_pad, h[4], cudaMemcpyDeviceToHost) != cudaSuccess)
-    return done(fail(ctx, cudaGetLastError(), "cudaMemcpy(dst)"));
-  return done(SFB200_RC_OK);
+  return host_buffer_call(ctx, src, src_len, dst, dst_cap, written,
+                          [&](uint8_t* s, uint8_t* d, uint64_t* m, uint64_t* wr) {
+    const int rc = sfb200_compress_container_batch_device(ctx, container, s, m, m + 1, d, m + 2, m + 3,
+                                                          reinterpret_cast<uint8_t*>(m + 5), m + 4, 1, nullptr);
+    return rc != SFB200_RC_OK ? rc : read_meta(ctx, m, wr, status);
+  });
 }
 
 uint64_t sfb200_compress_bgzf_bound(uint64_t src_len)
@@ -2180,10 +2012,10 @@ int sfb200_compress_bgzf_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t sr
   const uint64_t r = std::max<uint64_t>(1, std::min(pieces, slots));
   // slots (r x 64 KiB) | src_off, src_len, dst_off, dst_cap (r x u64 each) | written (r + 1) | state (4) | status (r)
   const uint64_t meta_at = r * sfb::BGZF_SLOT;
-  int rc = grow(ctx, &ctx->d_bgzf, &ctx->d_bgzf_cap, meta_at + 8 * (5 * r + 5) + r + 64);
+  int rc = reserve(ctx, ctx->d_bgzf, meta_at + 8 * (5 * r + 5) + r + 64);
   if (rc != SFB200_RC_OK) return rc;
-  uint8_t* const slot = ctx->d_bgzf;
-  uint64_t* const so = reinterpret_cast<uint64_t*>(ctx->d_bgzf + meta_at);
+  uint8_t* const slot = ctx->d_bgzf.p;
+  uint64_t* const so = reinterpret_cast<uint64_t*>(ctx->d_bgzf.p + meta_at);
   uint64_t* const sl = so + r;
   uint64_t* const dof = sl + r;
   uint64_t* const dc = dof + r;
@@ -2239,18 +2071,10 @@ int sfb200_compress_bgzf(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, ui
 {
   if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
   SFB_ENTER(ctx);
-  int rc = grow(ctx, &ctx->d_src, &ctx->d_src_cap, static_cast<uint64_t>(src_len) + 64);
-  if (rc != SFB200_RC_OK) return rc;
-  rc = grow(ctx, &ctx->d_dst, &ctx->d_dst_cap, static_cast<uint64_t>(dst_cap) + 64);
-  if (rc != SFB200_RC_OK) return rc;
-  if (src_len) SFB_TRY(ctx, cudaMemcpy(ctx->d_src, src, src_len, cudaMemcpyHostToDevice));
-  uint64_t wr = 0;
-  rc = sfb200_compress_bgzf_device(ctx, ctx->d_src, src_len, ctx->d_dst, dst_cap, status, &wr, members, nullptr);
-  if (rc != SFB200_RC_OK) return rc;
-  if (wr > dst_cap) return SFB200_RC_CUDA_ERROR;  // (cannot happen)
-  if (wr) SFB_TRY(ctx, cudaMemcpy(dst, ctx->d_dst, wr, cudaMemcpyDeviceToHost));  // only what was written
-  if (written) *written = wr;
-  return SFB200_RC_OK;
+  return host_buffer_call(ctx, src, src_len, dst, dst_cap, written,
+                          [&](uint8_t* s, uint8_t* d, uint64_t*, uint64_t* wr) {
+    return sfb200_compress_bgzf_device(ctx, s, src_len, d, dst_cap, status, wr, members, nullptr);
+  });
 }
 
 }  // extern "C"
