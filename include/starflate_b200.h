@@ -167,7 +167,8 @@ int sfb200_compress_batch_device(sfb200_ctx* ctx, const uint8_t* src_base, const
                                  const uint64_t* src_len, uint8_t* dst_base, const uint64_t* dst_off,
                                  const uint64_t* dst_cap, uint8_t* status, uint64_t* written, uint64_t n,
                                  void* cuda_stream);
-/* One stream in host memory. */
+/* One stream in host memory.  It is compressed by ONE warp (about 10 MB/s); a large buffer goes
+ * through sfb200_compress_parallel* instead, which writes one stream at batch speed. */
 int sfb200_compress(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* dst, size_t dst_cap,
                     uint8_t* status, uint64_t* written);
 
@@ -271,7 +272,7 @@ int sfb200_compress_container_batch_device(sfb200_ctx* ctx, int container, const
                                            const uint64_t* src_off, const uint64_t* src_len, uint8_t* dst_base,
                                            const uint64_t* dst_off, const uint64_t* dst_cap, uint8_t* status,
                                            uint64_t* written, uint64_t n, void* cuda_stream);
-/* One stream in host memory. */
+/* One stream in host memory, compressed by one warp: for a large buffer see sfb200_compress_parallel*. */
 int sfb200_compress_container(sfb200_ctx* ctx, int container, const uint8_t* src, size_t src_len, uint8_t* dst,
                               size_t dst_cap, uint8_t* status, uint64_t* written);
 
@@ -299,6 +300,36 @@ int sfb200_compress_bgzf_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t sr
  * are copied back. */
 int sfb200_compress_bgzf(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint8_t* dst, size_t dst_cap,
                          uint8_t* status, uint64_t* written, uint64_t* members);
+
+/* COMPRESSION of one buffer to ONE raw-DEFLATE, zlib or gzip stream at batch speed (what PNG IDAT, PDF
+ * FlateDecode, HTTP deflate, zip entries and single-member .gz files hold).  The input is cut into
+ * BGZF's pieces of 65 280 bytes; piece k is compressed by the batch compressor as one self-contained
+ * block (dynamic or fixed Huffman, or stored where neither is smaller than the piece + 5 bytes), BFINAL
+ * set only on the last piece, and the blocks follow one another at BIT granularity, with no gap and no
+ * empty stored block between them.  The last byte is padded with zero bits.  Header and trailer are
+ * byte-identical to sfb200_compress_container's (zlib 78 9c .. Adler-32; gzip 1f 8b 08 00, MTIME 0,
+ * XFL 0, OS 255 .. CRC-32, ISIZE = src_len mod 2^32), the checksum over the whole source computed on
+ * the device.  For src_len <= 65 280 the output is exactly sfb200_compress_container's.  The stream is
+ * one dynamic block per piece, which sfb200_decompress* decodes block by block side by side.
+ * `container`: RAW, ZLIB or GZIP; AUTO (or anything else) is SFB200_RC_BAD_ARGUMENT.  Any src_len,
+ * 4 GiB and more included.
+ *   *status   Success; SFB200_DST_TOO_SMALL when the stream does not fit dst_cap (never with dst_cap >=
+ *             sfb200_compress_parallel_bound(container, src_len) = header + trailer + src_len +
+ *             6 x max(1, ceil(src_len / 65 280))): *written = 0, no byte past dst_cap is touched and the
+ *             bytes before it are unspecified.
+ *   *written  (may be NULL) the stream's size.
+ * `src` and `dst` are DEVICE pointers, the results HOST pointers; synchronous on `cuda_stream`.
+ * Scratch and rounds are those of sfb200_compress_bgzf_device (SFB200_BGZF_SCRATCH_MB), with five kernel
+ * launches per round and no host round trip between them.  src is read twice (the compressor, then the
+ * checksum and the bytes of stored pieces); dst is written once. */
+uint64_t sfb200_compress_parallel_bound(int container, uint64_t src_len);
+int sfb200_compress_parallel_device(sfb200_ctx* ctx, int container, const uint8_t* src, uint64_t src_len,
+                                    uint8_t* dst, uint64_t dst_cap, uint8_t* status, uint64_t* written,
+                                    void* cuda_stream);
+/* The same with HOST buffers: input and output are staged on the device whole; only the bytes written
+ * are copied back. */
+int sfb200_compress_parallel(sfb200_ctx* ctx, int container, const uint8_t* src, size_t src_len,
+                             uint8_t* dst, size_t dst_cap, uint8_t* status, uint64_t* written);
 
 /* Position-weighted 64-bit checksum of each stream's output region [0, len[i]) computed on the
  * device (used by tests/bench to verify multi-GiB outputs without a device->host copy):

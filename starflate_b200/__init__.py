@@ -397,6 +397,46 @@ class Context:
         self._check(rc, "sfb200_compress_bgzf_device")
         return st.value, wr.value, nm.value
 
+    def compress_parallel_bound(self, container, n: int) -> int:
+        f = self.lib.sfb200_compress_parallel_bound
+        f.argtypes = [C.c_int, C.c_uint64]
+        f.restype = C.c_uint64
+        return int(f(container, n))
+
+    def compress_parallel(self, container, src: bytes, dst_cap: int = -1):
+        """One buffer in host memory -> (status, ONE raw-DEFLATE / zlib / gzip stream), its pieces
+        compressed side by side (sfb200_compress_parallel)."""
+        if dst_cap < 0:
+            dst_cap = self.compress_parallel_bound(container, len(src))
+        s = np.frombuffer(src, dtype=np.uint8) if len(src) else np.zeros(1, np.uint8)
+        d = np.zeros(max(dst_cap, 1), dtype=np.uint8)
+        st, wr = C.c_uint8(0), C.c_uint64(0)
+        f = self.lib.sfb200_compress_parallel
+        f.argtypes = [C.c_void_p, C.c_int, _u8p, C.c_size_t, _u8p, C.c_size_t, C.POINTER(C.c_uint8),
+                      C.POINTER(C.c_uint64)]
+        f.restype = C.c_int
+        self._check(f(self.h, container, _p(s, _u8p), len(src), _p(d, _u8p), dst_cap, C.byref(st), C.byref(wr)),
+                    "sfb200_compress_parallel")
+        return st.value, d[:wr.value].tobytes()
+
+    def compress_parallel_device(self, container, src, dst, stream=None):
+        """A uint8 CUDA tensor as one raw-DEFLATE / zlib / gzip stream into another (synchronous)
+        -> (status, written)."""
+        import torch
+        assert src.is_cuda and src.dtype == torch.uint8 and src.is_contiguous()
+        assert dst.is_cuda and dst.dtype == torch.uint8 and dst.is_contiguous()
+        if stream is None:
+            stream = torch.cuda.current_stream(src.device).cuda_stream
+        st, wr = C.c_uint8(0), C.c_uint64(0)
+        f = self.lib.sfb200_compress_parallel_device
+        f.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint8),
+                      C.POINTER(C.c_uint64), C.c_void_p]
+        f.restype = C.c_int
+        rc = f(self.h, container, src.data_ptr(), src.numel(), dst.data_ptr(), dst.numel(), C.byref(st), C.byref(wr),
+               stream)
+        self._check(rc, "sfb200_compress_parallel_device")
+        return st.value, wr.value
+
     def inflate_stream(self) -> "InflateStream":
         """Chunked input for one stream (sfb200_inflate_stream_*)."""
         return InflateStream(self)

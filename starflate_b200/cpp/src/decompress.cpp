@@ -245,6 +245,21 @@ auto compress_bgzf(std::span<const std::byte> src, std::span<std::byte> dst, std
   return static_cast<ContainerStatus>(status);
 }
 
+auto compress_parallel(std::span<const std::byte> src, std::span<std::byte> dst, Container container,
+                       std::size_t* written) -> ContainerStatus
+{
+  if (container == Container::Auto) return ContainerStatus::Error;
+  std::uint8_t status = 0;
+  std::uint64_t wr = 0;
+  const auto lease = pool().borrow();
+  const int rc = sfb200_compress_parallel(lease.get(), static_cast<int>(container),
+                                          reinterpret_cast<const std::uint8_t*>(src.data()), src.size(),
+                                          reinterpret_cast<std::uint8_t*>(dst.data()), dst.size(), &status, &wr);
+  if (rc != SFB200_RC_OK) return static_cast<ContainerStatus>(infra("sfb200_compress_parallel", rc, lease.get()));
+  if (written) *written = static_cast<std::size_t>(wr);
+  return static_cast<ContainerStatus>(status);
+}
+
 auto compress_bound(Container container, std::size_t src_size) -> std::size_t
 {
   return static_cast<std::size_t>(sfb200_compress_container_bound(static_cast<int>(container), src_size));
@@ -253,6 +268,11 @@ auto compress_bound(Container container, std::size_t src_size) -> std::size_t
 auto compress_bgzf_bound(std::size_t src_size) -> std::size_t
 {
   return static_cast<std::size_t>(sfb200_compress_bgzf_bound(src_size));
+}
+
+auto compress_parallel_bound(Container container, std::size_t src_size) -> std::size_t
+{
+  return static_cast<std::size_t>(sfb200_compress_parallel_bound(static_cast<int>(container), src_size));
 }
 
 auto decompress_batch(std::span<const std::span<const std::byte>> src,

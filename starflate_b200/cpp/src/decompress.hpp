@@ -112,9 +112,16 @@ auto compress_container(std::span<const std::byte> src, std::span<std::byte> dst
 /// members written, the EOF marker included.
 auto compress_bgzf(std::span<const std::byte> src, std::span<std::byte> dst, std::size_t* written = nullptr,
                    std::size_t* members = nullptr) -> ContainerStatus;
+/// Compresses src into dst as ONE raw-DEFLATE, zlib or gzip stream at batch speed (Auto is Error): pieces
+/// of 65 280 bytes compressed side by side as self-contained blocks, joined bit-exactly.  For inputs up
+/// to one piece the output is compress_container's.  Success, or DstTooSmall (nothing written);
+/// dst.size() >= compress_parallel_bound(container, src.size()) always fits.
+auto compress_parallel(std::span<const std::byte> src, std::span<std::byte> dst, Container container,
+                       std::size_t* written = nullptr) -> ContainerStatus;
 /// The dst.size() that always holds the output (0 for Auto).
 auto compress_bound(Container container, std::size_t src_size) -> std::size_t;
 auto compress_bgzf_bound(std::size_t src_size) -> std::size_t;
+auto compress_parallel_bound(Container container, std::size_t src_size) -> std::size_t;
 
 // ---- extension: the batched form the GPU is built for ------------------------------------------
 /// Stream i reads src[i] and writes dst[i] (host memory); status[i] / written[i] receive its

@@ -12,6 +12,7 @@
 #include "gzip_file.cuh"
 #include "deflate_compress.cuh"
 #include "container_write.cuh"
+#include "compress_parallel.cuh"
 
 #include <cstdio>
 #include <cstdlib>
@@ -315,7 +316,8 @@ int sfb200_create(int device, sfb200_ctx** out)
                                          : reinterpret_cast<const void*>(sfb::lz_window_kernel<6>);
   const void* lz = ctx->lz_v1 ? reinterpret_cast<const void*>(sfb::lz_resolve_kernel) : lzw;
   // the kernels the calls launch (pass 1, size discovery, the END decode of gzip members, the container
-  // checksums and seal, compression, pass 2): a context has them all
+  // checksums and seal, compression and its piece mode, the parallel stream's stitch, pass 2): a
+  // context has them all
   int lz_per_sm = 0;
   if (setup_kernel(sfb::huff_lanes_kernel<LaneCfg>, LaneCfg::SMEM_BYTES, true, LaneCfg::WARPS * 32, &ctx->ctas_per_sm,
                    &ctx->regs_per_thread) != cudaSuccess ||
@@ -326,6 +328,8 @@ int sfb200_create(int device, sfb200_ctx** out)
       setup_kernel(sfb::container_seal_kernel, sfb::CHECK_SMEM_BYTES, false) != cudaSuccess ||
       setup_kernel(sfb::deflate_compress_kernel, sfb::CMP_SMEM_BYTES, false, sfb::CMP_WARPS * 32,
                    &ctx->compress_ctas_per_sm) != cudaSuccess ||
+      setup_kernel(sfb::deflate_compress_pieces_kernel, sfb::CMP_SMEM_BYTES, false) != cudaSuccess ||
+      setup_kernel(sfb::par_stitch_kernel, sfb::CHECK_SMEM_BYTES, false) != cudaSuccess ||
       setup_kernel(lz, 0, false, sfb::LZ_THREADS, &lz_per_sm, &ctx->lz_regs_per_thread) != cudaSuccess || lz_per_sm < 1)
     return bail(SFB200_RC_CUDA_ERROR);
   ctx->compress_ctas_per_sm = std::max(1, ctx->compress_ctas_per_sm);
@@ -2074,6 +2078,124 @@ int sfb200_compress_bgzf(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, ui
   return host_buffer_call(ctx, src, src_len, dst, dst_cap, written,
                           [&](uint8_t* s, uint8_t* d, uint64_t*, uint64_t* wr) {
     return sfb200_compress_bgzf_device(ctx, s, src_len, d, dst_cap, status, wr, members, nullptr);
+  });
+}
+
+
+// One buffer as one raw-DEFLATE / zlib / gzip stream (compress_parallel.cuh): BGZF's pieces and rounds,
+// the blocks joined at bit granularity.
+//
+// Bound: a piece of L bytes compressed as a Huffman block is kept only when ceil(bits / 8) <= L + 5,
+// so it takes at most 8 (L + 5) bits.  A stored piece takes align8(B + 3) - B + 32 + 8 L bits, at most
+// 10 + 32 + 8 L = 8 (L + 5) + 2 (when it starts at bit phase 6).  Over p pieces of n bytes in all that is
+// at most 8 n + 42 p bits, which with the zero padding of the last byte is n + 5 p + ceil(2 p / 8) <=
+// n + 6 p bytes, plus header and trailer.
+uint64_t sfb200_compress_parallel_bound(int container, uint64_t src_len)
+{
+  if (container < SFB200_CONTAINER_RAW || container > SFB200_CONTAINER_GZIP) return 0;
+  const uint64_t frame = container == SFB200_CONTAINER_ZLIB ? 6 : container == SFB200_CONTAINER_GZIP ? 18 : 0;
+  const uint64_t pieces = std::max<uint64_t>(1, (src_len + sfb::BGZF_PIECE - 1) / sfb::BGZF_PIECE);
+  return frame + src_len + 6 * pieces;
+}
+
+int sfb200_compress_parallel_device(sfb200_ctx* ctx, int container, const uint8_t* src, uint64_t src_len,
+                                    uint8_t* dst, uint64_t dst_cap, uint8_t* status, uint64_t* written,
+                                    void* cuda_stream)
+{
+  if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
+  if (container < SFB200_CONTAINER_RAW || container > SFB200_CONTAINER_GZIP) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  const uint64_t pieces = std::max<uint64_t>(1, (src_len + sfb::BGZF_PIECE - 1) / sfb::BGZF_PIECE);
+  uint64_t budget_mb = 8192;  // BGZF's scratch budget: 64 KiB per piece of a round (SFB200_BGZF_SCRATCH_MB)
+  if (const char* e = std::getenv("SFB200_BGZF_SCRATCH_MB")) budget_mb = std::max<long long>(1, std::atoll(e));
+  const uint64_t slots = std::max<uint64_t>(1, (budget_mb << 20) / sfb::BGZF_SLOT);
+  const uint64_t r = std::min(pieces, slots);
+  // slots (r x 64 KiB) | src_off, src_len, dst_off, dst_cap (r x u64 each) | pos (r + 1) | state |
+  // sums (r x u32) | kinds (r)
+  const uint64_t meta_at = r * sfb::BGZF_SLOT;
+  int rc = reserve(ctx, ctx->d_bgzf, meta_at + 8 * (5 * r + 1 + sfb::PAR_STATE_WORDS) + 5 * r + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  uint64_t* const so = reinterpret_cast<uint64_t*>(ctx->d_bgzf.p + meta_at);
+  uint64_t* const sl = so + r;
+  uint64_t* const dof = sl + r;
+  uint64_t* const dc = dof + r;
+  uint64_t* const pos = dc + r;
+  uint64_t* const state = pos + r + 1;
+  uint32_t* const sums = reinterpret_cast<uint32_t*>(state + sfb::PAR_STATE_WORDS);
+  uint8_t* const kinds = reinterpret_cast<uint8_t*>(sums + r);
+  const uint64_t hb = container == SFB200_CONTAINER_ZLIB ? 2 : container == SFB200_CONTAINER_GZIP ? 10 : 0;
+  uint64_t init[sfb::PAR_STATE_WORDS] = {};
+  init[sfb::PAR_BASE] = 8 * hb;
+  init[sfb::PAR_SUM] = container == SFB200_CONTAINER_ZLIB ? 1 : 0;  // the Adler-32 / CRC-32 of nothing
+  SFB_TRY(ctx, cudaMemcpyAsync(state, init, sizeof init, cudaMemcpyHostToDevice, st));
+  sfb::CompressArgs c;
+  c.src_base = src;
+  c.src_off = so;
+  c.src_len = sl;
+  c.dst_base = ctx->d_bgzf.p;
+  c.dst_off = dof;
+  c.dst_cap = dc;
+  c.status = kinds;
+  c.written = pos;
+  c.counter = ctx->d_counter.as<unsigned long long>();
+  c.fixed_only = 0;
+  sfb::ParArgs a{};
+  a.src = src;
+  a.src_off = so;
+  a.src_len = sl;
+  a.slots = ctx->d_bgzf.p;
+  a.kind = kinds;
+  a.pos = pos;
+  a.sum = sums;
+  a.dst = dst;
+  a.dst_cap = dst_cap;
+  a.state = state;
+  a.container = static_cast<uint32_t>(container);
+  const uint64_t resident = static_cast<uint64_t>(ctx->sm_count) * static_cast<uint64_t>(ctx->compress_ctas_per_sm);
+  uint64_t first = 0;
+  do {  // one round per r pieces (an empty input is one empty piece)
+    const uint64_t n = std::min(r, pieces - first);
+    const bool last = first + n >= pieces;
+    sfb::bgzf_split_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(src_len, sfb::BGZF_PIECE, first, n,
+                                                                                 so, sl, dof, dc);
+    SFB_TRY(ctx, cudaGetLastError());
+    SFB_TRY(ctx, cudaMemsetAsync(ctx->d_counter.p, 0, sizeof(unsigned long long), st));
+    c.n = n;
+    a.n = n;
+    a.last = last ? n - 1 : ~0ull;
+    const uint64_t want = (n + sfb::CMP_WARPS - 1) / sfb::CMP_WARPS;
+    sfb::deflate_compress_pieces_kernel<<<grid_size(want, resident), sfb::CMP_WARPS * 32, sfb::CMP_SMEM_BYTES, st>>>(
+        c, a.last);
+    SFB_TRY(ctx, cudaGetLastError());
+    sfb::par_scan_kernel<<<1, sfb::PAR_THREADS, 0, st>>>(a);
+    SFB_TRY(ctx, cudaGetLastError());
+    const uint64_t swant = (n * 32 + sfb::CHECK_THREADS - 1) / sfb::CHECK_THREADS;
+    const uint64_t sresident = static_cast<uint64_t>(ctx->sm_count);  // (one block per SM: 128 KiB of tables)
+    sfb::par_stitch_kernel<<<grid_size(swant, sresident), sfb::CHECK_THREADS, sfb::CHECK_SMEM_BYTES, st>>>(a);
+    SFB_TRY(ctx, cudaGetLastError());
+    sfb::par_advance_kernel<<<1, sfb::PAR_THREADS, 0, st>>>(a, last ? 1 : 0);
+    SFB_TRY(ctx, cudaGetLastError());
+    ctx->launches += 5;
+    first += n;
+  } while (first < pieces);
+  uint64_t res[2] = {0, 0};
+  SFB_TRY(ctx, cudaMemcpyAsync(res, state + sfb::PAR_STATUS, sizeof res, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  *status = static_cast<uint8_t>(res[0]);
+  if (written) *written = res[1];
+  return SFB200_RC_OK;
+}
+
+int sfb200_compress_parallel(sfb200_ctx* ctx, int container, const uint8_t* src, size_t src_len, uint8_t* dst,
+                             size_t dst_cap, uint8_t* status, uint64_t* written)
+{
+  if (!ctx || !status || (!src && src_len) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
+  if (container < SFB200_CONTAINER_RAW || container > SFB200_CONTAINER_GZIP) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  return host_buffer_call(ctx, src, src_len, dst, dst_cap, written,
+                          [&](uint8_t* s, uint8_t* d, uint64_t*, uint64_t* wr) {
+    return sfb200_compress_parallel_device(ctx, container, s, src_len, d, dst_cap, status, wr, nullptr);
   });
 }
 

@@ -512,7 +512,14 @@ __device__ __forceinline__ void cmp_parse(const uint8_t* s, uint32_t n, uint16_t
   __syncwarp();
 }
 
-__global__ void __launch_bounds__(CMP_WARPS * 32) deflate_compress_kernel(const CompressArgs a)
+// Piece mode (PIECES, compress_parallel.cuh): stream si is one piece of a larger buffer.  BFINAL is
+// set only on stream `last`; nothing is written for a piece that falls back to a stored block (the
+// stitch kernel writes it from the source at its final bit position); status is ST_SUCCESS or
+// CMP_PIECE_STORED, written the block's exact size in BITS (0 when stored).
+constexpr uint8_t CMP_PIECE_STORED = 0x80;
+
+template <bool PIECES>
+__device__ __forceinline__ void cmp_streams(const CompressArgs& a, uint64_t last)
 {
 #ifdef SFB_CPU_EMU
   uint8_t* const smem = reinterpret_cast<uint8_t*>(SFB_EMU_SMEM);
@@ -537,6 +544,7 @@ __global__ void __launch_bounds__(CMP_WARPS * 32) deflate_compress_kernel(const 
     if (lane == 0) si = atomicAdd(a.counter, 1ull);
     si = __shfl_sync(FULL, si, 0);
     if (si >= a.n) break;
+    const bool fin = !PIECES || si == last;   // BFINAL
     const uint64_t slen = a.src_len[si], cap64 = a.dst_cap[si];
     if (slen >= 0xffffff00ull) {
       if (lane == 0) {
@@ -685,8 +693,8 @@ __global__ void __launch_bounds__(CMP_WARPS * 32) deflate_compress_kernel(const 
     // ---- pass B: the block ---------------------------------------------------------------------
     if (dynamic) {
       const uint8_t order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
-      // BFINAL = 1, BTYPE = 10, HLIT, HDIST, HCLEN
-      w.put(5u | ((hlit - 257u) << 3) | ((hdist - 1u) << 8) | ((hclen - 4u) << 13), lane == 0u ? 17u : 0u);
+      // BFINAL, BTYPE = 10, HLIT, HDIST, HCLEN
+      w.put((fin ? 5u : 4u) | ((hlit - 257u) << 3) | ((hdist - 1u) << 8) | ((hclen - 4u) << 13), lane == 0u ? 17u : 0u);
       w.put(lane < hclen ? l_cl[order[lane < 19u ? lane : 0u]] : 0u, lane < hclen ? 3u : 0u);
       for (uint32_t base = 0; base < nseq; base += 32u) {
         uint64_t bits = 0;
@@ -703,12 +711,22 @@ __global__ void __launch_bounds__(CMP_WARPS * 32) deflate_compress_kernel(const 
       w.put(t_ll[256] & 0xffffu, lane == 0u ? t_ll[256] >> 16 : 0u);   // end of block
     } else {
       uint64_t dummy = 0;
-      w.put(3u, lane == 0u ? 3u : 0u);   // BFINAL = 1, BTYPE = 01
+      w.put(fin ? 3u : 2u, lane == 0u ? 3u : 0u);   // BFINAL, BTYPE = 01
       cmp_parse<1>(s, n, tab, lane, w, t_ll, t_d, &dummy);
       w.put(0u, lane == 0u ? 7u : 0u);   // end of block: seven zero bits
     }
+    const uint64_t bits = 32ull * w.wbase + w.cur;
     const uint64_t comp = w.close();
     const uint64_t stored = cmp_stored_size(n);
+    if constexpr (PIECES) {   // the same choice of block as below (the stored size does not depend on where it lands)
+      const bool as_stored = comp > stored || comp > cap;
+      if (lane == 0) {
+        a.status[si] = as_stored ? CMP_PIECE_STORED : static_cast<uint8_t>(ST_SUCCESS);
+        a.written[si] = as_stored ? 0 : bits;
+      }
+      __syncwarp();
+      continue;
+    }
     uint64_t out = comp;
     int st = ST_SUCCESS;
     if (comp > stored || comp > cap) {
@@ -727,6 +745,15 @@ __global__ void __launch_bounds__(CMP_WARPS * 32) deflate_compress_kernel(const 
     }
     __syncwarp();
   }
+}
+
+__global__ void __launch_bounds__(CMP_WARPS * 32) deflate_compress_kernel(const CompressArgs a) { cmp_streams<false>(a, 0); }
+
+// piece mode: `last` = the index of the stream that ends the buffer (none: ~0).  (Five CTAs per SM is
+// what the shared memory allows anyway; without the hint ptxas takes 64 registers and spills.)
+__global__ void __launch_bounds__(CMP_WARPS * 32, 5) deflate_compress_pieces_kernel(const CompressArgs a, uint64_t last)
+{
+  cmp_streams<true>(a, last);
 }
 
 }  // namespace sfb
