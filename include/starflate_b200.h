@@ -255,6 +255,54 @@ int sfb200_decompress_gzip_file(sfb200_ctx* ctx, const uint8_t* src, size_t src_
 int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, uint64_t* size, uint64_t* members,
                           int* complete);
 
+/* ZIP ARCHIVES (PKWARE APPNOTE 6.3 as Python's zipfile reads them: ZIP64, prepended bytes, data
+ * descriptors).  The entry table is the interface: list it, optionally filter or reorder its rows,
+ * then extract them.  Deflated (method 8) entries are decoded side by side by the batch path, stored
+ * (method 0) ones copied; the CRC-32 of every entry's output is checked against the central
+ * directory, all on the device.  Sizes and CRC come from the central directory; data descriptors
+ * are skipped, not read.  Other methods, encryption and split archives are not supported. */
+typedef struct sfb200_zip_entry {  /* 64 bytes */
+  uint64_t name_off;   /* file name bytes: src[name_off .. + name_len) (central directory) */
+  uint64_t data_off;   /* stored / compressed bytes: src[data_off .. + comp_size) */
+  uint64_t comp_size;
+  uint64_t size;       /* uncompressed size (central directory) */
+  uint64_t dst_off;    /* where extract writes the entry; list fills it packed in directory order */
+  uint64_t written;    /* extract: bytes produced */
+  uint32_t crc32;
+  uint16_t method, flags;
+  uint16_t name_len;
+  uint8_t status;      /* list: Success, or SFB200_BAD_CONTAINER for a row that cannot be extracted
+                        * (bad local header, data outside the file, a method other than 0 / 8,
+                        * encryption); extract: the entry's result (below) */
+  uint8_t pad[5];
+} sfb200_zip_entry;
+/* *status: Success, or SFB200_BAD_CONTAINER for the archive as a whole (no end-of-central-directory
+ * record, a split archive, a central directory whose chain of records does not hold exactly the
+ * record's count).  *count = entries in the archive (0 when it is rejected); only the first
+ * min(count, cap) rows are written (cap 0 sizes the table).  *total_size = sum of `size` = the dst_cap
+ * a packed extract needs.  src and entries are DEVICE pointers, the three results HOST pointers;
+ * synchronous on cuda_stream.  Memory touched: aligned 16-byte loads inside the blocks that hold the
+ * archive's bytes. */
+int sfb200_zip_list_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, sfb200_zip_entry* entries,
+                           uint64_t cap, uint8_t* status, uint64_t* count, uint64_t* total_size, void* cuda_stream);
+/* The same with HOST buffers (the archive is staged on the device whole). */
+int sfb200_zip_list(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, sfb200_zip_entry* entries, uint64_t cap,
+                    uint8_t* status, uint64_t* count, uint64_t* total_size);
+/* Decodes rows [0, n) of `entries` (any subset or order of a list's rows) into
+ * dst[dst_off .. + size) and writes status / written into the rows.  Regions must not overlap.
+ * Per-row status: the DEFLATE status of the payload; SFB200_CHECKSUM_MISMATCH (the output's CRC-32 is
+ * not the central directory's); SFB200_SIZE_MISMATCH (the output size is not `size`, a stored entry
+ * whose comp_size is not its size, or a payload that produces more than `size` while dst had room);
+ * SFB200_DST_TOO_SMALL (dst ends inside the entry's region: every byte that fits is produced);
+ * SFB200_BAD_CONTAINER (a row list marked so, data outside src, an unsupported method or
+ * encryption); SFB200_ERROR (a deflated entry of >= 2^32 - 256 bytes, compressed or not; stored
+ * entries have no size limit).  src, entries and dst are DEVICE pointers; synchronous on cuda_stream. */
+int sfb200_zip_extract_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, sfb200_zip_entry* entries,
+                              uint64_t n, uint8_t* dst, uint64_t dst_cap, void* cuda_stream);
+/* The same with HOST buffers: only the bytes produced are copied back (dst keeps its other bytes). */
+int sfb200_zip_extract(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, sfb200_zip_entry* entries, uint64_t n,
+                       uint8_t* dst, size_t dst_cap);
+
 /* COMPRESSION to zlib (RFC 1950) and gzip (RFC 1952): sfb200_compress_batch_device's streams with
  * header and trailer, the Adler-32 / CRC-32 (and ISIZE) of each stream's SOURCE bytes computed on the
  * device.  zlib: 78 9c, payload, Adler-32 big endian.  gzip: 1f 8b 08 00, MTIME 0, XFL 0, OS 255

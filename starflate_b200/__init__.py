@@ -14,13 +14,19 @@ import numpy as np
 
 from . import build as _build
 
-__all__ = ["Context", "StarflateError", "STATUS_NAMES", "load_library", "library_path"]
+__all__ = ["Context", "StarflateError", "STATUS_NAMES", "ZIP_ENTRY", "load_library", "library_path"]
 
 STATUS_NAMES = {
     0: "Success", 1: "Error", 2: "InvalidBlockHeader", 3: "NoCompressionLenMismatch",
     4: "DstTooSmall", 5: "SrcTooSmall", 6: "InvalidLitOrLen", 7: "InvalidDistance",
 }
 _RC_NAMES = {0: "OK", 1: "NO_DEVICE", 2: "BAD_ARGUMENT", 3: "CUDA_ERROR", 4: "OUT_OF_MEMORY"}
+
+# one row of a zip archive's entry table (include/starflate_b200.h: sfb200_zip_entry)
+ZIP_ENTRY = np.dtype([("name_off", "<u8"), ("data_off", "<u8"), ("comp_size", "<u8"), ("size", "<u8"),
+                      ("dst_off", "<u8"), ("written", "<u8"), ("crc32", "<u4"), ("method", "<u2"),
+                      ("flags", "<u2"), ("name_len", "<u2"), ("status", "u1"), ("pad", "u1", (5,))])
+assert ZIP_ENTRY.itemsize == 64
 
 
 class StarflateError(RuntimeError):
@@ -207,6 +213,88 @@ class Context:
         f.restype = C.c_int
         self._check(f(self.h, _p(s, _u8p), len(src), C.byref(sz), C.byref(nm), C.byref(cp)), "sfb200_gzip_file_size")
         return sz.value, nm.value, bool(cp.value)
+
+    # -- zip archives: list the entry table, then extract any subset or order of its rows -----------
+    @staticmethod
+    def _zip_rows_guess(n_bytes: int) -> int:
+        """Rows to offer the first listing call: every central-directory record takes >= 46 bytes, and
+        the table is kept to 1/16 of the archive's size unless that is below 65 536 rows; an archive
+        with more entries than this is listed a second time with room for all of them."""
+        return min(n_bytes // 46, max(65536, n_bytes // 1024))
+
+    def zip_list(self, data: bytes):
+        """-> (status, entries, names): `entries` a ZIP_ENTRY numpy array (the rows of
+        sfb200_zip_list), `names` the entries' file names decoded as zipfile decodes them (UTF-8 when
+        flag bit 11 is set, else cp437).  status 8 (BadContainer): not an archive this reads."""
+        s = np.frombuffer(data, dtype=np.uint8) if len(data) else np.zeros(1, np.uint8)
+        f = self.lib.sfb200_zip_list
+        f.argtypes = [C.c_void_p, _u8p, C.c_size_t, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint8),
+                      C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+        f.restype = C.c_int
+        st, n, total = C.c_uint8(0), C.c_uint64(0), C.c_uint64(0)
+        rows = np.zeros(max(self._zip_rows_guess(len(data)), 1), ZIP_ENTRY)
+        for _ in range(2):
+            self._check(f(self.h, _p(s, _u8p), len(data), rows.ctypes.data, len(rows), C.byref(st), C.byref(n),
+                          C.byref(total)), "sfb200_zip_list")
+            if n.value <= len(rows):
+                break
+            rows = np.zeros(n.value, ZIP_ENTRY)
+        rows = rows[:n.value]
+        names = [bytes(data[o:o + k]).decode("utf-8" if fl & 0x800 else "cp437")
+                 for o, k, fl in zip(rows["name_off"].tolist(), rows["name_len"].tolist(), rows["flags"].tolist())]
+        return st.value, rows, names
+
+    def zip_extract(self, data: bytes, entries: np.ndarray, dst_cap: int, fill: int = 0):
+        """Extract the rows of `entries` (a ZIP_ENTRY array, e.g. zip_list's or a subset of it) into a
+        dst of dst_cap bytes -> (dst bytes, the rows with status / written filled in)."""
+        s = np.frombuffer(data, dtype=np.uint8) if len(data) else np.zeros(1, np.uint8)
+        rows = np.ascontiguousarray(entries, dtype=ZIP_ENTRY).copy()
+        d = np.full(max(dst_cap, 1), fill, dtype=np.uint8)
+        f = self.lib.sfb200_zip_extract
+        f.argtypes = [C.c_void_p, _u8p, C.c_size_t, C.c_void_p, C.c_uint64, _u8p, C.c_size_t]
+        f.restype = C.c_int
+        self._check(f(self.h, _p(s, _u8p), len(data), rows.ctypes.data if len(rows) else None, len(rows), _p(d, _u8p),
+                      dst_cap), "sfb200_zip_extract")
+        return d[:dst_cap].tobytes(), rows
+
+    def zip_list_device(self, src, stream=None):
+        """An archive in a uint8 CUDA tensor -> (status, entries, total_size): `entries` a uint8 CUDA
+        tensor of shape (n, 64) holding the rows (ZIP_ENTRY layout; .cpu().numpy().view(ZIP_ENTRY))."""
+        import torch
+        assert src.is_cuda and src.dtype == torch.uint8 and src.is_contiguous()
+        if stream is None:
+            stream = torch.cuda.current_stream(src.device).cuda_stream
+        f = self.lib.sfb200_zip_list_device
+        f.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint8),
+                      C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
+        f.restype = C.c_int
+        st, n, total = C.c_uint8(0), C.c_uint64(0), C.c_uint64(0)
+        rows = torch.empty((max(self._zip_rows_guess(src.numel()), 1), 64), dtype=torch.uint8, device=src.device)
+        for _ in range(2):
+            self._check(f(self.h, src.data_ptr(), src.numel(), rows.data_ptr(), rows.shape[0], C.byref(st), C.byref(n),
+                          C.byref(total), stream), "sfb200_zip_list_device")
+            if n.value <= rows.shape[0]:
+                break
+            rows = torch.empty((n.value, 64), dtype=torch.uint8, device=src.device)
+        rows = rows[:n.value]
+        return st.value, rows, total.value
+
+    def zip_extract_device(self, src, entries, dst, stream=None):
+        """Extract the rows of `entries` (a uint8 CUDA tensor of shape (n, 64), e.g. zip_list_device's)
+        into the uint8 CUDA tensor dst; status / written are written into the rows (synchronous)."""
+        import torch
+        assert src.is_cuda and src.dtype == torch.uint8 and src.is_contiguous()
+        assert dst.is_cuda and dst.dtype == torch.uint8 and dst.is_contiguous()
+        assert entries.is_cuda and entries.dtype == torch.uint8 and entries.is_contiguous()
+        assert entries.numel() % 64 == 0
+        if stream is None:
+            stream = torch.cuda.current_stream(src.device).cuda_stream
+        f = self.lib.sfb200_zip_extract_device
+        f.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p]
+        f.restype = C.c_int
+        n = entries.numel() // 64
+        self._check(f(self.h, src.data_ptr(), src.numel(), entries.data_ptr() if n else None, n, dst.data_ptr(),
+                      dst.numel(), stream), "sfb200_zip_extract_device")
 
     def decompressed_size_batch_device(self, src, src_off, src_len, status, size, stream=None):
         """Size discovery: status[i] / size[i] of a decode into an unlimited dst; nothing is stored."""

@@ -216,6 +216,38 @@ auto gzip_file_size(std::span<const std::byte> src) -> std::optional<std::size_t
   return static_cast<std::size_t>(size);
 }
 
+auto zip_list(std::span<const std::byte> src) -> std::expected<std::vector<ZipEntry>, ContainerStatus>
+{
+  static_assert(sizeof(ZipEntry) == sizeof(sfb200_zip_entry));
+  std::uint8_t status = 0;
+  std::uint64_t count = 0;
+  const auto lease = pool().borrow();
+  const auto* s = reinterpret_cast<const std::uint8_t*>(src.data());
+  int rc = sfb200_zip_list(lease.get(), s, src.size(), nullptr, 0, &status, &count, nullptr);
+  std::vector<ZipEntry> rows;
+  if (rc == SFB200_RC_OK && status == 0 && count) {
+    rows.resize(count);
+    rc = sfb200_zip_list(lease.get(), s, src.size(), reinterpret_cast<sfb200_zip_entry*>(rows.data()), count, &status,
+                         &count, nullptr);
+  }
+  if (rc != SFB200_RC_OK) return std::unexpected{static_cast<ContainerStatus>(infra("sfb200_zip_list", rc, lease.get()))};
+  if (status != 0) return std::unexpected{static_cast<ContainerStatus>(status)};
+  return rows;
+}
+
+auto zip_extract(std::span<const std::byte> src, std::span<ZipEntry> entries, std::span<std::byte> dst) -> bool
+{
+  const auto lease = pool().borrow();
+  const int rc = sfb200_zip_extract(lease.get(), reinterpret_cast<const std::uint8_t*>(src.data()), src.size(),
+                                    reinterpret_cast<sfb200_zip_entry*>(entries.data()), entries.size(),
+                                    reinterpret_cast<std::uint8_t*>(dst.data()), dst.size());
+  if (rc != SFB200_RC_OK) {
+    infra("sfb200_zip_extract", rc, lease.get());
+    return false;
+  }
+  return true;
+}
+
 auto compress_container(std::span<const std::byte> src, std::span<std::byte> dst, Container container,
                         std::size_t* written) -> ContainerStatus
 {

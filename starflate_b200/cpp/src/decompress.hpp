@@ -14,6 +14,7 @@
 #include <ranges>
 #include <optional>
 #include <span>
+#include <vector>
 
 namespace starflate {
 
@@ -100,6 +101,26 @@ auto decompress_gzip_file(std::span<const std::byte> src, std::span<std::byte> d
 /// The sum of ISIZE over the BGZF members of src — the dst.size() decompress_gzip_file needs — or
 /// nothing when they do not cover the file (a member without the BGZF field, trailing bytes).
 auto gzip_file_size(std::span<const std::byte> src) -> std::optional<std::size_t>;
+
+// ---- extension: zip archives -----------------------------------------------------------------
+/// One entry of a zip archive (the C ABI's sfb200_zip_entry): where its name and data lie in the
+/// archive, its sizes and CRC-32 from the central directory, where zip_extract writes it and what that
+/// produced.  `status`: ContainerStatus values.
+struct ZipEntry
+{
+  std::uint64_t name_off, data_off, comp_size, size, dst_off, written;
+  std::uint32_t crc32;
+  std::uint16_t method, flags, name_len;
+  std::uint8_t status;
+  std::uint8_t pad[5];
+};
+static_assert(sizeof(ZipEntry) == 64);
+/// The entry table of a zip archive (dst_off packed in directory order), or BadContainer (or the
+/// infrastructure failure) for an archive this cannot read.
+auto zip_list(std::span<const std::byte> src) -> std::expected<std::vector<ZipEntry>, ContainerStatus>;
+/// Extracts the given rows (any subset or order of zip_list's) into dst[dst_off .. + size), checking
+/// every entry's CRC-32; status / written are written into the rows.  False on an infrastructure failure.
+auto zip_extract(std::span<const std::byte> src, std::span<ZipEntry> entries, std::span<std::byte> dst) -> bool;
 
 // ---- extension: compression to raw DEFLATE, zlib, gzip and BGZF ---------------------------------
 /// Compresses src into dst as one raw-DEFLATE, zlib or gzip stream (Auto is Error), the checksum of

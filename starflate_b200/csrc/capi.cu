@@ -13,6 +13,7 @@
 #include "deflate_compress.cuh"
 #include "container_write.cuh"
 #include "compress_parallel.cuh"
+#include "zip_file.cuh"
 
 #include <cstdio>
 #include <cstdlib>
@@ -21,6 +22,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 namespace {
@@ -128,6 +130,11 @@ struct sfb200_ctx {
   DevBuf d_gzf;      // gzip files (gzip_file.cuh): the walk's step, result, probe metadata, tile counts
   DevBuf d_gzc;      // ... candidates and jump tables
   DevBuf d_gzm;      // ... the member table (kGzfMemberBytes per member, gzm_members)
+  DevBuf d_zip;      // zip archives (zip_file.cuh): ZipInfo, the chain's step, tile counts
+  DevBuf d_zipl;     // ... listing: CD record positions and lengths, sizes and their scan
+  DevBuf d_zipx;     // ... extraction: the decoder's arrays, slots, kinds, piece counts
+  DevBuf d_zipc;     // ... the piece CRCs
+  DevBuf d_zips;     // ... windows of decoder groups whose regions are not back to back in dst
   DevBuf d_wrap;     // writing containers (container_write.cuh): the payloads' offsets and capacities
   DevBuf d_bgzf;     // writing BGZF: a round's scratch slots, the compressor's arrays, the call's state
   DevBuf d_find;     // single-stream pass 1 (block_finder.cuh): counters, hash table, jobs, candidates
@@ -330,6 +337,7 @@ int sfb200_create(int device, sfb200_ctx** out)
                    &ctx->compress_ctas_per_sm) != cudaSuccess ||
       setup_kernel(sfb::deflate_compress_pieces_kernel, sfb::CMP_SMEM_BYTES, false) != cudaSuccess ||
       setup_kernel(sfb::par_stitch_kernel, sfb::CHECK_SMEM_BYTES, false) != cudaSuccess ||
+      setup_kernel(sfb::zip_piece_kernel, sfb::CHECK_SMEM_BYTES, false) != cudaSuccess ||
       setup_kernel(lz, 0, false, sfb::LZ_THREADS, &lz_per_sm, &ctx->lz_regs_per_thread) != cudaSuccess || lz_per_sm < 1)
     return bail(SFB200_RC_CUDA_ERROR);
   ctx->compress_ctas_per_sm = std::max(1, ctx->compress_ctas_per_sm);
@@ -1914,6 +1922,346 @@ int sfb200_gzip_file_size(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, u
   if (members) *members = r.members;
   if (complete) *complete = r.complete ? 1 : 0;
   return SFB200_RC_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// zip archives (zip_file.cuh).  Listing: the EOCD (one small read-back), the CD's candidates (one
+// more), then the chain, the rows and their packed offsets with one read-back at the end.
+// Extraction: the split and slot kernels sort the rows; deflated entries go through the raw batch
+// path — those of at least kZipLarge bytes apart from the rest, so that one large entry does not
+// become one lane of the lane kernel (a lane decodes some 10 MB/s: a 1 GiB entry among 65 536 small
+// ones would take the whole batch 100 s) —, each group on a window holding only its own outputs, so
+// that the router's choice and its scratch follow the group and not what else dst holds; then the
+// piece kernel copies stored entries (and groups decoded in scratch) and checksums every entry's
+// output in pieces, and the result kernel combines the pieces' CRCs per row.
+namespace {
+constexpr uint64_t kZipLarge = 1ull << 20;  // DESIGN.md §3 "zip archives": the sweep that chose it
+// Group 1 (entries >= kZipLarge) one call each or as one batch: a fixed cost per call and the
+// single-stream rate, against one warp's rate for the largest entry.  Measured on B200 (DESIGN.md §3):
+// 64 entries of 16 MiB one call each 117.9 ms, as one batch 258 ms; one 1 GiB entry alone 45.5 ms.
+constexpr uint64_t kZipStage = 64ull << 20;  // host extract: produced regions this close come back in one copy
+constexpr double kZipCallMs = 1.13;                     // per call, beside its bytes
+constexpr double kZipStreamBpms = 23.6e6;               // bytes per ms, single-stream route
+constexpr double kZipWarpBpms = 65.0e3;                 // bytes per ms, one warp per entry
+
+struct ZipListResult {
+  uint8_t status = sfb::ST_BAD_CONTAINER;
+  uint64_t count = 0, total = 0;
+};
+
+int zip_list_impl(sfb200_ctx* ctx, const uint8_t* src, uint64_t len, sfb::ZipEntry* rows, uint64_t cap,
+                  cudaStream_t st, ZipListResult* res)
+{
+  *res = ZipListResult{};
+  // ZipInfo (64 B) | the chain's step (128 B) | tile counts
+  int rc = reserve(ctx, ctx->d_zip, 64 + 128 + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  sfb::zip_eocd_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(src, len, ctx->d_zip.as<sfb::ZipInfo>());
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 1;
+  sfb::ZipInfo info{};
+  SFB_TRY(ctx, cudaMemcpyAsync(&info, ctx->d_zip.p, sizeof info, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  if (info.status != 0) return SFB200_RC_OK;
+  const uint64_t n = info.n, cd = info.cd_end - info.cd_begin;
+  // ---- candidates over the CD (positions relative to its start) ------------------------------------
+  sfb::GzfArgs a{};
+  a.src = src + info.cd_begin;
+  a.len = cd;
+  a.dst_cap = ~0ull;
+  const uint64_t tile = static_cast<uint64_t>(sfb::GZF_THREADS) * sfb::GZF_BYTES;
+  const uint64_t tiles = cd ? (cd + (reinterpret_cast<uintptr_t>(a.src) & 15u) + tile - 1) / tile : 0;
+  rc = reserve(ctx, ctx->d_zip, 64 + 128 + 8 * (tiles + 1), 64);
+  if (rc != SFB200_RC_OK) return rc;
+  sfb::ZipInfo* const d_info = ctx->d_zip.as<sfb::ZipInfo>();
+  a.step = reinterpret_cast<sfb::GzfStep*>(ctx->d_zip.p + 64);
+  a.tile_count = reinterpret_cast<uint64_t*>(ctx->d_zip.p + 192);
+  uint64_t m = 0;
+  if (tiles) {
+    sfb::zip_count_kernel<<<static_cast<unsigned>(tiles), sfb::GZF_THREADS, 0, st>>>(a);
+    sfb::gzf_exscan_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(a.tile_count, tiles);
+    SFB_TRY(ctx, cudaGetLastError());
+    ctx->launches += 2;
+    SFB_TRY(ctx, cudaMemcpyAsync(&m, a.tile_count + tiles, 8, cudaMemcpyDeviceToHost, st));
+    SFB_TRY(ctx, cudaStreamSynchronize(st));
+  }
+  if (n > m) return SFB200_RC_OK;  // fewer records than the EOCD counts
+  if (m >= 0xffffffffull) {         // (candidate indices are 32-bit: a CD of > 180 GiB)
+    ctx->err = "zip archive: more than 2^32 - 2 central directory record candidates";
+    return SFB200_RC_BAD_ARGUMENT;
+  }
+  uint32_t tables = 1;
+  while ((1ull << tables) < m + 1) ++tables;
+  if (const char* e = std::getenv("SFB200_GZIP_CHAIN"))  // (tests: =walk takes the fallback)
+    if (e[0] == 'w') tables = 1;
+  auto cand_bytes = [&](uint32_t t) { return 16 * m + 4 * (m + 1) * static_cast<uint64_t>(t) + 64; };
+  rc = reserve(ctx, ctx->d_gzc, cand_bytes(tables));
+  if (rc == SFB200_RC_OUT_OF_MEMORY && tables > 1) {  // one thread walks the chain instead
+    cudaGetLastError();
+    ctx->err.clear();
+    tables = 1;
+    rc = reserve(ctx, ctx->d_gzc, cand_bytes(tables));
+  }
+  if (rc != SFB200_RC_OK) return rc;
+  a.cpos = ctx->d_gzc.as<uint64_t>();
+  a.cnext = a.cpos + m;
+  a.jump = reinterpret_cast<uint32_t*>(a.cnext + m);
+  a.m = m;
+  a.n_tables = tables;
+  // record positions and lengths (m each), the sizes and their scan (n + 1)
+  rc = reserve(ctx, ctx->d_zipl, 8 * (2 * m + n + 1) + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  a.mpos = ctx->d_zipl.as<uint64_t>();
+  a.mlen = a.mpos + m;
+  uint64_t* const sizes = a.mlen + m;
+  sfb::GzfStep h{};
+  h.head = 0;  // the chain starts at the CD's first byte
+  SFB_TRY(ctx, cudaMemcpyAsync(a.step, &h, sizeof h, cudaMemcpyHostToDevice, st));
+  const unsigned cgrid = static_cast<unsigned>((m + 1 + 255) / 256);
+  if (tiles) sfb::zip_scatter_kernel<<<static_cast<unsigned>(tiles), sfb::GZF_THREADS, 0, st>>>(a);
+  sfb::gzf_succ_kernel<<<cgrid, 256, 0, st>>>(a);
+  for (uint32_t r = 0; r + 1 < tables; ++r) sfb::gzf_jump_kernel<<<cgrid, 256, 0, st>>>(a, r);
+  if (tables == 1) {
+    sfb::gzf_walk_kernel<<<1, 1, 0, st>>>(a);
+  } else {
+    sfb::gzf_chain_kernel<<<1, 1, 0, st>>>(a);
+    sfb::gzf_expand_kernel<<<cgrid, 256, 0, st>>>(a);
+    ctx->launches += 1;
+  }
+  ctx->launches += (tiles ? 1 : 0) + tables + 1;
+  // ---- the rows ----------------------------------------------------------------------------------
+  sfb::ZipArgs z{};
+  z.src = src;
+  z.len = len;
+  z.info = d_info;
+  z.step = a.step;
+  z.mpos = a.mpos;
+  z.rows = rows;
+  z.cap = cap;
+  z.size = sizes;
+  if (n) sfb::zip_entry_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(z);
+  sfb::gzf_exscan_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(sizes, n);
+  const uint64_t shown = std::min(n, cap);
+  if (shown) sfb::zip_offsets_kernel<<<static_cast<unsigned>((shown + 255) / 256), 256, 0, st>>>(z);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 1 + (n ? 1 : 0) + (shown ? 1 : 0);
+  uint64_t total = 0;
+  SFB_TRY(ctx, cudaMemcpyAsync(&h, a.step, sizeof h, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaMemcpyAsync(&total, sizes + n, 8, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  if (h.count != n || h.stop != cd) return SFB200_RC_OK;  // the records do not fill the CD as counted
+  res->status = SFB200_SUCCESS;
+  res->count = n;
+  res->total = total;
+  return SFB200_RC_OK;
+}
+
+int zip_extract_impl(sfb200_ctx* ctx, const uint8_t* src, uint64_t len, sfb::ZipEntry* rows, uint64_t n, uint8_t* dst,
+                     uint64_t dst_cap, cudaStream_t st)
+{
+  if (n == 0) return SFB200_RC_OK;
+  if (n >= 0xffffffffull) return SFB200_RC_BAD_ARGUMENT;  // (decoder slots are 32-bit)
+  // six u64 arrays of the decoder, piece counts and four group columns (n + 1 each), five span words
+  // | slots (u32) | kinds, decoder statuses (u8)
+  const uint64_t words = 6 * n + 5 * (n + 1) + 5;
+  int rc = reserve(ctx, ctx->d_zipx, 8 * words + 4 * n + 2 * n + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  sfb::ZipExArgs x{};
+  x.src = src;
+  x.len = len;
+  x.rows = rows;
+  x.n = n;
+  x.dst = dst;
+  x.dst_cap = dst_cap;
+  x.large = kZipLarge;
+  x.d_off = ctx->d_zipx.as<uint64_t>();
+  x.d_len = x.d_off + n;
+  x.d_pos = x.d_len + n;
+  x.d_room = x.d_pos + n;
+  x.d_written = x.d_room + n;
+  x.d_dst = x.d_written + n;
+  x.pieces = x.d_dst + n;
+  x.group = x.pieces + n + 1;
+  x.span = reinterpret_cast<unsigned long long*>(x.group + 4 * (n + 1));
+  x.slot = reinterpret_cast<uint32_t*>(x.span + 5);
+  x.kind = reinterpret_cast<uint8_t*>(x.slot + n);
+  x.d_status = x.kind + n;
+  const unsigned long long span0[5] = {~0ull, 0, ~0ull, 0, 0};
+  SFB_TRY(ctx, cudaMemcpyAsync(x.span, span0, sizeof span0, cudaMemcpyHostToDevice, st));
+  const unsigned rgrid = static_cast<unsigned>((n + 255) / 256);
+  sfb::zip_split_kernel<<<rgrid, 256, 0, st>>>(x);
+  sfb::gzf_exscan_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(x.pieces, n);
+  for (int c = 0; c < 4; ++c) sfb::gzf_exscan_kernel<<<1, sfb::GZF_SCAN_THREADS, 0, st>>>(x.group + c * (n + 1), n);
+  sfb::zip_slot_kernel<<<rgrid, 256, 0, st>>>(x);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 7;
+  uint64_t h[5], sp[5];  // g0 count, g0 bytes, g1 count, g1 bytes, pieces | spans, largest g1 room
+  for (int c = 0; c < 4; ++c)
+    SFB_TRY(ctx, cudaMemcpyAsync(h + c, x.group + c * (n + 1) + n, 8, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaMemcpyAsync(h + 4, x.pieces + n, 8, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaMemcpyAsync(sp, x.span, sizeof sp, cudaMemcpyDeviceToHost, st));
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  const uint64_t cnt[2] = {h[0], h[2]}, bytes[2] = {h[1], h[3]}, pieces = h[4];
+  // Group 1 one entry per call (each on its own window, on the single-stream route) or as one batch
+  // (a warp per entry): the batch costs about its largest entry at one warp's rate, the calls a fixed
+  // cost each plus their bytes at the single-stream rate (DESIGN.md §3 "zip archives", measured).
+  const bool alone = cnt[1] && static_cast<double>(cnt[1]) * kZipCallMs + static_cast<double>(bytes[1]) / kZipStreamBpms <
+                                   static_cast<double>(sp[4]) / kZipWarpBpms;
+  // each batched group's window: dst where its regions lie back to back, else scratch
+  bool in_place[2];
+  uint64_t scratch_at[2] = {0, 0}, need = 0;
+  for (int g = 0; g < 2; ++g) {
+    in_place[g] = sp[2 * g] == sp[2 * g + 1];
+    if (cnt[g] && !in_place[g] && !(g == 1 && alone)) {
+      scratch_at[g] = need;
+      need += bytes[g] + 16;
+    }
+  }
+  if (need) {
+    rc = reserve(ctx, ctx->d_zips, need);
+    if (rc != SFB200_RC_OK) return rc;
+  }
+  for (int g = 0; g < 2; ++g) {
+    if (!cnt[g] || (g == 1 && alone)) continue;
+    const uint64_t b = g ? cnt[0] : 0;
+    uint8_t* const win = in_place[g] ? dst + (sp[2 * g] - sfb::ZIP_BIAS) : ctx->d_zips.p + scratch_at[g];
+    if (!in_place[g]) x.scratch[g] = win;
+    rc = sfb200_decompress_batch_device(ctx, src, x.d_off + b, x.d_len + b, win, bytes[g], x.d_pos + b, x.d_room + b,
+                                        x.d_status + b, x.d_written + b, cnt[g], st);
+    if (rc != SFB200_RC_OK) return rc;
+  }
+  if (alone) {  // each on its own dst window: its scratch is in proportion to its size
+    std::vector<uint64_t> doff(cnt[1]), room(cnt[1]);
+    SFB_TRY(ctx, cudaMemcpyAsync(doff.data(), x.d_dst + cnt[0], 8 * cnt[1], cudaMemcpyDeviceToHost, st));
+    SFB_TRY(ctx, cudaMemcpyAsync(room.data(), x.d_room + cnt[0], 8 * cnt[1], cudaMemcpyDeviceToHost, st));
+    SFB_TRY(ctx, cudaStreamSynchronize(st));
+    uint64_t* const d_zero = reinterpret_cast<uint64_t*>(x.span);  // (read back already: a zero dst offset)
+    SFB_TRY(ctx, cudaMemsetAsync(d_zero, 0, 8, st));
+    for (uint64_t j = 0, i = cnt[0]; j < cnt[1]; ++j, ++i) {
+      rc = sfb200_decompress_batch_device(ctx, src, x.d_off + i, x.d_len + i, dst + doff[j], room[j], d_zero,
+                                          x.d_room + i, x.d_status + i, x.d_written + i, 1, st);
+      if (rc != SFB200_RC_OK) return rc;
+    }
+  }
+  // ---- stored copies, copies out of scratch, CRCs, results ---------------------------------------
+  rc = reserve(ctx, ctx->d_zipc, 4 * pieces + 64);
+  if (rc != SFB200_RC_OK) return rc;
+  x.pcrc = ctx->d_zipc.as<uint32_t>();
+  if (pieces) {
+    const uint64_t want = (pieces * 32 + sfb::CHECK_THREADS - 1) / sfb::CHECK_THREADS;
+    const uint64_t resident = static_cast<uint64_t>(ctx->sm_count);  // (one block per SM: 128 KiB of tables)
+    sfb::zip_piece_kernel<<<grid_size(want, resident), sfb::CHECK_THREADS, sfb::CHECK_SMEM_BYTES, st>>>(x);
+    ctx->launches += 1;
+  }
+  sfb::zip_result_kernel<<<rgrid, 256, 0, st>>>(x);
+  SFB_TRY(ctx, cudaGetLastError());
+  ctx->launches += 1;
+  SFB_TRY(ctx, cudaStreamSynchronize(st));
+  return SFB200_RC_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int sfb200_zip_list_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, sfb200_zip_entry* entries,
+                           uint64_t cap, uint8_t* status, uint64_t* count, uint64_t* total_size, void* cuda_stream)
+{
+  static_assert(sizeof(sfb200_zip_entry) == sizeof(sfb::ZipEntry), "one row layout");
+  if (!ctx || !status || !count || (!src && src_len) || (!entries && cap)) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  ZipListResult r;
+  const int rc = zip_list_impl(ctx, src, src_len, reinterpret_cast<sfb::ZipEntry*>(entries), cap,
+                               static_cast<cudaStream_t>(cuda_stream), &r);
+  if (rc != SFB200_RC_OK) return rc;
+  *status = r.status;
+  *count = r.count;
+  if (total_size) *total_size = r.total;
+  return SFB200_RC_OK;
+}
+
+int sfb200_zip_list(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, sfb200_zip_entry* entries, uint64_t cap,
+                    uint8_t* status, uint64_t* count, uint64_t* total_size)
+{
+  if (!ctx || !status || !count || (!src && src_len) || (!entries && cap) || cap > (1ull << 40))
+    return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  ZipListResult r;
+  const int rc = host_buffer_call(ctx, src, src_len, reinterpret_cast<uint8_t*>(entries), cap * sizeof(sfb200_zip_entry),
+                                  nullptr, [&](uint8_t* s, uint8_t* d, uint64_t*, uint64_t* wr) {
+    const int e = zip_list_impl(ctx, s, src_len, reinterpret_cast<sfb::ZipEntry*>(d), cap, nullptr, &r);
+    *wr = std::min(r.count, cap) * sizeof(sfb200_zip_entry);
+    return e;
+  });
+  if (rc != SFB200_RC_OK) return rc;
+  *status = r.status;
+  *count = r.count;
+  if (total_size) *total_size = r.total;
+  return SFB200_RC_OK;
+}
+
+int sfb200_zip_extract_device(sfb200_ctx* ctx, const uint8_t* src, uint64_t src_len, sfb200_zip_entry* entries,
+                              uint64_t n, uint8_t* dst, uint64_t dst_cap, void* cuda_stream)
+{
+  if (!ctx || (!src && src_len) || (!entries && n) || (!dst && dst_cap)) return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  return zip_extract_impl(ctx, src, src_len, reinterpret_cast<sfb::ZipEntry*>(entries), n, dst, dst_cap,
+                          static_cast<cudaStream_t>(cuda_stream));
+}
+
+int sfb200_zip_extract(sfb200_ctx* ctx, const uint8_t* src, size_t src_len, sfb200_zip_entry* entries, uint64_t n,
+                       uint8_t* dst, size_t dst_cap)
+{
+  if (!ctx || (!src && src_len) || (!entries && n) || (!dst && dst_cap) || n > (1ull << 40))
+    return SFB200_RC_BAD_ARGUMENT;
+  SFB_ENTER(ctx);
+  return host_buffer_call(ctx, src, src_len, dst, dst_cap, nullptr,
+                          [&](uint8_t* s, uint8_t* d, uint64_t*, uint64_t* wr) -> int {
+    *wr = 0;  // (the rows' regions come back below, not a prefix of dst)
+    const uint64_t bytes = n * sizeof(sfb200_zip_entry);
+    int rc = reserve(ctx, ctx->d_zipl, bytes + 64);
+    if (rc != SFB200_RC_OK) return rc;
+    auto* const rows = ctx->d_zipl.as<sfb::ZipEntry>();
+    if (n) SFB_TRY(ctx, cudaMemcpyAsync(rows, entries, bytes, cudaMemcpyHostToDevice, nullptr));
+    rc = zip_extract_impl(ctx, s, src_len, rows, n, d, dst_cap, nullptr);
+    if (rc != SFB200_RC_OK) return rc;
+    if (n) SFB_TRY(ctx, cudaMemcpy(entries, rows, bytes, cudaMemcpyDeviceToHost));
+    // only the bytes produced: the rows' [dst_off, + written) in dst order, adjacent ones merged into
+    // runs; runs that lie within kZipStage bytes of each other come back in one copy through a host
+    // staging buffer, so that a scattered subset costs one copy per kZipStage bytes, not one per row
+    std::vector<std::pair<uint64_t, uint64_t>> runs;  // [lo, hi)
+    {
+      std::vector<uint64_t> order;
+      order.reserve(n);
+      for (uint64_t i = 0; i < n; ++i)
+        if (entries[i].written) order.push_back(i);
+      auto start = [&](uint64_t i) { return std::min<uint64_t>(entries[i].dst_off, dst_cap); };
+      std::sort(order.begin(), order.end(), [&](uint64_t p, uint64_t q) { return start(p) < start(q); });
+      for (const uint64_t i : order) {
+        const uint64_t lo = start(i), hi = std::min<uint64_t>(lo + entries[i].written, dst_cap);
+        if (!runs.empty() && lo <= runs.back().second) runs.back().second = std::max(runs.back().second, hi);
+        else runs.emplace_back(lo, hi);
+      }
+    }
+    std::vector<uint8_t> stage;
+    for (size_t k = 0; k < runs.size();) {
+      size_t e = k + 1;  // runs [k, e) share one staged copy
+      while (e < runs.size() && runs[e].second - runs[k].first <= kZipStage) ++e;
+      if (e == k + 1) {
+        SFB_TRY(ctx, cudaMemcpy(dst + runs[k].first, d + runs[k].first, runs[k].second - runs[k].first,
+                                cudaMemcpyDeviceToHost));
+      } else {
+        const uint64_t lo = runs[k].first, hi = runs[e - 1].second;
+        stage.resize(hi - lo);
+        SFB_TRY(ctx, cudaMemcpy(stage.data(), d + lo, hi - lo, cudaMemcpyDeviceToHost));
+        for (size_t j = k; j < e; ++j)
+          std::memcpy(dst + runs[j].first, stage.data() + (runs[j].first - lo), runs[j].second - runs[j].first);
+      }
+      k = e;
+    }
+    return SFB200_RC_OK;
+  });
 }
 
 }  // extern "C"
