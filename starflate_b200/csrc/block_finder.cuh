@@ -351,7 +351,7 @@ __global__ void __launch_bounds__(FIND_THREADS) verify_candidates_kernel(const F
   }
 }
 
-#ifndef SFB_CPU_EMU  // (tests/cpu_emu runs the finder kernels on one host thread and the walk above)
+#if !defined(SFB_CPU_EMU) || defined(SFB_EMU_BLOCK)  // (tests/cpu_emu: emu_block.cpp runs this on 1024 host threads)
 
 // The same chain, in parallel, by ONE block (the walk above takes 0.5 us per block of the stream:
 // 6 ms for the 12 000 blocks of a 1 GiB stream).  Pointer jumping over the jobs: J[j] = the job 2^k

@@ -71,7 +71,7 @@ __device__ __forceinline__ uint32_t lz_type_rank(const PrepArgs& a, uint64_t i)
 
 constexpr int PREP_THREADS = 256;
 
-#ifndef SFB_CPU_EMU  // (block-level kernels: exercised on the device only)
+#if !defined(SFB_CPU_EMU) || defined(SFB_EMU_BLOCK)  // (block-level kernels: tests/cpu_emu/emu_block.cpp)
 
 __global__ void __launch_bounds__(PREP_THREADS) prep_count_kernel(const PrepArgs a)
 {

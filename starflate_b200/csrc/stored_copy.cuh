@@ -74,7 +74,7 @@ __device__ __forceinline__ void stored_warp_copy(const uint8_t* s, uint8_t* d, u
   for (uint32_t i = head + 16u * slots + lane; i < n; i += 32u) d[i] = s[i];
 }
 
-#ifndef SFB_CPU_EMU
+#if !defined(SFB_CPU_EMU) || defined(SFB_EMU_BLOCK)
 __global__ void __launch_bounds__(STORED_THREADS) stored_streams_kernel(const StoredArgs a)
 {
   constexpr unsigned FULL = 0xffffffffu;
